@@ -26,6 +26,7 @@ if ROOT not in sys.path:
 
 METRIC = "vcycle_fine_grid_dof_per_s"
 UNIT = "DOF/s"
+DUMP_SAMPLE = 1 << 22          # float64 entries of the iterate written by --dump-outputs: 32 MB
 
 
 def parse_args():
@@ -75,7 +76,26 @@ def parse_args():
                          "cycle at 8 GPUs) but a worse smoother: V(1,1) convergence factor 0.23 instead of 0.20 "
                          "(profiles/r01_convergence_factors.txt), so it loses on time to solution")
     ap.add_argument("--min-rows-per-rank", type=int, default=int(os.environ.get("MGB_MIN_ROWS", "65536")))
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR as float64 .npy files: "
+                         "solution.npy (the fine-grid iterate, or a fixed seeded sample of %d of its entries) and "
+                         "residual_norm.npy (the residual norm that step computed); the inputs depend on the arguments "
+                         "only, so two builds can be compared output for output" % DUMP_SAMPLE)
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+def dump_outputs(path, solution, residual_norm):
+    """--dump-outputs: the iterate (all of it up to DUMP_SAMPLE entries, otherwise the entries at a fixed seeded sample
+    of indices in increasing order) and the residual norm, as float64 .npy files under `path`."""
+    x = np.asarray(solution, dtype=np.float64).reshape(-1)
+    if x.size > DUMP_SAMPLE:
+        x = x[np.sort(np.random.default_rng(0).choice(x.size, DUMP_SAMPLE, replace=False))]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "solution.npy"), x)
+    np.save(os.path.join(path, "residual_norm.npy"), np.array([residual_norm], dtype=np.float64))
 
 
 def workload_name(a, n):
@@ -247,20 +267,16 @@ def run_reference(a):
     o = OracleMultigrid(A, rhs, Qs, smoother=sm, omega=2.0 / 3.0, hoist_setup=False)
     x = np.zeros_like(rhs)
     Af = o.matrix
-    budget = 150.0
-    t_begin = time.perf_counter()
-    done = 0
     for it in range(a.warmup + a.steps):
         t0 = time.perf_counter()
         r = rhs - Af.dot(x)
-        np.linalg.norm(r)
+        res = np.linalg.norm(r)
         x = o.v_cycle(Af, x, rhs, a.nu, a.levels)
         dt = time.perf_counter() - t0
         if it >= a.warmup:
             times.append(dt)
-        done += 1
-        if time.perf_counter() - t_begin > budget and len(times) >= 1:
-            break
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, x, res)
     per = float(np.mean(times))
     val = (n + 1) ** 2 / per
     sample = ("%dx%d grid (%d DOF) of the same %d-level V(%d,%d) configuration, %d timed cycles, Galerkin products "
@@ -509,6 +525,11 @@ def run_b200(a):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms_total = float(t.item())
     ms_step = ms_total / a.steps
+    if a.dump_outputs:
+        x_last, norm_last = h.get_x(view=True), h.last_norm()   # partitioned: get_x gathers the row blocks of all ranks
+        if rank == 0:
+            dump_outputs(a.dump_outputs, x_last, norm_last)
+        del x_last
     if a.profile_step:
         torch.cuda.synchronize()
         torch.cuda.profiler.start()

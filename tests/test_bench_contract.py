@@ -1,16 +1,24 @@
-"""bench.py contract checks that need no GPU: the reference arm (`--impl reference`: the oracle with the reference's
-per-cycle Galerkin products and LU, on host cores) prints ONE JSON line with the keys the driver reads, and the
-argument parser accepts the driver's command lines."""
+"""bench.py contract checks: the reference arm (`--impl reference`: the oracle with the reference's per-cycle Galerkin
+products and LU, on host cores) prints ONE JSON line with the keys a caller reads, the argument parser accepts the
+documented command lines, and --dump-outputs writes what the last timed step computed (the B200 arm's check needs a
+GPU)."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
+from helpers import history_tolerance
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def run_bench(*args, env=None):
-    e = dict(os.environ, CUDA_VISIBLE_DEVICES="", **(env or {}))
+def run_bench(*args, env=None, gpu=False):
+    e = dict(os.environ, **(env or {}))
+    if not gpu:
+        e["CUDA_VISIBLE_DEVICES"] = ""
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True,
                          timeout=600, env=e, cwd=ROOT)
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
@@ -39,3 +47,50 @@ def test_reference_arm_on_a_non_zero_rank_exits_without_work():
                           "--steps", "1", "--warmup", "0", "--cpu-n", "32"], capture_output=True, text=True,
                          timeout=300, env=e, cwd=ROOT)
     assert out.returncode == 0 and not [l for l in out.stdout.splitlines() if l.startswith("{")]
+
+
+def load_dump(path):
+    out = {name: np.load(os.path.join(path, name + ".npy")) for name in ("solution", "residual_norm")}
+    assert all(v.dtype == np.float64 for v in out.values()) and out["residual_norm"].shape == (1,)
+    return out
+
+
+def test_reference_arm_dumps_its_last_step(tmp_path):
+    """--steps sets the number of timed steps; --dump-outputs writes the iterate the last step left and the residual
+    norm it computed (that of the iterate it started from), the same bits in two runs"""
+    from learnmultigrid_b200 import problems as P
+    d = run_bench("--impl", "reference", "--steps", "1", "--warmup", "0", "--cpu-n", "32",
+                  "--dump-outputs", str(tmp_path / "first"))
+    assert d["steps"] == 1
+    first = load_dump(tmp_path / "first")
+    assert first["solution"].shape == (33 * 33,)
+    assert first["residual_norm"][0] == np.linalg.norm(P.structured_rhs_2d(32))        # started from x = 0
+    dumps = []
+    for k in range(2):
+        d = run_bench("--impl", "reference", "--steps", "3", "--warmup", "1", "--cpu-n", "32",
+                      "--dump-outputs", str(tmp_path / str(k)))
+        assert d["steps"] == 3
+        dumps.append(load_dump(tmp_path / str(k)))
+    for name in dumps[0]:
+        assert np.array_equal(dumps[0][name], dumps[1][name])
+    assert dumps[0]["residual_norm"][0] < first["residual_norm"][0]
+
+
+@pytest.mark.gpu
+def test_b200_arm_dumps_its_last_step(tmp_path):
+    """the timed path's iterate after exactly --steps cycles from zero and the residual norm of that iterate, the same
+    bits in two runs"""
+    from learnmultigrid_b200 import problems as P
+    N = 128
+    dumps = []
+    for k, warmup in enumerate((1, 4)):
+        d = run_bench("--gpus", "1", "--steps", "4", "--warmup", str(warmup), "--n", str(N), "--levels", "4",
+                      "--no-cpu-baseline", "--no-e2e", "--no-extra", "--dump-outputs", str(tmp_path / str(k)), gpu=True)
+        assert d["steps"] == 4
+        dumps.append(load_dump(tmp_path / str(k)))
+    for name in dumps[0]:
+        assert np.array_equal(dumps[0][name], dumps[1][name])
+    A, b = P.structured_laplacian_2d(N), P.structured_rhs_2d(N).reshape(-1)
+    x = dumps[0]["solution"]
+    assert x.shape == ((N + 1) ** 2,)
+    assert abs(dumps[0]["residual_norm"][0] - np.linalg.norm(b - A @ x)) <= history_tolerance(A, x)

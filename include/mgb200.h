@@ -102,7 +102,13 @@ typedef struct {
      * deduplicating the records (structured levels have a handful; at most 65534).  h_spec_*: optional host-side hints, for launches
      * over the rows [h_spec_row[k], h_spec_row[k+1]) the record most of those slices use is h_spec_rec[9 * k] (its id)
      * with the offsets h_spec_rec[9 * k + 1 .. 9 * k + 8]; the launch passes it by value and the kernel gathers with
-     * it BEFORE the slice's id has arrived (n_spec = 0: record 0, the most frequent one, is assumed). */
+     * it BEFORE the slice's id has arrived (n_spec = 0: record 0, the most frequent one, is assumed).
+     * nrec < 0: the same fields hold -nrec SLICE PATTERNS instead (transfer operators, whose columns live in another
+     * level's numbering; L = uniform_len <= 8): entry j of lane l of a slice s with id r has the column base[s] +
+     * d_rec_table[(r * L + j) * 32 + l] and the value d_rec_vals[(r * L + j) * 32 + l]; base[s] = the slice's first
+     * stored column (entry 0 of lane 0) = d_rec_table[-nrec * L * 32 + s].  h_spec_rec[9 * k] is the pattern most slices
+     * of block k use, h_spec_rec[9 * k + 1] how many of them do in per mille (the other 7 ints unused), h_spec_vals
+     * unused. */
     const uint16_t *d_slice_rec;
     const int32_t *d_rec_table;
     int32_t nrec, n_spec;
@@ -144,6 +150,11 @@ int mg_set_value_dict(int enabled);
  * setting. */
 int mg_set_implied_values(int enabled);
 int mg_set_implied_columns(int enabled);
+/* Implied transfer columns (default 1; results identical): SpMV (restriction) and prolongation launches over matrices
+ * that carry slice patterns (mg_sell.nrec < 0) read a record id and a base column per slice instead of the columns and
+ * values of its rows (launches of at least mg_set_implied_min_rows rows).  Returns the previous setting; a negative
+ * argument only returns it. */
+int mg_set_implied_transfers(int enabled);
 /* launches of fewer rows keep loading their columns (one dependent load less on latency-bound launches); returns the
  * previous floor (default 2^19) */
 int64_t mg_set_implied_min_rows(int64_t rows);

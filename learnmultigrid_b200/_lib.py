@@ -143,6 +143,7 @@ _SIGNATURES = {
     "mg_pcg_iterate": (c_int, [c_vp, ctypes.POINTER(mg_level), c_int, ctypes.POINTER(mg_cycle_params),
                                ctypes.POINTER(mg_pcg), c_int, c_vp]),
     "mg_set_implied_columns": (c_int, [c_int]),
+    "mg_set_implied_transfers": (c_int, [c_int]),
     "mg_sell_residual": (c_int, [ctypes.POINTER(mg_sell), c_vp, c_vp, c_vp, c_vp]),
     "mg_sell_residual_norm2": (c_int, [ctypes.POINTER(mg_sell), c_vp, c_vp, c_vp, c_vp, c_vp]),
     "mg_norm_workspace_size": (c_i64, [c_i64]),
@@ -280,6 +281,8 @@ def load():
         lib.mg_set_fused_exchange(0)
     if os.environ.get("MGB_IMPLIED_COLUMNS", "1") == "0":
         lib.mg_set_implied_columns(0)
+    if os.environ.get("MGB_IMPLIED_TRANSFERS", "1") == "0":
+        lib.mg_set_implied_transfers(0)
     if "MGB_IMPLIED_MIN_ROWS" in os.environ:
         lib.mg_set_implied_min_rows(int(os.environ["MGB_IMPLIED_MIN_ROWS"]))
     if os.environ.get("MGB_VALUE_DICT", "1") == "0":

@@ -515,6 +515,117 @@ sell_short_kernel(SellArgs A, const double *x, const double *aux, double *y) {
     }
 }
 
+// ---- implied transfer columns: slice patterns ---------------------------------------------------------------------
+// A transfer operator's columns live in the other level's colour-blocked numbering, so `col = row + off[j]` (implied
+// columns above) never holds.  What does hold, for almost every slice of a structured hierarchy, is that the slice's
+// columns are its first stored column (entry 0 of lane 0, the base) plus one of a few LEN x 32 delta patterns, and its
+// values one of a few value patterns (linear interpolation: 1, 1/2 and the padding's 0): mg_sell with nrec < 0
+// (engine.DeviceSell._attach_patterns, formats.pattern_records).  A slice then reads a two-byte record id and a
+// four-byte base, both from dense per-slice arrays that a CTA's warps share in L1, instead of 32*LEN*(4+1) bytes of
+// columns and dictionary bytes; the pattern itself comes from L1 (the records of a launch are a few KB).
+// SPEC (the restriction: one record covers nearly every slice of a colour block): the launch carries the record most
+// slices of each row block use, the thread loads its deltas by lane from L1 at once and issues the x gathers as soon as
+// the base arrives, before the slice's own id is known; slices of another record redo their gathers.  Without SPEC (the
+// prolongation: its slices split over about four patterns per colour -- grid-line parity x the colour of lane 0 -- so
+// three quarters would miss and gather twice) the thread waits for the id and reads that record: base and id (L2 / L1)
+// -> deltas (L1) -> x, where the explicit kernel has columns (DRAM) -> x.  Irregular slices (0xffff) read their columns
+// and values.  Products are added in storage order from the same doubles: the same bits as sell_kernel and
+// sell_short_kernel.  R rows per thread, 256 apart, for the one- and two-entry rows of a prolongation.
+constexpr int kPatBlocks = 8;       // row blocks with their own expected record per launch
+
+struct PatArgs {
+    const unsigned short *__restrict__ rec;    // [nslices] record id, 0xffff = read the slice's columns and values
+    const int32_t *__restrict__ base;          // [nslices] first stored column of the slice
+    const int32_t *__restrict__ delta;         // [nrec][LEN][32] column - base
+    const double *__restrict__ pvals;          // [nrec][LEN][32] values
+    const int32_t *__restrict__ cols;
+    const double *__restrict__ vals;
+    int32_t spec_row[kPatBlocks];              // block k = rows [spec_row[k], spec_row[k+1]) (unused: INT32_MAX)
+    int32_t spec_id[kPatBlocks];               // ... and the record its launch expects (SPEC)
+    int32_t row_begin, row_end, first_row;
+    uint32_t col_max;                          // ncols - 1: speculative columns are clamped to it
+};
+
+template <int MODE, int LEN, int R, bool SPEC>
+__global__ void __launch_bounds__(kBlock, LEN >= 8 ? 4 : 5)
+sell_pattern_kernel(PatArgs A, const double *x, const double *aux, double *y) {
+    static_assert(MODE == SPMV || MODE == PROLONG, "slice patterns: SpMV and prolongation only");
+    pdl_prologue();
+    const int lane = threadIdx.x & 31;
+    int32_t row[R], bs[R], cc[R][LEN];
+    unsigned id[R];
+    bool in[R];
+    double vv[R][LEN], xx[R][LEN], av[R];
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        row[r] = A.first_row + ((int32_t)blockIdx.x * R + r) * kBlock + (int32_t)threadIdx.x;
+        in[r] = row[r] < A.row_end;                           // warp-uniform except in the last slice
+        bs[r] = in[r] ? __ldg(A.base + (row[r] >> 5)) : 0;
+        id[r] = in[r] ? ld_const_u16(A.rec + (row[r] >> 5)) : 0u;
+    }
+    int spec[R];
+    if (SPEC) {
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            spec[r] = A.spec_id[0];
+#pragma unroll
+            for (int k = 1; k < kPatBlocks; ++k) spec[r] = row[r] >= A.spec_row[k] ? A.spec_id[k] : spec[r];
+#pragma unroll
+            for (int j = 0; j < LEN; ++j) cc[r][j] = __ldg(A.delta + (spec[r] * LEN + j) * kSlice + lane);
+        }
+    }
+#pragma unroll
+    for (int r = 0; r < R; ++r) av[r] = (MODE == PROLONG && in[r] && row[r] >= A.row_begin) ? aux[row[r]] : 0.0;
+    if (SPEC) {
+        // speculative gathers: exact for slices of the expected record, clamped into the vector for any other
+#pragma unroll
+        for (int r = 0; r < R; ++r)
+            if (in[r]) {
+#pragma unroll
+                for (int j = 0; j < LEN; ++j)
+                    xx[r][j] = ld_gather(x, (int32_t)min((uint32_t)(bs[r] + cc[r][j]), A.col_max));
+            }
+    }
+    bool redo[R];
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        redo[r] = in[r] && (!SPEC || id[r] != (unsigned)spec[r]);
+        if (!in[r]) continue;
+        if (SPEC && !redo[r]) {
+#pragma unroll
+            for (int j = 0; j < LEN; ++j) vv[r][j] = __ldg(A.pvals + (spec[r] * LEN + j) * kSlice + lane);
+        } else if (id[r] == (unsigned)kRecIrregular) {        // warp-uniform
+            const int64_t ent = (int64_t)(row[r] >> 5) * (kSlice * LEN) + lane;
+#pragma unroll
+            for (int j = 0; j < LEN; ++j) {
+                cc[r][j] = ld_stream(A.cols + ent + j * kSlice);
+                vv[r][j] = ld_stream(A.vals + ent + j * kSlice);
+            }
+        } else {
+            const int o = (int)id[r] * LEN * kSlice + lane;
+#pragma unroll
+            for (int j = 0; j < LEN; ++j) {
+                cc[r][j] = bs[r] + __ldg(A.delta + o + j * kSlice);
+                vv[r][j] = __ldg(A.pvals + o + j * kSlice);
+            }
+        }
+    }
+#pragma unroll
+    for (int r = 0; r < R; ++r)
+        if (redo[r]) {
+#pragma unroll
+            for (int j = 0; j < LEN; ++j) xx[r][j] = ld_gather(x, cc[r][j]);
+        }
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        if (!in[r] || row[r] < A.row_begin) continue;
+        double sum = 0.0;
+#pragma unroll
+        for (int j = 0; j < LEN; ++j) sum = mul_add_unfused(sum, vv[r][j], xx[r][j]);
+        y[row[r]] = MODE == PROLONG ? __dadd_rn(av[r], sum) : sum;
+    }
+}
+
 // The same kernel carrying an exchange site (multi-GPU, csrc/comm.cu): the first npeers*ctas_per_peer CTAs push the
 // boundary values the previous kernel produced, poll for the peers' packets and unpack them into the halo of x; the
 // compute CTAs whose slice reads halo columns (mask) wait for that, all others start at once.  The exchange latency
@@ -671,6 +782,69 @@ extern int g_value_dict;            // use the value dictionaries of matrices th
 extern int g_implied_values;        // use the value records of matrices that carry them (on top of the two above)
 extern int g_short_rows_per_thread; // rows per thread of sell_short_kernel (1 = off, 2 or 4)
 extern int64_t g_short_min_rows;    // ... for launches of at least this many rows
+extern int g_implied_transfers;     // use the slice patterns of matrices that carry them (sell_pattern_kernel)
+
+inline bool sell_use_patterns(const mg_sell *A, int64_t row0, int64_t row1) {
+    const int64_t ml = A->max_slice_len;
+    return g_implied_transfers && A->d_slice_rec && A->d_rec_table && A->d_rec_vals && A->nrec < 0 &&
+           A->uniform_len == ml && ml >= 1 && ml <= 8 && row1 - row0 >= g_implied_min_rows;
+}
+
+template <int MODE>
+int launch_sell_pattern(const mg_sell *A, const double *x, const double *aux, double *y, int64_t row0, int64_t row1,
+                        cudaStream_t st, const char *name, int *nblocks_out) {
+    const int L = (int)A->max_slice_len;
+    PatArgs a;
+    a.rec = A->d_slice_rec;
+    a.delta = A->d_rec_table;
+    a.base = A->d_rec_table + (int64_t)(-A->nrec) * L * kSlice;   // the table holds the bases behind the patterns
+    a.pvals = A->d_rec_vals;
+    a.cols = A->d_cols;
+    a.vals = A->d_vals;
+    // the expected record of each row block (mg_sell.h_spec_*; without hints record 0, the most frequent one) and how
+    // many of the block's slices use it (per mille): the launch speculates when every block it touches is mostly one
+    // record
+    for (int k = 0; k < kPatBlocks; ++k) {
+        a.spec_row[k] = k == 0 ? 0 : INT32_MAX;
+        a.spec_id[k] = 0;
+    }
+    bool spec = false;
+    if (A->h_spec_row && A->h_spec_rec && A->n_spec > 0) {
+        spec = true;
+        for (int k = 0; k < A->n_spec; ++k) {
+            if (k < kPatBlocks) {
+                a.spec_row[k] = k == 0 ? 0 : (int32_t)A->h_spec_row[k];
+                a.spec_id[k] = A->h_spec_rec[9 * k];
+            }
+            if (A->h_spec_row[k] < row1 && A->h_spec_row[k + 1] > row0 && A->h_spec_rec[9 * k + 1] < 500) spec = false;
+        }
+    }
+    a.row_begin = (int32_t)row0;
+    a.row_end = (int32_t)row1;
+    a.first_row = (int32_t)(row0 & ~(int64_t)(kSlice - 1));
+    a.col_max = (uint32_t)(A->ncols > 0 ? A->ncols - 1 : 0);
+    const int R = L <= 2 ? 2 : 1;
+    const unsigned grid = (unsigned)(((row1 - a.first_row + kBlock - 1) / kBlock + R - 1) / R);
+#define MG_PAT(LL, RR)                                                                                          \
+    do {                                                                                                        \
+        if (spec) launch_k(sell_pattern_kernel<MODE, LL, RR, true>, grid, kBlock, st, a, x, aux, y);            \
+        else launch_k(sell_pattern_kernel<MODE, LL, RR, false>, grid, kBlock, st, a, x, aux, y);                \
+    } while (0)
+    switch (L) {
+        case 1: MG_PAT(1, 2); break;
+        case 2: MG_PAT(2, 2); break;
+        case 3: MG_PAT(3, 1); break;
+        case 4: MG_PAT(4, 1); break;
+        case 5: MG_PAT(5, 1); break;
+        case 6: MG_PAT(6, 1); break;
+        case 7: MG_PAT(7, 1); break;
+        default: MG_PAT(8, 1); break;
+    }
+#undef MG_PAT
+    MG_CHECK_LAUNCH(name);
+    if (nblocks_out) *nblocks_out = (int)grid;
+    return MG_OK;
+}
 
 template <int MODE>
 int launch_sell_tma(const mg_sell *M, int64_t max_len, const double *x, const double *b, const double *aux, double *y,
@@ -778,6 +952,9 @@ static int launch_sell(const mg_sell *A, const double *x, const double *b, const
                 return rc;
             }
         }
+    }
+    if constexpr (MODE == SPMV || MODE == PROLONG) {
+        if (!fuse && sell_use_patterns(A, row0, row1)) return launch_sell_pattern<MODE>(A, x, aux, y, row0, row1, st, name, nblocks_out);
     }
     SellArgs a = sell_args(A, row0, row1, r_out);
     if (sell_use_implied(A, row0, row1)) sell_pick_spec(A, row0, a);

@@ -17,6 +17,7 @@ int g_implied_columns = 1;
 int64_t g_implied_min_rows = 1 << 19;
 int g_value_dict = 1;                // value dictionaries (valdict.cu) are used where a matrix carries one
 int g_implied_values = 1;            // value records (sell_core.cuh, IMPV) are used where a matrix carries them
+int g_implied_transfers = 1;         // slice patterns (sell_core.cuh, sell_pattern_kernel) where a matrix carries them
 // rows of one or two entries (linear transfers): R rows per thread on large launches (sell_short_kernel)
 int g_short_rows_per_thread = 2;
 int64_t g_short_min_rows = 1 << 18;
@@ -248,6 +249,11 @@ int mg_level_inspect(const mg_sell *A, int ncolors, const int64_t *d_color_ptr, 
 int mg_set_implied_columns(int enabled) {
     const int prev = g_implied_columns;
     g_implied_columns = enabled ? 1 : 0;
+    return prev;
+}
+int mg_set_implied_transfers(int enabled) {
+    const int prev = g_implied_transfers;
+    if (enabled >= 0) g_implied_transfers = enabled ? 1 : 0;
     return prev;
 }
 int64_t mg_set_implied_min_rows(int64_t rows) {

@@ -44,6 +44,7 @@ class DeviceSell:
                                    self.max_len, self.uniform_len)
         self._attach_value_dict()
         self._attach_slice_offsets()
+        self._attach_patterns()
 
     VALUE_DICT_MIN_ROWS = 1 << 16      # smaller matrices are latency-bound launches: a dictionary buys nothing there
 
@@ -115,6 +116,71 @@ class DeviceSell:
             self.struct.d_rec_vals = self.rec_vals.data_ptr()
         self.set_spec_blocks([0, self.shape[0]])
 
+    PATTERN_SAMPLE = 4096        # slices looked at first: a matrix whose sample shares few patterns is skipped
+
+    def _attach_patterns(self):
+        """Implied transfer columns (sell_core.cuh, sell_pattern_kernel): for a rectangular uniform matrix with <= 8
+        entries per row -- a transfer operator, whose columns live in the other level's numbering -- a record id and a
+        base column (the slice's first stored column) per slice; the records (formats.pattern_records) hold the columns
+        relative to the base and the values of the slice's 32 rows.  They sit in the fields of the implied columns,
+        which a transfer operator does not use, flagged by nrec < 0; the bases follow the patterns in d_rec_table
+        (include/mgb200.h).  Kept when at least half of the slices have a record (structured hierarchies: 98-99.99 %);
+        an evenly spaced sample of slices is deduplicated first, so that matrices whose slices share nothing
+        (unstructured numberings, the Galerkin levels of variable coefficients) cost only that.
+        MGB_IMPLIED_TRANSFERS=0 switches it off."""
+        self.pat_rec = self.pat_table = self.pat_vals = None
+        self.pattern_slices = 0
+        floor = int(os.environ.get("MGB_IMPLIED_MIN_ROWS", self.IMPLIED_MIN_ROWS))
+        L = self.uniform_len
+        if (os.environ.get("MGB_IMPLIED_TRANSFERS", "1") == "0" or self.slice_rec is not None
+                or self.shape[0] == self.shape[1] or not 1 <= L <= 8 or self.shape[0] < max(floor, 1)):
+            return
+        import torch
+        nsl = (self.shape[0] + 31) // 32
+        if nsl > 2 * self.PATTERN_SAMPLE:
+            pick = torch.linspace(0, nsl - 2, self.PATTERN_SAMPLE, device=self.cols.device).long()
+            sc = self.cols.view(nsl, 32 * L)[pick].reshape(-1)
+            sv = self.vals.view(nsl, 32 * L)[pick].reshape(-1)
+            *_, nreg = F.pattern_records(torch, sc, sv, self.PATTERN_SAMPLE * 32, L)
+            if 2 * nreg < self.PATTERN_SAMPLE:
+                return
+        base, ids, delta, pvals, nreg = F.pattern_records(torch, self.cols, self.vals, self.shape[0], L)
+        if 2 * nreg < nsl:
+            return
+        self.pat_rec, self.pat_vals = ids, pvals
+        self.pat_table = torch.cat([delta.reshape(-1), base])           # patterns, then the base of every slice
+        self.pattern_slices = nreg
+        s = self.struct
+        s.d_slice_rec, s.d_rec_table, s.d_rec_vals = ids.data_ptr(), self.pat_table.data_ptr(), pvals.data_ptr()
+        s.nrec = -int(delta.shape[0])
+        self.set_pattern_blocks([0, self.shape[0]])
+
+    def set_pattern_blocks(self, row_ptr):
+        """Tell the launcher which pattern the slices of each row block [row_ptr[k], row_ptr[k+1]) mostly use (the
+        colour blocks of the level the rows belong to) and how many of them do: where that is most, a launch gathers
+        with it before the slice's own id has arrived (mg_sell.h_spec_*; the kernel knows 8 blocks, later rows count to
+        the eighth)."""
+        if self.pat_rec is None:
+            return
+        import torch
+        row_ptr = [int(v) for v in row_ptr]
+        if len(row_ptr) > 9:
+            row_ptr = row_ptr[:8] + row_ptr[-1:]
+        nb = len(row_ptr) - 1
+        rows = (ctypes.c_int64 * (nb + 1))(*row_ptr)
+        rec = (ctypes.c_int32 * (9 * max(nb, 1)))()
+        for k in range(nb):
+            ids = self.pat_rec[row_ptr[k] // 32:max((row_ptr[k + 1] + 31) // 32, row_ptr[k] // 32 + 1)]
+            n = ids.numel()
+            ids = ids[ids >= 0]
+            cnt = torch.bincount(ids.long(), minlength=1) if ids.numel() else torch.zeros(1, dtype=torch.int64)
+            rec[9 * k] = int(cnt.argmax().item())
+            rec[9 * k + 1] = int(1000 * int(cnt.max().item()) // max(n, 1))
+        self._spec_keep = (rows, rec)
+        self.struct.n_spec = nb
+        self.struct.h_spec_row = ctypes.cast(rows, ctypes.POINTER(ctypes.c_int64))
+        self.struct.h_spec_rec = ctypes.cast(rec, ctypes.POINTER(ctypes.c_int32))
+
     @property
     def slice_off(self):
         """per-slice offset records [nslices][8] rebuilt from ids + table (tests; None without implied columns)"""
@@ -172,6 +238,7 @@ class DeviceSell:
                                    self.uniform_len)
         self._attach_value_dict()
         self._attach_slice_offsets()
+        self._attach_patterns()
         return self
 
     def bytes(self):
@@ -179,8 +246,13 @@ class DeviceSell:
 
     def stream_bytes(self):
         """bytes one pass over the matrix actually reads: values, and columns or -- for regular slices of a matrix with
-        implied columns (large launches) -- 4 bytes of offset per slice and entry index"""
+        implied columns (large launches) -- 4 bytes of offset per slice and entry index; with slice patterns the id
+        and base column of every slice and the columns and values of the slices without a record"""
         nsl = (self.shape[0] + 31) // 32
+        if self.pat_rec is not None and _lib.load().mg_set_implied_transfers(-1):
+            # slice patterns (as the library is switched now): an id and a base column per slice; slices without a
+            # record read their columns and values (8 B each)
+            return (nsl - self.pattern_slices) * 32 * self.uniform_len * 12 + 6 * nsl
         vbytes = 1 if (self.val_idx is not None and os.environ.get("MGB_VALUE_DICT", "1") != "0") else 8
         if self.slice_rec is None or self.shape[0] < self.IMPLIED_MIN_ROWS or nsl == 0:
             return self.padded * (4 + vbytes) + (0 if self.uniform_len else self.slice_ptr.numel() * 8)
@@ -355,6 +427,9 @@ class DeviceHierarchy:
         every row has a non-zero diagonal.  Levels whose flags were already set by the builder (partitioned levels:
         the facts must hold for the GLOBAL operator, distributed.py) only get their diagonal here."""
         torch, dev = self.torch, self.device
+        for lev, nxt in zip(self.levels[:-1], self.levels[1:]):
+            if getattr(lev, "QT", None) is not None and getattr(nxt, "color_ptr", None) is not None:
+                lev.QT.set_pattern_blocks(nxt.color_ptr)
         flag = torch.zeros(1, dtype=torch.int32, device=dev)
         st = _lib.stream_handle(torch)
         for lev in self.levels:
@@ -362,6 +437,8 @@ class DeviceHierarchy:
                 continue
             lev.diag = torch.empty(lev.n, dtype=torch.float64, device=dev)
             lev.A.set_spec_blocks(lev.color_ptr)          # launches run over colour blocks: one offset record each
+            if getattr(lev, "Q", None) is not None:
+                lev.Q.set_pattern_blocks(lev.color_ptr)       # Q's rows are this level's, Q^T's the next level's
             have = getattr(lev, "flags", None) is not None
             cp = torch.tensor([int(v) for v in lev.color_ptr], dtype=torch.int64, device=dev)
             flag.zero_()

@@ -280,6 +280,75 @@ def sell_slice_offsets(sell, nrows, length):
     return off
 
 
+def sell_slice_patterns(sell, nrows, length):
+    """Slice patterns of a UNIFORM SELL-32 matrix (every slice `length` entries per row): base[s] = the column of entry 0
+    of lane 0, delta[s, j, lane] = column - base[s] and vals[s, j, lane] the values, so that entry j of row 32 s + lane
+    has column base[s] + delta[s, j, lane].  Unlike sell_slice_offsets this holds for every slice, whichever index space
+    the columns live in (transfer operators: another level's colour-blocked numbering); what makes a slice cheap is that
+    many slices share one (delta, vals) pattern.  full[s] = the slice holds no row beyond the matrix.  Host twin of
+    pattern_records (which deduplicates the patterns on any torch device)."""
+    slice_ptr, cols, vals = sell
+    nsl = len(slice_ptr) - 1
+    c = np.asarray(cols, dtype=np.int64).reshape(nsl, length, SLICE)          # [slice][entry][lane]
+    base = c[:, 0, 0].copy() if nsl else np.zeros(0, dtype=np.int64)
+    delta = c - base[:, None, None]
+    full = (np.arange(nsl) + 1) * SLICE <= nrows
+    return base, delta, np.asarray(vals, dtype=np.float64).reshape(nsl, length, SLICE), full
+
+
+def pattern_records(torch, cols, vals, nrows, length, max_records=256, min_slices=2, chunk=1 << 16):
+    """Deduplicated slice patterns of a uniform SELL-32 matrix with `length` <= 8 entries per row (engine.DeviceSell;
+    sell_core.cuh, sell_pattern_kernel).  A slice keeps a 32-bit base column and a 16-bit record id; record r holds
+    delta[r][j][lane] (int32) and vals[r][j][lane] (float64), and entry j of lane `lane` of the slice has the column
+    base + delta and exactly that value (sell_slice_patterns defines base and delta).  Records are ranked by how many
+    slices use them; at most `max_records` of those used by at least `min_slices` slices are kept (the table stays
+    L1-sized), every other slice -- and a slice with rows beyond the matrix -- gets id -1 (0xffff to the kernels) and
+    keeps reading its columns and values.
+
+    Two 62-bit sums of the slice's pattern with fixed weights group the slices; each slice is then compared with the
+    first slice of its group, entry by entry, so a hash collision only costs a slice its record, never a wrong column.
+    Pure tensor code (any device): the CPU suite runs it on host tensors against sell_slice_patterns.
+    Returns (base int32 [nslices], ids int16 [nslices], delta int32 [nrec, length, 32], vals f64 [nrec, length, 32],
+    slices with a record)."""
+    dev = cols.device
+    nsl = int(cols.numel()) // (32 * length)
+    K = 32 * length
+    c = cols.view(nsl, K)
+    base = c[:, 0].contiguous()
+    vbits = vals.view(nsl, K).view(torch.int64)
+    gen = torch.Generator().manual_seed(20251)
+    w = torch.randint(1, 1 << 20, (2, 3, K), generator=gen, dtype=torch.int64).to(dev)
+
+    def pattern(s):               # [n, 3K] int64 of the slices s (a range or an index tensor), elements in [-2^32, 2^32)
+        d = c[s].to(torch.int64) - base[s].to(torch.int64)[:, None]
+        v = vbits[s]
+        return torch.cat([d, v >> 32, v & 0xffffffff], dim=1)
+
+    keys = torch.empty(nsl, 2, dtype=torch.int64, device=dev)
+    for s0 in range(0, nsl, chunk):      # |element| < 2^33, weight < 2^20, 3K <= 768 terms: no int64 overflow
+        s = slice(s0, min(s0 + chunk, nsl))
+        p = pattern(s)
+        keys[s, 0] = (p * w[0].reshape(1, -1)).sum(dim=1)
+        keys[s, 1] = (p * w[1].reshape(1, -1)).sum(dim=1)
+    _, inverse, counts = torch.unique(keys, dim=0, return_inverse=True, return_counts=True)
+    first = torch.full((counts.numel(),), nsl, dtype=torch.int64, device=dev)
+    first.scatter_reduce_(0, inverse, torch.arange(nsl, device=dev), reduce="amin")
+    ok = (torch.arange(nsl, device=dev) + 1) * 32 <= nrows
+    for s0 in range(0, nsl, chunk):      # exact check against the group's first slice
+        s = slice(s0, min(s0 + chunk, nsl))
+        ok[s] &= (pattern(s) == pattern(first[inverse[s]])).all(dim=1)
+    counts = torch.bincount(inverse[ok], minlength=counts.numel())
+    order = torch.argsort(counts, descending=True, stable=True)
+    order = order[counts[order] >= min_slices][:max_records]
+    rank_of = torch.full((counts.numel(),), -1, dtype=torch.int64, device=dev)
+    rank_of[order] = torch.arange(order.numel(), device=dev)
+    ids = torch.where(ok, rank_of[inverse], torch.full_like(inverse, -1)).to(torch.int16)
+    rep = first[order]
+    delta = (c[rep].to(torch.int64) - base[rep, None].to(torch.int64)).to(torch.int32).view(-1, length, 32).contiguous()
+    rvals = vals.view(nsl, K)[rep].view(-1, length, 32).contiguous()
+    return base.to(torch.int32), ids, delta, rvals, int((ids >= 0).sum().item())
+
+
 def slice_records(torch, off, val_idx=None, val_table=None, uniform_len=0, max_records=32766):
     """Deduplicated slice records of a uniform SELL-32 matrix (engine.DeviceSell; sell_core.cuh IMPL / IMPV kernels).
 

@@ -189,6 +189,15 @@ int64_t mg_set_wide_max_rows(int64_t rows);
 /* x_out = x + omega*(dinv*(b - A x)) */
 int mg_sell_jacobi(const mg_sell *A, const double *d_dinv, const double *d_x, const double *d_b,
                    double *d_x_out, double omega, void *stream);
+/* One step of the Chebyshev smoother (all rows): t = dinv*(b - A x) with the residual in storage order,
+ * dn = c_r*t (first != 0: step 0, d only written) or dn = (c_d*d) + (c_r*t) (first == 0, c_d != 0), then
+ * x_out = x + dn and d = dn (in place); every product and sum rounded on its own.  x_out must not alias x. */
+int mg_sell_chebyshev(const mg_sell *A, const double *d_dinv, const double *d_x, const double *d_b, double *d_d,
+                      double *d_x_out, double c_d, double c_r, int first, void *stream);
+/* Step 0 of the Chebyshev smoother on a zero iterate without the matrix: d = c_r*(dinv*b), x_out = 0 + d over n
+ * entries -- the bits of mg_sell_chebyshev(first = 1) with x = 0. */
+int mg_chebyshev_zero_first(int64_t n, double c_r, const double *d_dinv, const double *d_b, double *d_d,
+                            double *d_x_out, void *stream);
 /* Gauss-Seidel update of the rows [row0,row1) in place (one colour of a colour-blocked ordering). */
 int mg_sell_gs_rows(const mg_sell *A, double *d_x, const double *d_b, int64_t row0, int64_t row1,
                     void *stream);
@@ -557,7 +566,7 @@ int64_t mg_host_lex_levels(int64_t n, const int32_t *h_indptr, const int32_t *h_
 
 /* ------------------------------------------------------------------------------------------------ */
 /* The V-cycle (Multigrid.v_cycle, Multigrid.py:77-124) over a prebuilt hierarchy.                   */
-enum { MG_SMOOTH_JACOBI = 0, MG_SMOOTH_MCGS = 1, MG_SMOOTH_LEXGS = 2 };
+enum { MG_SMOOTH_JACOBI = 0, MG_SMOOTH_MCGS = 1, MG_SMOOTH_LEXGS = 2, MG_SMOOTH_CHEBY = 3 };
 enum { MG_COARSE_DENSE = 0, MG_COARSE_BCR = 1 };
 
 typedef struct {
@@ -587,6 +596,11 @@ typedef struct {
     uint32_t flags;                       /* MG_LEVEL_*                                                              */
     uint32_t pad_;
     const double *d_diag;                 /* the diagonal as the Gauss-Seidel kernel finds it (0: none); optional    */
+    /* Chebyshev smoother (MG_SMOOTH_CHEBY): the polynomial's degree and a HOST table of cheb_degree pairs
+     * (c_d, c_r), step k at [2k, 2k+1] (c_d of step 0 unused); the step's d lives in d_r                           */
+    int32_t cheb_degree;
+    int32_t pad2_;
+    const double *h_cheb_coef;
 } mg_level;
 /* multicolour Gauss-Seidel only.  PROPER_COLORING: no row has a non-zero entry in the column of ANOTHER row of its own
  * colour.  NONZERO_DIAG: every row has a non-zero diagonal entry (so a colour sweep overwrites every row it visits). */

@@ -18,7 +18,7 @@ c_int = ctypes.c_int
 c_dbl = ctypes.c_double
 c_vp = ctypes.c_void_p
 
-MG_SMOOTH_JACOBI, MG_SMOOTH_MCGS, MG_SMOOTH_LEXGS = 0, 1, 2
+MG_SMOOTH_JACOBI, MG_SMOOTH_MCGS, MG_SMOOTH_LEXGS, MG_SMOOTH_CHEBY = 0, 1, 2, 3
 MG_COARSE_DENSE, MG_COARSE_BCR = 0, 1
 MG_LEVEL_PROPER_COLORING, MG_LEVEL_NONZERO_DIAG = 1, 2
 SLICE_IRREGULAR = -2 ** 31
@@ -94,7 +94,8 @@ class mg_level(ctypes.Structure):
                 ("d_x", c_vp), ("d_b", c_vp), ("d_r", c_vp), ("d_tmp", c_vp),
                 ("coarse_kind", ctypes.c_int32), ("d_coarse_inv", c_vp), ("coarse_bcr", c_vp),
                 ("dist", ctypes.POINTER(mg_dist_level)), ("coarse_bcr_dist", ctypes.POINTER(mg_bcr_dist)),
-                ("flags", ctypes.c_uint32), ("pad_", ctypes.c_uint32), ("d_diag", c_vp)]
+                ("flags", ctypes.c_uint32), ("pad_", ctypes.c_uint32), ("d_diag", c_vp),
+                ("cheb_degree", ctypes.c_int32), ("pad2_", ctypes.c_int32), ("h_cheb_coef", ctypes.POINTER(c_dbl))]
 
 
 class mg_cycle_params(ctypes.Structure):
@@ -153,6 +154,8 @@ _SIGNATURES = {
     "mg_set_wide_min_len": (c_i64, [c_i64]),
     "mg_set_wide_max_rows": (c_i64, [c_i64]),
     "mg_sell_jacobi": (c_int, [ctypes.POINTER(mg_sell), c_vp, c_vp, c_vp, c_vp, c_dbl, c_vp]),
+    "mg_sell_chebyshev": (c_int, [ctypes.POINTER(mg_sell), c_vp, c_vp, c_vp, c_vp, c_vp, c_dbl, c_dbl, c_int, c_vp]),
+    "mg_chebyshev_zero_first": (c_int, [c_i64, c_dbl, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "mg_sell_gs_rows": (c_int, [ctypes.POINTER(mg_sell), c_vp, c_vp, c_i64, c_i64, c_vp]),
     "mg_sell_prolong_correct": (c_int, [ctypes.POINTER(mg_sell), c_vp, c_vp, c_vp, c_vp]),
     "mg_dot": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),

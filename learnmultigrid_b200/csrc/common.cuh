@@ -36,7 +36,9 @@ inline int set_error(int code, const char *what, const char *detail) {
 
 // GS_RES / GS_NORM: colour sweep that also yields the residual / the squared residual norm of the swept rows
 // SPMV_DOT: y = A x and per-CTA partial sums of aux . y (the p . A p of conjugate gradients from the SpMV's registers)
-enum SellMode { SPMV = 0, RESID = 1, RESNORM = 2, JACOBI = 3, GS = 4, PROLONG = 5, GS_RES = 6, GS_NORM = 7, SPMV_DOT = 8 };
+// CHEBY: one step of the Chebyshev smoother (sell_modes_cheby.cu); after PROLONG, so the staged TMA path never sees it
+enum SellMode { SPMV = 0, RESID = 1, RESNORM = 2, JACOBI = 3, GS = 4, PROLONG = 5, GS_RES = 6, GS_NORM = 7, SPMV_DOT = 8,
+                CHEBY = 9 };
 
 constexpr int kSlice = 32;      // SELL slice height = one warp
 constexpr int kBlock = 256;     // threads per CTA of the streaming kernels

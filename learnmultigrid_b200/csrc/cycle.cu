@@ -115,7 +115,7 @@ struct Tail {
 static inline bool level_proper(const mg_level &L) { return g_cycle_fusion && (L.flags & MG_LEVEL_PROPER_COLORING); }
 
 // `steps` smoothing sweeps on level L.  cur points at the buffer holding the iterate and is updated
-// (Jacobi ping-pongs between d_x and d_tmp).  zero_guess: the iterate is known to be exactly zero and the
+// (Jacobi and Chebyshev ping-pong between d_x and d_tmp).  zero_guess: the iterate is known to be exactly zero and the
 // buffer has NOT been initialised.
 static int smooth(mg_comm *comm, const mg_level &L, const mg_cycle_params &P, int steps, double **cur, double **alt,
                   bool zero_guess, bool reverse, cudaStream_t st, Tail *tail = nullptr) {
@@ -141,6 +141,30 @@ static int smooth(mg_comm *comm, const mg_level &L, const mg_cycle_params &P, in
             MG_TRY(halo_all(comm, L, *alt, st));
             double *t = *cur; *cur = *alt; *alt = t;
         }
+        return MG_OK;
+    }
+    if (P.smoother == MG_SMOOTH_CHEBY) {
+        // `steps` applications of the degree-m polynomial, each restarting at step 0; d lives in d_r, which is free
+        // during the pre-smoothing (the residual is formed after it) and the post-smoothing (the restriction has read it)
+        const int deg = L.cheb_degree;
+        if (deg < 1 || !L.h_cheb_coef) return set_error(MG_ERR_INVALID, "mg_vcycle", "level has no Chebyshev coefficients");
+        for (int s = 0; s < steps; ++s)
+            for (int k = 0; k < deg; ++k) {
+                const double c_d = L.h_cheb_coef[2 * k], c_r = L.h_cheb_coef[2 * k + 1];
+                if (s == 0 && k == 0 && zero_guess) {
+                    if (P.zero_guess_skip) {
+                        // x = 0 + c_r (dinv b): the bits of the step on zeros, no matrix pass
+                        MG_TRY(sell_chebyshev_zero_first(L.n, c_r, L.d_dinv, L.d_b, L.d_r, *alt, st));
+                        MG_TRY(halo_all(comm, L, *alt, st));
+                        double *t = *cur; *cur = *alt; *alt = t;
+                        continue;
+                    }
+                    MG_TRY(vec_fill(vec_len(L), 0.0, *cur, st));
+                }
+                MG_TRY(sell_chebyshev(&L.A, L.d_dinv, *cur, L.d_b, L.d_r, *alt, c_d, c_r, k == 0, st));
+                MG_TRY(halo_all(comm, L, *alt, st));
+                double *t = *cur; *cur = *alt; *alt = t;
+            }
         return MG_OK;
     }
     if (P.smoother == MG_SMOOTH_MCGS) {
@@ -215,14 +239,16 @@ static int vcycle_rec(mg_comm *comm, const mg_level *levels, int nlevels, int l,
     }
     const mg_level &C = levels[l + 1];
     const bool jac = P.smoother == MG_SMOOTH_JACOBI;
+    const bool cheb = P.smoother == MG_SMOOTH_CHEBY;
     const bool mcgs = P.smoother == MG_SMOOTH_MCGS;
     const bool zero_guess = l > 0 || P.x0_zero != 0;
     double *cur = L.d_x, *alt = L.d_tmp;
     bool prolong_flip = false;
-    if (jac) {
-        // Jacobi flips buffers once per sweep.  The result must end in d_x: on coarse levels choose the
-        // start buffer (the zero guess is virtual), on level 0 let the prolongation write out of place.
-        const int flips = P.nu_pre + P.nu_post;
+    if (jac || cheb) {
+        // Jacobi flips buffers once per sweep, Chebyshev once per step (degree steps per sweep).  The result must end
+        // in d_x: on coarse levels choose the start buffer (the zero guess is virtual), on level 0 let the
+        // prolongation write out of place.
+        const int flips = (cheb ? L.cheb_degree : 1) * (P.nu_pre + P.nu_post);
         if (flips & 1) {
             if (zero_guess) { cur = L.d_tmp; alt = L.d_x; }
             else prolong_flip = true;

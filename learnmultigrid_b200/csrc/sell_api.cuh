@@ -24,6 +24,12 @@ int sell_reduce_partials(const double *partials, int64_t n, double *out, cudaStr
 int sell_residual_norm2(const mg_sell *A, const double *x, const double *b, double *partials, double *out, cudaStream_t st);
 int sell_jacobi(const mg_sell *A, const double *dinv, const double *x, const double *b, double *xo, double omega,
                 cudaStream_t st);
+// one Chebyshev step (sell_modes_cheby.cu): x_out = x + dn, d = dn; `first` = step 0 (c_d unused, d only written)
+int sell_chebyshev(const mg_sell *A, const double *dinv, const double *x, const double *b, double *d, double *xo,
+                   double c_d, double c_r, bool first, cudaStream_t st);
+// step 0 on a zero iterate without the matrix: d = c_r (dinv b), x_out = 0 + d over n entries
+int sell_chebyshev_zero_first(int64_t n, double c_r, const double *dinv, const double *b, double *d, double *xo,
+                              cudaStream_t st);
 // Gauss-Seidel on the rows of one colour, in place.  tail: also write the residual of these rows (with their new
 // values) to r_out, or their squared residuals as per-CTA partial sums (*nblocks of them) -- see sell_gs_tail_ok.
 int sell_gs_rows(const mg_sell *A, double *x, const double *b, int64_t row0, int64_t row1, const SellFuse *fuse,

@@ -40,6 +40,20 @@ struct SellArgs {
 __host__ __device__ constexpr bool mode_is_gs(int m) { return m == GS || m == GS_RES || m == GS_NORM; }
 __host__ __device__ constexpr bool mode_has_partials(int m) { return m == RESNORM || m == GS_NORM || m == SPMV_DOT; }
 __host__ __device__ constexpr bool mode_is_tail(int m) { return m == GS_RES || m == GS_NORM; }
+// modes whose epilogue reads the row's own old iterate and 1/diag (aux): damped Jacobi, Chebyshev
+__host__ __device__ constexpr bool mode_is_jacobi_like(int m) { return m == JACOBI || m == CHEBY; }
+
+// CHEBY: x_out = x + dn, d = dn with dn = c_r (dinv (b - A x)) on step 0 and (c_d d) + (c_r (dinv (b - A x))) after it,
+// every product and sum rounded on its own.  The launch carries c_r in `omega`, d in SellArgs::r_out and c_d's bit
+// pattern in the `partials` slot (zero bits: step 0, d is written but not read), so that the parameter block of every
+// other mode stays as it is.
+__device__ __forceinline__ double cheby_dn(double cd, bool has_d, double dv, double cr, double t) {
+    const double rt = __dmul_rn(cr, t);
+    return has_d ? __dadd_rn(__dmul_rn(cd, dv), rt) : rt;
+}
+__device__ __forceinline__ double cheby_cd(const double *slot) {
+    return __longlong_as_double((long long)(uintptr_t)slot);
+}
 
 // ---- implied columns ------------------------------------------------------------------------------------------------
 // On a structured stencil level nearly every slice is REGULAR: entry j of every one of its 32 rows has column
@@ -69,6 +83,8 @@ struct SellEp {
     const double *aux;
     double *y;
     double omega;
+    double cd;      // CHEBY: c_d
+    bool has_d;     // CHEBY: not step 0 (d is read)
 };
 
 // One row of at most LEN entries, everything in registers and in straight-line code: all cols/vals loads are issued
@@ -109,20 +125,22 @@ __device__ __forceinline__ void short_row(const SellArgs &A, int64_t ent, int64_
     // gather).  A prefetch holds no register (the sweeps sit at the 32-register limit of full occupancy; loading b early
     // spilled it straight back to local memory), the load at the point of use then hits L1.  PROLONG rows are short and
     // have registers to spare: their u is loaded.
-    constexpr bool kUsesB = MODE == RESID || MODE == RESNORM || MODE == JACOBI || mode_is_gs(MODE);
-    constexpr bool kUsesAux = MODE == JACOBI || MODE == SPMV_DOT;
+    constexpr bool kUsesB = MODE == RESID || MODE == RESNORM || mode_is_jacobi_like(MODE) || mode_is_gs(MODE);
+    constexpr bool kUsesAux = mode_is_jacobi_like(MODE) || MODE == SPMV_DOT;
     constexpr bool kEarly = kRowOperands == 3;
-    double bv = 0.0, av = 0.0, xr = 0.0;
+    double bv = 0.0, av = 0.0, xr = 0.0, dv = 0.0;
     if (active) {
         if (MODE == PROLONG) av = E.aux[row];
         if (kEarly) {
             if (kUsesB) bv = E.b[row];
             if (kUsesAux) av = E.aux[row];
-            if (MODE == JACOBI) xr = x[row];
+            if (mode_is_jacobi_like(MODE)) xr = x[row];
+            if (MODE == CHEBY && E.has_d) dv = A.r_out[row];
         } else {
             if (kUsesB) prefetch_row_operand(E.b + row);
             if (kUsesAux) prefetch_row_operand(E.aux + row);
-            if (MODE == JACOBI) prefetch_row_operand(x + row);
+            if (mode_is_jacobi_like(MODE)) prefetch_row_operand(x + row);
+            if (MODE == CHEBY && E.has_d) prefetch_row_operand(A.r_out + row);
         }
     }
     static_assert(!IMPV || (IMPL && VAL8 && !STAB && !PRED), "implied values ride on implied columns and a dictionary");
@@ -238,7 +256,8 @@ __device__ __forceinline__ void short_row(const SellArgs &A, int64_t ent, int64_
         if (!kEarly) {
             if (kUsesB) bv = E.b[row];
             if (kUsesAux) av = E.aux[row];
-            if (MODE == JACOBI) xr = x[row];
+            if (mode_is_jacobi_like(MODE)) xr = x[row];
+            if (MODE == CHEBY && E.has_d) dv = A.r_out[row];
         }
         if (MODE == SPMV) {
             E.y[row] = sum;
@@ -253,6 +272,10 @@ __device__ __forceinline__ void short_row(const SellArgs &A, int64_t ent, int64_
         } else if (MODE == JACOBI) {
             const double r = __dsub_rn(bv, sum);
             E.y[row] = __dadd_rn(xr, __dmul_rn(E.omega, __dmul_rn(av, r)));
+        } else if (MODE == CHEBY) {
+            const double dn = cheby_dn(E.cd, E.has_d, dv, E.omega, __dmul_rn(av, __dsub_rn(bv, sum)));
+            A.r_out[row] = dn;
+            E.y[row] = __dadd_rn(xr, dn);
         } else if (MODE == PROLONG) {
             E.y[row] = __dadd_rn(av, sum);   // aux = u (may alias y)
         } else {                             // Gauss-Seidel family
@@ -374,7 +397,7 @@ sell_body(const SellArgs &A, const double *x, const double *__restrict__ b, cons
         const int32_t *__restrict__ c = A.cols + base + lane;
         if (LEN > 0) {
             constexpr int L = LEN > 0 ? LEN : 1;
-            const SellEp E{b, aux, y, omega};
+            const SellEp E{b, aux, y, omega, MODE == CHEBY ? cheby_cd(partials) : 0.0, MODE == CHEBY && partials != nullptr};
             if (IMPL) {
                 short_row<MODE, L, false, true, VAL8, STAB, IMPV>(A, base + lane, slice, L, x, row, active, E, contrib, hw, fx, out, stab);
             } else if (UNIFORM || len == L) {
@@ -385,10 +408,11 @@ sell_body(const SellArgs &A, const double *x, const double *__restrict__ b, cons
         } else {
             double sum = 0.0, diag = 0.0;
             // the row's own vector entries first (see short_row): not one more round trip behind the last chunk
-            double bv = 0.0, av = 0.0, xr = 0.0;
-            if ((MODE == RESID || MODE == RESNORM || MODE == JACOBI || MODE == GS) && active) bv = b[row];
-            if ((MODE == PROLONG || MODE == JACOBI || MODE == SPMV_DOT) && active) av = aux[row];
-            if (MODE == JACOBI && active) xr = x[row];
+            double bv = 0.0, av = 0.0, xr = 0.0, dv = 0.0;
+            if ((MODE == RESID || MODE == RESNORM || mode_is_jacobi_like(MODE) || MODE == GS) && active) bv = b[row];
+            if ((MODE == PROLONG || mode_is_jacobi_like(MODE) || MODE == SPMV_DOT) && active) av = aux[row];
+            if (mode_is_jacobi_like(MODE) && active) xr = x[row];
+            if (MODE == CHEBY && partials != nullptr && active) dv = A.r_out[row];
             int k = 0;
             for (; k + 4 <= len; k += 4) {
                 row_chunk<MODE, 4>(c + k * kSlice, v + k * kSlice, x, row, sum, diag, hw, fx);
@@ -412,6 +436,11 @@ sell_body(const SellArgs &A, const double *x, const double *__restrict__ b, cons
                 } else if (MODE == JACOBI) {
                     const double r = __dsub_rn(bv, sum);
                     y[row] = __dadd_rn(xr, __dmul_rn(omega, __dmul_rn(av, r)));
+                } else if (MODE == CHEBY) {
+                    const double dn = cheby_dn(cheby_cd(partials), partials != nullptr, dv, omega,
+                                               __dmul_rn(av, __dsub_rn(bv, sum)));
+                    A.r_out[row] = dn;
+                    y[row] = __dadd_rn(xr, dn);
                 } else if (MODE == GS) {
                     if (diag != 0.0) y[row] = __ddiv_rn(__dsub_rn(bv, sum), diag);
                 } else if (MODE == PROLONG) {
@@ -689,7 +718,7 @@ sell_wide_kernel(SellArgs A, int uniform_len, const double *x, const double *__r
     double bv = 0.0, av = 0.0;
     if (finisher) {
         if (MODE != SPMV && MODE != PROLONG && MODE != SPMV_DOT) bv = b[row];
-        if (MODE == JACOBI || MODE == PROLONG || MODE == SPMV_DOT) av = aux[row];
+        if (mode_is_jacobi_like(MODE) || MODE == PROLONG || MODE == SPMV_DOT) av = aux[row];
     }
     const double *__restrict__ v = A.vals + base + lane;
     const int32_t *__restrict__ c = A.cols + base + lane;
@@ -717,8 +746,9 @@ sell_wide_kernel(SellArgs A, int uniform_len, const double *x, const double *__r
             }
         }
     }
-    double xr = 0.0;
-    if (MODE == JACOBI && finisher) xr = x[row];
+    double xr = 0.0, dv = 0.0;
+    if (mode_is_jacobi_like(MODE) && finisher) xr = x[row];
+    if (MODE == CHEBY && finisher && partials != nullptr) dv = A.r_out[row];
     __syncthreads();
     double contrib = 0.0;
     if (finisher) {
@@ -741,6 +771,10 @@ sell_wide_kernel(SellArgs A, int uniform_len, const double *x, const double *__r
         } else if (MODE == JACOBI) {
             const double r = __dsub_rn(bv, sum);
             y[row] = __dadd_rn(xr, __dmul_rn(omega, __dmul_rn(av, r)));
+        } else if (MODE == CHEBY) {
+            const double dn = cheby_dn(cheby_cd(partials), partials != nullptr, dv, omega, __dmul_rn(av, __dsub_rn(bv, sum)));
+            A.r_out[row] = dn;
+            y[row] = __dadd_rn(xr, dn);
         } else if (MODE == PROLONG) {
             y[row] = __dadd_rn(av, sum);
         } else {                       // Gauss-Seidel family, see short_row

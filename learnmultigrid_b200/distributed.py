@@ -196,20 +196,22 @@ class DistributedHierarchy(DeviceHierarchy):
 
     def __init__(self, A, Q_list, fabric, smoother="jacobi", colors=None, device=None, min_rows_per_rank=65536,
                  n_dist=None, dense_coarse_max=DENSE_COARSE_MAX, keep_host=False, region_bytes=16 << 20,
-                 max_sites=512, timeout_s=10.0, split_coarse_solve=True, bcr_split_min_blocks=32):
+                 max_sites=512, timeout_s=10.0, split_coarse_solve=True, bcr_split_min_blocks=32, cheby_degree=2,
+                 cheby_bounds=None):
         torch = _lib.require_cuda()
         self.split_coarse_solve = bool(split_coarse_solve)
         self.bcr_split_min_blocks = int(bcr_split_min_blocks)
         self.torch = torch
         self.lib = _lib.load()
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        if smoother not in ("jacobi", "mcgs"):
-            raise ValueError("partitioned levels support 'jacobi' and 'mcgs' (index-order Gauss-Seidel is serial "
-                             "across row blocks)")
+        if smoother not in ("jacobi", "mcgs", "chebyshev"):
+            raise ValueError("partitioned levels support 'jacobi', 'mcgs' and 'chebyshev' (index-order Gauss-Seidel is "
+                             "serial across row blocks)")
         self.smoother = smoother
         self.nlevels = len(Q_list) + 1
         if self.nlevels < 2:
             raise ValueError("need at least one transfer operator (levels >= 2)")
+        self._chebyshev_args(cheby_degree, cheby_bounds)
         self.fabric = fabric
         self.rank, self.world = fabric.rank, fabric.world
         self.keep_host = keep_host
@@ -290,6 +292,8 @@ class DistributedHierarchy(DeviceHierarchy):
         self._setup = S
         L = self.nlevels
         A_host0, A_nat, Q_nat, QT_nat = SD.build_natural(S, A, Q_list)
+        if self.smoother == "chebyshev":
+            self._chebyshev_setup(S, A_nat)      # from the GLOBAL operators: the same bounds on every rank
         ns = [a.shape[0] for a in A_nat]
         self._global_n = ns
         self._global_nnzA = [a.nnz for a in A_nat]
@@ -567,7 +571,7 @@ class DistributedHierarchy(DeviceHierarchy):
             self.last_launches = int(self.lib.mg_last_launch_count())
             return
         key = (L, params.smoother, params.nu_pre, params.nu_post, params.omega, params.zero_guess_skip,
-               params.reverse_post, params.x0_zero, bool(with_norm), bool(norm_after), bool(dry))
+               params.reverse_post, params.x0_zero, bool(with_norm), bool(norm_after), bool(dry), self._cheby_key)
         g = self._graphs.get(key)
         if g is None:
             cap = torch.cuda.Stream(device=self.device)

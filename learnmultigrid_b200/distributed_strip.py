@@ -63,6 +63,9 @@ class StripHierarchy(DistributedHierarchy):
     def __init__(self, A_blk, Q_blks, offsets, fabric, n_dist, smoother="jacobi", colors=None, device=None,
                  dense_coarse_max=DENSE_COARSE_MAX, region_bytes=16 << 20, max_sites=512, timeout_s=10.0,
                  split_coarse_solve=True, bcr_split_min_blocks=32, device_products=True):
+        if smoother == "chebyshev":
+            raise ValueError("StripHierarchy supports 'jacobi' and 'mcgs'; the Chebyshev smoother needs the global "
+                             "operators for its bounds (use DistributedHierarchy)")
         self._strip_inputs = (A_blk, list(Q_blks), [np.asarray(o, dtype=np.int64) for o in offsets])
         self._device_products = bool(device_products)
         super().__init__(None, [None] * len(Q_blks), fabric, smoother=smoother, colors=colors, device=device,

@@ -278,22 +278,27 @@ class DeviceHierarchy:
     A        : fine operator (anything SciPy accepts), n0 x n0
     Q_list   : transfer operators [Q_0 (n0 x n1), Q_1, ...]; levels = len(Q_list) + 1
     smoother : "jacobi" | "mcgs" (multicolour Gauss-Seidel) | "lexgs" (exact index-order Gauss-Seidel)
+               | "chebyshev" (Chebyshev polynomial in D^-1 A; natural order, no colouring, like "jacobi")
     colors   : optional list of per-level colour arrays for "mcgs" (default: first-fit greedy colouring)
+    cheby_degree : degree of the Chebyshev polynomial (steps per smoothing sweep)
+    cheby_bounds : None (default: [0.3, 1.1] x a 10-step Lanczos estimate of lambda_max(D^-1 A) per level) or one
+                   (lo, hi) pair per smoothing level (levels - 1 of them)
     setup    : "device" (SpGEMM / transposes / SELL build by CUDA kernels) or "host" (NumPy/SciPy cross-check)
     """
 
     def __init__(self, A, Q_list, smoother="jacobi", colors=None, device=None, setup="device",
-                 dense_coarse_max=DENSE_COARSE_MAX, keep_host=True):
+                 dense_coarse_max=DENSE_COARSE_MAX, keep_host=True, cheby_degree=2, cheby_bounds=None):
         torch = _lib.require_cuda()
         self.torch = torch
         self.lib = _lib.load()
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        if smoother not in ("jacobi", "mcgs", "lexgs"):
+        if smoother not in ("jacobi", "mcgs", "lexgs", "chebyshev"):
             raise ValueError("unknown smoother %r" % (smoother,))
         self.smoother = smoother
         self.nlevels = len(Q_list) + 1
         if self.nlevels < 2:
             raise ValueError("need at least one transfer operator (levels >= 2)")
+        self._chebyshev_args(cheby_degree, cheby_bounds)
         self.keep_host = keep_host
         self._graphs = {}
         self._keep = []          # tensors / ctypes buffers that must outlive the level structs
@@ -307,11 +312,44 @@ class DeviceHierarchy:
         self._finish_structs()
 
     # ------------------------------------------------------------------------------------------------
+    def _chebyshev_args(self, degree, bounds):
+        """validate the Chebyshev options (ValueError) before anything is built"""
+        self.cheby_degree = self.cheby_bounds = self.cheby_coefficients = self.cheby_lambda = None
+        self._cheby_key = None
+        if self.smoother != "chebyshev":
+            return
+        if bounds is not None:
+            bounds = [tuple(float(v) for v in b) for b in bounds]
+            if len(bounds) != self.nlevels - 1 or any(len(b) != 2 for b in bounds):
+                raise ValueError("cheby_bounds needs one (lo, hi) pair per smoothing level (%d)" % (self.nlevels - 1))
+        F.chebyshev_check(degree, bounds)
+        self.cheby_degree = int(degree)
+        self.cheby_bounds = bounds
+
+    def _chebyshev_setup(self, S, A_nat):
+        """Bounds and coefficient tables of the Chebyshev smoother, from the levels' operators in natural order (DevCSR,
+        the GLOBAL operators on a partitioned hierarchy: every rank computes the same bits).  Given bounds are kept;
+        otherwise [0.3, 1.1] x the Lanczos estimate of lambda_max(D^-1 A_l) (setup_device.chebyshev_lambda_max)."""
+        if self.cheby_bounds is None:
+            self.cheby_lambda = [SD.chebyshev_lambda_max(S, A_nat[l]) for l in range(self.nlevels - 1)]
+            lo, hi = F.CHEBY_INTERVAL
+            self.cheby_bounds = [(lo * lam, hi * lam) for lam in self.cheby_lambda]
+        self.cheby_coefficients = [F.chebyshev_coefficients(lo, hi, self.cheby_degree) for lo, hi in self.cheby_bounds]
+        # part of every graph key: a table the captured launches were not made with never replays them
+        self._cheby_key = tuple(c.tobytes() for c in self.cheby_coefficients)
+
     def _setup_host(self, A, Q_list, colors, dense_coarse_max):
         """Hierarchy build with SciPy/NumPy on the host (formats.build_host_hierarchy), then upload."""
         torch, dev = self.torch, self.device
         L = self.nlevels
         host = F.build_host_hierarchy(A, Q_list, self.smoother, colors, with_sell=True)
+        if self.smoother == "chebyshev":
+            S = SD.DeviceSetup(torch, dev)
+            up = [SD.DevCSR(d["A_nat"].shape, *(torch.from_numpy(np.ascontiguousarray(a, dtype=t)).to(dev) for a, t in
+                                                  ((d["A_nat"].indptr, np.int32), (d["A_nat"].indices, np.int32),
+                                                   (d["A_nat"].data, np.float64)))) for d in host[:-1]]
+            self._chebyshev_setup(S, up)
+            del up
         self.host_A = [d["A_nat"] for d in host] if self.keep_host else None
         self.host_Q = [d.get("Q_nat") for d in host[:-1]] if self.keep_host else None
         self.colors = [d["colors"] for d in host]
@@ -406,6 +444,12 @@ class DeviceHierarchy:
                     s.flags = int(getattr(lev, "flags", 0))
                     if getattr(lev, "diag", None) is not None:
                         s.d_diag = lev.diag.data_ptr()
+                if self.cheby_coefficients is not None:
+                    tab = np.ascontiguousarray(self.cheby_coefficients[l], dtype=np.float64).reshape(-1)
+                    ct = (ctypes.c_double * len(tab))(*[float(v) for v in tab])
+                    self._keep.append(ct)
+                    s.cheb_degree = self.cheby_degree
+                    s.h_cheb_coef = ctypes.cast(ct, ctypes.POINTER(ctypes.c_double))
                 if getattr(lev, "csr", None) is not None and getattr(lev, "lex_ptr", None) is not None:
                     s.d_csr_indptr, s.d_csr_indices, s.d_csr_values = (t.data_ptr() for t in lev.csr)
                     s.d_lex_level_ptr = lev.lex_ptr.data_ptr()
@@ -551,7 +595,8 @@ class DeviceHierarchy:
     def make_params(self, nu_pre=1, nu_post=None, omega=1.0, zero_guess_skip=True, reverse_post=False, x0_zero=False):
         """x0_zero: the cycle starts from a zero iterate on level 0 WITHOUT reading (or needing) the contents of x --
         a preconditioner application z = M^-1 r."""
-        sm = {"jacobi": _lib.MG_SMOOTH_JACOBI, "mcgs": _lib.MG_SMOOTH_MCGS, "lexgs": _lib.MG_SMOOTH_LEXGS}[self.smoother]
+        sm = {"jacobi": _lib.MG_SMOOTH_JACOBI, "mcgs": _lib.MG_SMOOTH_MCGS, "lexgs": _lib.MG_SMOOTH_LEXGS,
+              "chebyshev": _lib.MG_SMOOTH_CHEBY}[self.smoother]
         return _lib.mg_cycle_params(sm, int(nu_pre), int(nu_pre if nu_post is None else nu_post), float(omega),
                                     1 if zero_guess_skip else 0, 1 if reverse_post else 0, 1 if x0_zero else 0, 0)
 
@@ -574,7 +619,7 @@ class DeviceHierarchy:
             self.last_launches = int(self.lib.mg_last_launch_count())
             return
         key = (L, params.smoother, params.nu_pre, params.nu_post, params.omega, params.zero_guess_skip,
-               params.reverse_post, params.x0_zero, bool(with_norm))
+               params.reverse_post, params.x0_zero, bool(with_norm), self._cheby_key)
         g = self._graphs.get(key)
         if g is None:
             cap = torch.cuda.Stream(device=self.device)
@@ -637,7 +682,7 @@ class DeviceHierarchy:
 
         def iterate(first):
             key = (first, None if params is None else (params.smoother, params.nu_pre, params.nu_post, params.omega,
-                                                       params.zero_guess_skip, params.reverse_post))
+                                                       params.zero_guess_skip, params.reverse_post, self._cheby_key))
             g = self._cg_graphs.get(key)
             if g is None:
                 if self.smoother == "lexgs" and params is not None:      # cooperative launches are not captured
@@ -728,9 +773,15 @@ class DeviceHierarchy:
             def rows_pass(R, write_vec, read_b=True):      # matrix share + b + output + distinct x entries gathered
                 return SA * R / max(n, 1) + (8 * R if read_b else 0) + 8 * R * write_vec + 8 * min(n, lenA * R)
             mc = self.smoother == "mcgs" and L_.color_ptr is not None
+            cheb = self.smoother == "chebyshev"
             fused = mc and fusion and int(getattr(L_, "flags", 0)) & 1
             skip_prolong = fused and int(getattr(L_, "flags", 0)) & 2 and nu_post > 0
-            if mc:
+            if cheb:
+                # step k: matrix, b, x gathers, x_out, plus x_i and dinv_i, d written, and d read after step 0
+                deg = self.cheby_degree
+                sweep = deg * (rows_pass(n, 1) + 16 * n + 8 * n) + (deg - 1) * 8 * n
+                last = first = 0
+            elif mc:
                 sizes = np.diff(np.asarray(L_.color_ptr, dtype=np.int64))
                 sweep = sum(SA * c / max(n, 1) + 16 * c + 8 * min(n - c, (lenA - 1) * c) for c in sizes)
                 last, first = int(sizes[-1]), int(sizes[0])
@@ -739,7 +790,9 @@ class DeviceHierarchy:
                 last = first = 0
             b = (nu_pre + nu_post) * sweep
             if l > 0 and nu_pre > 0:
-                if mc and fusion and getattr(L_, "diag", None) is not None:
+                if cheb:                                       # step 0 on zeros: dinv, b, d, x; no matrix
+                    b += 32 * n - (rows_pass(n, 1) + 24 * n)
+                elif mc and fusion and getattr(L_, "diag", None) is not None:
                     b += 8 * n + 16 * first - (SA * first / max(n, 1) + 16 * first + 8 * min(n - first, (lenA - 1) * first))
                 else:
                     b += 8 * n                                 # zero fill

@@ -387,3 +387,102 @@ def slice_records(torch, off, val_idx=None, val_table=None, uniform_len=0, max_r
     rec_vals = None if vrec is None else val_table[recs[order][:, 8:16].long()].contiguous()
     return ids, rec_table, rec_vals, int((ids >= 0).sum().item())
 
+
+
+# ---- Chebyshev smoother: coefficients, start vector, Lanczos (host twin) -------------------------------------------
+CHEBY_LANCZOS_STEPS = 10
+CHEBY_INTERVAL = (0.3, 1.1)       # default [lo, hi] as fractions of the Lanczos estimate of lambda_max(D^-1 A)
+
+
+def chebyshev_check(degree, bounds=None):
+    """ValueError unless degree is an integer >= 1 and bounds (None, or one (lo, hi) pair per smoothing level) has
+    0 < lo < hi, both finite."""
+    if isinstance(degree, bool) or not isinstance(degree, (int, np.integer)) or int(degree) < 1:
+        raise ValueError("Chebyshev degree must be an integer >= 1, got %r" % (degree,))
+    if bounds is None:
+        return
+    for b in bounds:
+        lo, hi = (float(v) for v in b)
+        if not (np.isfinite(lo) and np.isfinite(hi) and lo > 0.0 and hi > lo):
+            raise ValueError("Chebyshev bounds need 0 < lo < hi, got (%r, %r)" % (lo, hi))
+
+
+def chebyshev_coefficients(lo, hi, degree):
+    """The (degree, 2) table of (c_d, c_r) of the Chebyshev smoother over [lo, hi] (c_d of step 0 is unused, 0 here).
+    Step k of one application: dn = c_r t (k = 0) or (c_d d) + (c_r t), x += dn, d = dn, with t = D^-1 (b - A x).
+    The error after `degree` steps is T_deg((theta - lambda)/delta) / T_deg(sigma) times the start error in every
+    eigenvector of D^-1 A with eigenvalue lambda.  float64, in this exact order (the device cycle and the oracle read
+    the same table)."""
+    chebyshev_check(degree, [(lo, hi)])
+    lo, hi = float(lo), float(hi)
+    theta = (hi + lo) / 2.0
+    delta = (hi - lo) / 2.0
+    sigma = theta / delta
+    rho = 1.0 / sigma
+    out = np.zeros((int(degree), 2), dtype=np.float64)
+    out[0, 1] = 1.0 / theta
+    for k in range(1, int(degree)):
+        rho_k = 1.0 / (2.0 * sigma - rho)
+        out[k, 0] = rho_k * rho
+        out[k, 1] = 2.0 * rho_k / delta
+        rho = rho_k
+    return out
+
+
+def chebyshev_start_vector(idx):
+    """Lanczos start vector: a counter-based hash of the GLOBAL row index (NumPy or torch int64 array, indices below
+    2^31), uniform in [-1/2, 1/2).  Integer arithmetic only, so it is the same bits on the host, on any device, in any
+    row ordering and on every rank."""
+    M = 0xffffffff
+    h = (idx * 2654435761) & M
+    h = h ^ (h >> 16)
+    h = (h * 0x45d9f3b) & M
+    h = h ^ (h >> 16)
+    h = (h * 0x45d9f3b) & M
+    h = h ^ (h >> 16)
+    f = h.astype(np.float64) if isinstance(h, np.ndarray) else h.double()
+    return f * (1.0 / 4294967296.0) - 0.5
+
+
+def lanczos_tridiagonal_max(alphas, betas):
+    """largest eigenvalue of the symmetric tridiagonal Lanczos matrix (NumPy, float64)"""
+    k = len(alphas)
+    T = np.diag(np.asarray(alphas, dtype=np.float64))
+    if k > 1:
+        off = np.asarray(betas[:k - 1], dtype=np.float64)
+        T += np.diag(off, 1) + np.diag(off, -1)
+    return float(np.linalg.eigvalsh(T)[-1])
+
+
+def lanczos_breakdown(beta, alphas):
+    """Lanczos stops early when the new vector has (numerically) vanished: the Krylov space is invariant"""
+    return not (beta > 1e-14 * max(abs(a) for a in alphas))
+
+
+def chebyshev_lambda_max_host(A, steps=CHEBY_LANCZOS_STEPS):
+    """Host twin (NumPy) of the device estimate of lambda_max(D^-1 A): `steps` Lanczos steps on D^-1/2 A D^-1/2 from
+    chebyshev_start_vector, the same sequence of operations as setup_device.chebyshev_lambda_max."""
+    A = sp.csr_matrix(A)
+    d = A.diagonal()
+    if not np.all(d > 0.0):
+        raise ValueError("the Chebyshev smoother needs a positive diagonal")
+    s = np.sqrt(1.0 / d)
+    n = A.shape[0]
+    v = chebyshev_start_vector(np.arange(n, dtype=np.int64))
+    v = v * (1.0 / np.sqrt(np.dot(v, v)))
+    v_prev = None
+    alphas, betas = [], []
+    beta = 0.0
+    for k in range(int(steps)):
+        w = s * (A @ (s * v))
+        a = float(np.dot(w, v))
+        w = w - a * v
+        if v_prev is not None:
+            w = w - beta * v_prev
+        alphas.append(a)
+        beta = float(np.sqrt(np.dot(w, w)))
+        if k == steps - 1 or lanczos_breakdown(beta, alphas):
+            break
+        betas.append(beta)
+        v_prev, v = v, w * (1.0 / beta)
+    return lanczos_tridiagonal_max(alphas, betas)

@@ -440,6 +440,9 @@ def setup_device(h, A, Q_list, colors, dense_coarse_max):
     h.colors = level_colors(S, h.smoother, colors, A_host0, A_nat, t_patterns)
     del t_patterns
     tm.mark("colouring")
+    if h.smoother == "chebyshev":
+        h._chebyshev_setup(S, A_nat)
+        tm.mark("Chebyshev bounds (Lanczos)")
     perms, iperms, cptrs = [], [], []
     for l in range(L):
         if h.colors.device(l) is not None:
@@ -473,3 +476,51 @@ def download_level_matrix(h, l):
     if A is None:
         raise _lib.MgError("level matrices were not kept (keep_host=False)")
     return h._setup.download(A[l])
+
+
+def chebyshev_lambda_max(S, A, steps=F.CHEBY_LANCZOS_STEPS):
+    """Estimate of lambda_max(D^-1 A) for the Chebyshev smoother: `steps` Lanczos steps on D^-1/2 A D^-1/2 on the
+    device (mg_spmv_csr, mg_dot, mg_axpby; the diagonal scalings are element-wise products), the tridiagonal
+    eigenproblem with NumPy.  A is the level's operator in NATURAL order (DevCSR); the start vector is a hash of the
+    global row index (formats.chebyshev_start_vector), so every rank and every ordering gets the same bits.  The
+    operations are those of formats.chebyshev_lambda_max_host."""
+    torch, lib, dev = S.torch, S.lib, S.dev
+    n = A.shape[0]
+    st = S.st()
+    dinv = S.dinv(A, None)
+    if not bool(torch.all(dinv > 0.0).item()):
+        raise ValueError("the Chebyshev smoother needs a positive diagonal")
+    s = torch.sqrt(dinv)
+    ws = torch.empty(1 << 16, dtype=torch.float64, device=dev)
+    out = torch.empty(1, dtype=torch.float64, device=dev)
+
+    def dot(x, y):
+        _lib.check(lib.mg_dot(n, x.data_ptr(), y.data_ptr(), ws.data_ptr(), out.data_ptr(), st), "mg_dot")
+        return float(out.item())
+
+    def axpby(a, x, b, y, o):
+        _lib.check(lib.mg_axpby(n, float(a), x.data_ptr(), float(b), _lib.ptr(y), o.data_ptr(), st), "mg_axpby")
+
+    v = F.chebyshev_start_vector(torch.arange(n, dtype=torch.int64, device=dev))
+    axpby(1.0 / np.sqrt(dot(v, v)), v, 0.0, None, v)
+    v_prev = torch.empty_like(v)
+    u = torch.empty_like(v)
+    w = torch.empty_like(v)
+    alphas, betas = [], []
+    beta = 0.0
+    for k in range(int(steps)):
+        torch.mul(s, v, out=u)
+        _lib.check(lib.mg_spmv_csr(n, *A.ptrs(), u.data_ptr(), w.data_ptr(), st), "mg_spmv_csr")
+        torch.mul(s, w, out=w)
+        a = dot(w, v)
+        axpby(1.0, w, -a, v, w)
+        if k > 0:
+            axpby(1.0, w, -beta, v_prev, w)
+        alphas.append(a)
+        beta = float(np.sqrt(dot(w, w)))
+        if k == steps - 1 or F.lanczos_breakdown(beta, alphas):
+            break
+        betas.append(beta)
+        v_prev, v = v, v_prev
+        axpby(1.0 / beta, w, 0.0, None, v)
+    return F.lanczos_tridiagonal_max(alphas, betas)

@@ -14,6 +14,9 @@ Differences, all explicit:
     Gauss-Seidel (:88,121).  Here "GaussSeidel" selects multicolour Gauss-Seidel (`gs_order="multicolor"`,
     default) or the exact index-order sweep (`gs_order="lexicographic"`, bit-for-bit the reference's smoother);
     "Jacobi" selects damped Jacobi with `omega` (Jacobi.py:35 is omega=1, which does not smooth; default 2/3).
+    "Chebyshev" (extension) selects the Chebyshev polynomial smoother in D^-1 A: `cheby_degree` steps per sweep
+    (default 2) over [0.3, 1.1] x a Lanczos estimate of lambda_max(D^-1 A) per level, or over `cheby_bounds`
+    (one (lo, hi) pair per smoothing level).  It needs no colouring and is symmetric, so it also preconditions CG.
   * `l2_proj` may be a list [Q_0, Q_1, ...] giving a transfer operator for every level.  Levels without one
     use the reference's 1D linear interpolator (Multigrid.interpolator, :126-147), as the reference does
     below the first level (:188-197).
@@ -62,7 +65,7 @@ class Multigrid(IterativeSolver):
     # ------------------------------------------------------------------------------------------------
     def solve(self, levels=2, smoother="Jacobi", smooth_steps=1, max_iterations=100, error=1e-08,
               initial_guess=None, cycle="V", first_call=False, *, omega=2.0 / 3.0, gs_order="multicolor",
-              colors=None, use_graph=True):
+              colors=None, use_graph=True, cheby_degree=2, cheby_bounds=None):
         if initial_guess is None:
             self.solution = np.zeros(shape=(self.get_dimension(), 1))
         else:
@@ -71,7 +74,8 @@ class Multigrid(IterativeSolver):
         if not callable(cycle_method):
             print("Cycle type unknown, exit...")
             sys.exit(0)                                            # Multigrid.py:55-57
-        h = self._hierarchy(levels, smoother, gs_order, colors, first_call)
+        h = self._hierarchy(levels, smoother, gs_order, colors, first_call,
+                            **self._cheby_kw(smoother, cheby_degree, cheby_bounds))
         params = h.make_params(nu_pre=smooth_steps, nu_post=smooth_steps, omega=omega)
         h.set_rhs(self.rhs)
         if initial_guess is None:
@@ -123,13 +127,15 @@ class Multigrid(IterativeSolver):
 
     # ------------------------------------------------------------------------------------------------
     def v_cycle(self, A, u0, rhs, smoother, smooth_steps, error, levels, first_call=False, *, omega=2.0 / 3.0,
-                gs_order="multicolor", colors=None):
+                gs_order="multicolor", colors=None, cheby_degree=2, cheby_bounds=None):
         """One V-cycle for (A, rhs) starting from u0; returns the new iterate as an (n,1) array
         (Multigrid.py:77-124).  The hierarchy is cached as long as the same matrix object is passed."""
         if A is self.matrix:
-            h = self._hierarchy(levels, smoother, gs_order, colors, first_call)
+            h = self._hierarchy(levels, smoother, gs_order, colors, first_call,
+                                **self._cheby_kw(smoother, cheby_degree, cheby_bounds))
         else:
-            h = self._build(A, levels, smoother, gs_order, colors, first_call)
+            h = self._build(A, levels, smoother, gs_order, colors, first_call,
+                            **self._cheby_kw(smoother, cheby_degree, cheby_bounds))
         params = h.make_params(nu_pre=smooth_steps, nu_post=smooth_steps, omega=omega)
         h.set_rhs(rhs)
         h.set_x(u0)
@@ -179,9 +185,16 @@ class Multigrid(IterativeSolver):
         return []
 
     @staticmethod
+    def _cheby_kw(smoother, degree, bounds):
+        """the Chebyshev options as keywords of _hierarchy / _build (none for the other smoothers)"""
+        return {"cheby_degree": degree, "cheby_bounds": bounds} if smoother == "Chebyshev" else {}
+
+    @staticmethod
     def _smoother_kind(smoother, gs_order):
         if smoother == "Jacobi":
             return "jacobi"
+        if smoother == "Chebyshev":
+            return "chebyshev"
         if smoother == "GaussSeidel":
             if gs_order == "multicolor":
                 return "mcgs"
@@ -191,11 +204,15 @@ class Multigrid(IterativeSolver):
         # the reference fails with "'str' object is not callable" for an unknown name (Multigrid.py:79-80)
         raise TypeError("'str' object is not callable (unknown smoother %r)" % (smoother,))
 
-    def _build(self, A, levels, smoother, gs_order, colors, first_call):
+    def _build(self, A, levels, smoother, gs_order, colors, first_call, cheby_degree=2, cheby_bounds=None):
         if levels < 2:
             raise ValueError("levels must be >= 2 (the reference recurses without bound for levels=1, "
                              "Multigrid.py:78,102)")
         kind = self._smoother_kind(smoother, gs_order)
+        cheby = {}
+        if kind == "chebyshev":
+            F.chebyshev_check(cheby_degree, cheby_bounds)
+            cheby = {"cheby_degree": cheby_degree, "cheby_bounds": cheby_bounds}
         save = self.matrix
         try:
             self.matrix = A
@@ -210,13 +227,16 @@ class Multigrid(IterativeSolver):
             A = src
         if self.fabric is not None and self.fabric.world > 1:
             from ..distributed import DistributedHierarchy
-            return DistributedHierarchy(A, qs, self.fabric, smoother=kind, colors=colors, **self.dist_options)
-        return DeviceHierarchy(A, qs, smoother=kind, colors=colors, setup=self.setup)
+            return DistributedHierarchy(A, qs, self.fabric, smoother=kind, colors=colors, **cheby, **self.dist_options)
+        return DeviceHierarchy(A, qs, smoother=kind, colors=colors, setup=self.setup, **cheby)
 
-    def _hierarchy(self, levels, smoother, gs_order, colors, first_call):
-        key = (levels, smoother, gs_order, bool(first_call), id(self.matrix), None if colors is None else id(colors))
+    def _hierarchy(self, levels, smoother, gs_order, colors, first_call, cheby_degree=2, cheby_bounds=None):
+        cb = None if cheby_bounds is None else tuple(tuple(float(v) for v in b) for b in cheby_bounds)
+        key = (levels, smoother, gs_order, bool(first_call), id(self.matrix), None if colors is None else id(colors),
+               cheby_degree if smoother == "Chebyshev" else None, cb if smoother == "Chebyshev" else None)
         if self._hier is None or self._hier_key != key:
-            self._hier = self._build(self.matrix, levels, smoother, gs_order, colors, first_call)
+            self._hier = self._build(self.matrix, levels, smoother, gs_order, colors, first_call,
+                                     **self._cheby_kw(smoother, cheby_degree, cheby_bounds))
             self._hier_key = key
         return self._hier
 
@@ -225,11 +245,14 @@ class Multigrid(IterativeSolver):
         return self._hier
 
     def as_preconditioner(self, levels=2, smoother="GaussSeidel", smooth_steps=1, omega=2.0 / 3.0,
-                          gs_order="multicolor", first_call=True, symmetric=True, colors=None):
+                          gs_order="multicolor", first_call=True, symmetric=True, colors=None, cheby_degree=2,
+                          cheby_bounds=None):
         """z = M^-1 r by one V-cycle from a zero guess, on natural-order device vectors (for solvers.CG).
         symmetric=True runs the multicolour post-smoothing in reverse colour order, so that M is symmetric for a
-        symmetric A (Galerkin coarse operators, restriction = Q^T); damped Jacobi is symmetric as it is."""
-        h = self._hierarchy(levels, smoother, gs_order, colors, first_call)
+        symmetric A (Galerkin coarse operators, restriction = Q^T); damped Jacobi and the Chebyshev polynomial are
+        symmetric as they are."""
+        h = self._hierarchy(levels, smoother, gs_order, colors, first_call,
+                            **self._cheby_kw(smoother, cheby_degree, cheby_bounds))
         params = h.make_params(nu_pre=smooth_steps, nu_post=smooth_steps, omega=omega,
                                reverse_post=bool(symmetric) and smoother == "GaussSeidel")
         lib, torch = h.lib, h.torch

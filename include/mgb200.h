@@ -525,6 +525,38 @@ int mg_host_nn_contributions(int64_t np_, const int32_t *h_fill, const double *h
 #endif
 
 /* ------------------------------------------------------------------------------------------------ */
+/* Classical AMG setup (csrc/amg_kernels.cu, driven by learnmultigrid_b200/amg.py): strength of connection on negative
+ * couplings, PMIS C/F splitting, direct interpolation.  CSR inputs with sorted columns, int32 ids, one thread per row;
+ * the definitions are in DESIGN.md §4.10 and tests/amg_oracle.py restates them.  States: 0 undecided, 1 C, 2 F. */
+/* strength S: j != i with -a_ij > 0 and -a_ij >= theta * max_{k!=i}(-a_ik), theta in [0, 1).  Count pass (d_count[n]),
+ * exclusive scan by the caller, fill pass (pattern + the values a_ij, columns ascending) */
+int mg_amg_strength_count(int64_t n, const int32_t *d_indptr, const int32_t *d_indices, const double *d_values,
+                          double theta, int32_t *d_count, void *stream);
+int mg_amg_strength_fill(int64_t n, const int32_t *d_indptr, const int32_t *d_indices, const double *d_values,
+                         double theta, const int32_t *d_s_indptr, int32_t *d_s_indices, double *d_s_values,
+                         void *stream);
+/* PMIS rounds on S and S^T (d_t_*: its transpose) with weights d_weights: points with an empty S^T row start F; per
+ * round `select` (an undecided point whose (w, i) beats every undecided point of its S and S^T rows turns C) and
+ * `mark` (an undecided point with a C point in its S row turns F), until nothing is undecided.  d_work: n + 1 int32.
+ * One host read-back per round (synchronises); returns the number of rounds (>= 0) or a negative status. */
+int mg_amg_pmis(int64_t n, const int32_t *d_s_indptr, const int32_t *d_s_indices, const int32_t *d_t_indptr,
+                const int32_t *d_t_indices, const double *d_weights, int32_t *d_state, int32_t *d_work, void *stream);
+/* promotion pass on the final states: an F point with a non-empty S row and no C point in it turns C.  d_state_out
+ * must not alias d_state; d_work: 1 int32.  Synchronises; returns the number of promoted points or a negative status. */
+int mg_amg_promote(int64_t n, const int32_t *d_s_indptr, const int32_t *d_s_indices, const int32_t *d_state,
+                   int32_t *d_state_out, int32_t *d_work, void *stream);
+/* direct interpolation Q (n x n_c): count pass (1 per C row, |S_i n C| per F row), exclusive scan by the caller, fill
+ * pass with d_cmap from mg_nn_compact.  The fill synchronises; if a_ii + (sum of the positive off-diagonal entries) is 0
+ * in an F row that interpolates, *h_bad_row receives the smallest such row and MG_ERR_SINGULAR is returned (else -1).
+ * d_work: 1 int32. */
+int mg_amg_interp_count(int64_t n, const int32_t *d_s_indptr, const int32_t *d_s_indices, const int32_t *d_state,
+                        int32_t *d_count, void *stream);
+int mg_amg_interp_fill(int64_t n, const int32_t *d_indptr, const int32_t *d_indices, const double *d_values,
+                       const int32_t *d_s_indptr, const int32_t *d_s_indices, const double *d_s_values,
+                       const int32_t *d_state, const int32_t *d_cmap, const int32_t *d_q_indptr,
+                       int32_t *d_q_indices, double *d_q_values, int32_t *d_work, int64_t *h_bad_row, void *stream);
+
+/* ------------------------------------------------------------------------------------------------ */
 /* host-side (serial, HOST pointers) setup helpers                                                    */
 /* First-fit greedy colouring in index order on the symmetrised pattern of A; returns ncolors (>0) or <0.
  * The colour order defines the multicolour Gauss-Seidel that replaces PyAMG's index-order sweep

@@ -221,6 +221,13 @@ _SIGNATURES = {
     "mg_nn_row_normalise": (c_int, [c_i64, c_vp, c_vp, c_vp]),
     "mg_nn_cut_count": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "mg_nn_cut_fill": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "mg_amg_strength_count": (c_int, [c_i64, c_vp, c_vp, c_vp, c_dbl, c_vp, c_vp]),
+    "mg_amg_strength_fill": (c_int, [c_i64, c_vp, c_vp, c_vp, c_dbl, c_vp, c_vp, c_vp, c_vp]),
+    "mg_amg_pmis": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "mg_amg_promote": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "mg_amg_interp_count": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "mg_amg_interp_fill": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                   ctypes.POINTER(c_i64), c_vp]),
     "mg_host_greedy_color": (c_int, [c_i64, c_vp, c_vp, c_vp]),
     "mg_host_greedy_color_block": (c_int, [c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int]),
     "mg_host_lex_levels": (c_i64, [c_i64, c_vp, c_vp, c_vp]),

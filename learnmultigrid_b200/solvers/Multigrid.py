@@ -3,6 +3,7 @@
     Multigrid(matrix, rhs)                    Multigrid.py:26-161
     GeometricMG(matrix, rhs)                  Multigrid.py:164-173
     SemiGeometricMG(matrix, rhs, l2_proj)     Multigrid.py:176-197
+    AlgebraicMG(matrix, rhs, theta=0.25)      extension: classical AMG transfer operators built from the matrix
 
 `solve()` keeps the reference's outer loop statement by statement (Multigrid.py:36-75): residual, 2-norm,
 the first-iteration sqrt(n) quirk (:64-66), history, ABSOLUTE tolerance test, one V-cycle.  The V-cycle itself
@@ -310,6 +311,84 @@ class SemiGeometricMG(Multigrid):
 
     def _given_transfers(self):
         return self.l_hierarchy
+
+
+class AlgebraicMG(Multigrid):
+    """AlgebraicMG(matrix, rhs, theta=0.25) -- classical AMG (extension; no reference counterpart in the engine): the
+    transfer operators come from the matrix alone, built on the device by learnmultigrid_b200/amg.py (strength of
+    connection on negative couplings with threshold `theta`, PMIS C/F splitting, direct interpolation), one level at a
+    time.  This is the multigrid the reference's 2D scripts compare against with PyAMG's ruge_stuben_solver; the
+    splitting is PMIS, not Ruge-Stueben's serial first pass, so the coarse grids differ from PyAMG's.
+
+    The operators are built on demand for the matrix a hierarchy is built for (solve, v_cycle, as_preconditioner,
+    distribute) and cached by matrix object; the operators for fewer levels are a prefix of those for more levels.
+    `define_hierarchy(levels)` builds them explicitly, `l_hierarchy` holds them (device CSR) and `amg_stats` their
+    per-level statistics and complexities.  A level that cannot be coarsened raises ValueError."""
+
+    def __init__(self, matrix, rhs, theta=0.25):
+        super().__init__(matrix, rhs)
+        from ..amg import check_theta
+        self.label = "AlgebraicMG"
+        self.theta = check_theta(theta)
+        self.l_hierarchy = []
+        self.amg_stats = None
+        self._amg_cache = {}            # "own" / "other" -> (matrix object, [Q_0, ...], per-level stats)
+        self._builder = None
+
+    def _ab(self):
+        if self._builder is None:
+            from ..amg import AmgBuilder
+            self._builder = AmgBuilder()
+        return self._builder
+
+    def _amg_source(self, A):
+        """the level-0 operator as the hierarchy will hold it (the caller's canonical CSR, or CSR of the stored CSC)"""
+        if hasattr(A, "ptrs"):
+            return A
+        src = getattr(self, "_matrix_src", None)
+        if (A is self._own_matrix() and src is not None and sp.isspmatrix_csr(src) and src.dtype == np.float64
+                and src.has_canonical_format):
+            return F.canonical_csr(src)
+        return F.solver_csr(A)
+
+    def _own_matrix(self):
+        return getattr(self, "_solver_matrix", self.matrix)
+
+    def _amg_transfers(self, A, levels):
+        """[Q_0 ... Q_{levels-2}] for operator A, from the cache or built.  The cache holds the operators of the solver's
+        own matrix and of the last other operator a V-cycle was asked for (v_cycle(A, ...)), each with the matrix
+        object it was built for; l_hierarchy and amg_stats always describe the solver's own matrix."""
+        from ..amg import complexities
+        if levels < 2:
+            raise ValueError("levels must be >= 2")
+        own = A is self._own_matrix()
+        slot = "own" if own else "other"
+        c = self._amg_cache.get(slot)
+        if c is None or c[0] is not A or len(c[1]) < levels - 1:
+            b = self._ab()
+            qs = b.define_hierarchy(self._amg_source(A), levels, self.theta)
+            c = self._amg_cache[slot] = (A, qs, [dict(s) for s in b.stats])
+        qs = list(c[1][:levels - 1])
+        if own:
+            stats = [dict(s) for s in c[2][:levels]]
+            stats[-1] = {"level": levels - 1, "rows": stats[-1]["rows"], "nnz": stats[-1]["nnz"]}
+            gc, oc = complexities([s["rows"] for s in stats], [s["nnz"] for s in stats])
+            self.amg_stats = {"theta": self.theta, "levels": stats, "grid_complexity": gc, "operator_complexity": oc}
+            self.l_hierarchy = qs
+        return qs
+
+    def define_hierarchy(self, levels=2):
+        return self._amg_transfers(self.matrix, levels)
+
+    def _transfer_list(self, levels, first_call):
+        return self._amg_transfers(self.matrix, levels)
+
+    def _build(self, A, levels, smoother, gs_order, colors, first_call, **kw):
+        self._solver_matrix = self.matrix           # _build swaps self.matrix for the operator it is given
+        try:
+            return super()._build(A, levels, smoother, gs_order, colors, first_call, **kw)
+        finally:
+            del self._solver_matrix
 
 
 class NeuralMG(Multigrid):

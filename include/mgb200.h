@@ -557,6 +557,47 @@ int mg_amg_interp_fill(int64_t n, const int32_t *d_indptr, const int32_t *d_indi
                        int32_t *d_q_indices, double *d_q_values, int32_t *d_work, int64_t *h_bad_row, void *stream);
 
 /* ------------------------------------------------------------------------------------------------ */
+/* Smoothed aggregation setup (csrc/sa_kernels.cu, driven by learnmultigrid_b200/sa.py): symmetric strength of
+ * connection, MIS(2) roots, aggregation, tentative prolongator, Jacobi-smoothing scale.  CSR inputs with sorted
+ * columns, int32 ids, one thread per row (or aggregate); the definitions are in DESIGN.md §4.11 and tests/sa_oracle.py
+ * restates them.  MIS(2) states: 0 OUT, 1 undecided, 2 IN (root). */
+/* d_diag[i] = the stored a_ii (0 where none is stored) */
+int mg_sa_diagonal(int64_t n, const int32_t *d_indptr, const int32_t *d_indices, const double *d_values,
+                   double *d_diag, void *stream);
+/* strength S: j != i with a_ij != 0 and a_ij * a_ij >= theta^2 * (|a_ii| * |a_jj|), theta in [0, 1) (theta^2 formed
+ * once on the host), d_diag from mg_sa_diagonal.  Count pass (d_count[n]), exclusive scan by the caller, fill pass
+ * (pattern + the values a_ij, columns ascending) */
+int mg_sa_strength_count(int64_t n, const int32_t *d_indptr, const int32_t *d_indices, const double *d_values,
+                         const double *d_diag, double theta, int32_t *d_count, void *stream);
+int mg_sa_strength_fill(int64_t n, const int32_t *d_indptr, const int32_t *d_indices, const double *d_values,
+                        const double *d_diag, double theta, const int32_t *d_s_indptr, int32_t *d_s_indices,
+                        double *d_s_values, void *stream);
+/* MIS(2) on the graph S u S^T (d_t_*: the transpose of S): isolated points start OUT, the others undecided; per round
+ * two passes propagate the maximum key (state, hash(i)) over {i} u S_i u S^T_i, and an undecided point turns IN if the
+ * maximum is its own key, OUT if the maximum's state is IN.  d_work: n + 1 int32, d_keys: 2n uint64.  One host read-back
+ * per round (synchronises); returns the number of rounds (>= 0) or a negative status. */
+int mg_sa_mis2(int64_t n, const int32_t *d_s_indptr, const int32_t *d_s_indices, const int32_t *d_t_indptr,
+               const int32_t *d_t_indices, int32_t *d_state, int32_t *d_work, uint64_t *d_keys, void *stream);
+/* aggregates d_agg[n] (-1: isolated) from the final MIS(2) states and d_cmap (mg_nn_compact over the roots): pass 1
+ * joins a point to the root among its neighbours, pass 2 an unassigned one to its pass-1 neighbour of largest
+ * (hash(j), j).  d_work: n + 2 int32.  Synchronises; a point with two distinct roots among its neighbours, or a
+ * non-isolated point left unassigned, is MG_ERR_INVALID with the smallest such point in *h_bad_row (else -1). */
+int mg_sa_aggregate(int64_t n, const int32_t *d_s_indptr, const int32_t *d_s_indices, const int32_t *d_t_indptr,
+                    const int32_t *d_t_indices, const int32_t *d_state, const int32_t *d_cmap, int32_t *d_agg,
+                    int32_t *d_work, int64_t *h_bad_row, void *stream);
+/* nu_a = sqrt(sum of the squares of row a of T^T, in storage order); one thread per aggregate */
+int mg_sa_aggregate_norm(int64_t nc, const int32_t *d_tt_indptr, const double *d_tt_values, double *d_nu,
+                         void *stream);
+/* tentative prolongator T (n x n_c, one entry per aggregated row): column d_agg[i], value d_b[i] / d_nu[d_agg[i]], or
+ * d_b[i] where d_nu is NULL (the pattern pass whose transpose gives nu); d_t_indptr: exclusive scan of d_agg >= 0 */
+int mg_sa_tentative_fill(int64_t n, const int32_t *d_agg, const int32_t *d_t_indptr, const double *d_b,
+                         const double *d_nu, int32_t *d_t_indices, double *d_t_values, void *stream);
+/* the values of I - omega_hat D^-1 A on A's pattern (d_out_values[nnz]): -(s_i * a_ij) off the diagonal,
+ * 1 - s_i * a_ii on it, s_i = omega_hat / a_ii */
+int mg_sa_smooth_scale(int64_t n, const int32_t *d_indptr, const int32_t *d_indices, const double *d_values,
+                       const double *d_diag, double omega_hat, double *d_out_values, void *stream);
+
+/* ------------------------------------------------------------------------------------------------ */
 /* host-side (serial, HOST pointers) setup helpers                                                    */
 /* First-fit greedy colouring in index order on the symmetrised pattern of A; returns ncolors (>0) or <0.
  * The colour order defines the multicolour Gauss-Seidel that replaces PyAMG's index-order sweep

@@ -228,6 +228,14 @@ _SIGNATURES = {
     "mg_amg_interp_count": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "mg_amg_interp_fill": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
                                    ctypes.POINTER(c_i64), c_vp]),
+    "mg_sa_diagonal": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "mg_sa_strength_count": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_dbl, c_vp, c_vp]),
+    "mg_sa_strength_fill": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_dbl, c_vp, c_vp, c_vp, c_vp]),
+    "mg_sa_mis2": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "mg_sa_aggregate": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.POINTER(c_i64), c_vp]),
+    "mg_sa_aggregate_norm": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp]),
+    "mg_sa_tentative_fill": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "mg_sa_smooth_scale": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_dbl, c_vp, c_vp]),
     "mg_host_greedy_color": (c_int, [c_i64, c_vp, c_vp, c_vp]),
     "mg_host_greedy_color_block": (c_int, [c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int]),
     "mg_host_lex_levels": (c_i64, [c_i64, c_vp, c_vp, c_vp]),

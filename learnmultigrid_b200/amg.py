@@ -135,16 +135,9 @@ class AmgBuilder:
         theta = check_theta(theta)
         if levels < 2:
             raise ValueError("levels must be >= 2")
-        t = self.torch
         Al = A if isinstance(A, SD.DevCSR) else self.upload(A)
         Qs, self.stats, self.trace = [], [], []
-        clock = time.perf_counter
-
-        def mark(t0):
-            t.cuda.synchronize()
-            now = clock()
-            return now, round((now - t0) * 1e3, 3)
-
+        clock, mark = time.perf_counter, self.mark
         for l in range(levels - 1):
             n = Al.shape[0]
             t0 = clock()
@@ -173,6 +166,12 @@ class AmgBuilder:
         if keep_intermediates:
             self.trace.append({"A": Al})
         return Qs
+
+    def mark(self, t0):
+        """(now, ms since t0) after the device has finished the work enqueued so far: the setup split's clock"""
+        self.torch.cuda.synchronize()
+        now = time.perf_counter()
+        return now, round((now - t0) * 1e3, 3)
 
     def complexities(self, levels=None):
         st = self.stats[:levels]

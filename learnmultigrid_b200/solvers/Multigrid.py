@@ -4,6 +4,8 @@
     GeometricMG(matrix, rhs)                  Multigrid.py:164-173
     SemiGeometricMG(matrix, rhs, l2_proj)     Multigrid.py:176-197
     AlgebraicMG(matrix, rhs, theta=0.25)      extension: classical AMG transfer operators built from the matrix
+    SmoothedAggregationMG(matrix, rhs, theta=0.0, omega=4/3)
+                                              extension: smoothed aggregation transfer operators built from the matrix
 
 `solve()` keeps the reference's outer loop statement by statement (Multigrid.py:36-75): residual, 2-norm,
 the first-iteration sqrt(n) quirk (:64-66), history, ABSOLUTE tolerance test, one V-cycle.  The V-cycle itself
@@ -341,6 +343,10 @@ class AlgebraicMG(Multigrid):
             self._builder = AmgBuilder()
         return self._builder
 
+    def _define_transfers(self, source, levels):
+        """the builder's transfer operators for `source` and the parameters amg_stats reports with them"""
+        return self._ab().define_hierarchy(source, levels, self.theta), {"theta": self.theta}
+
     def _amg_source(self, A):
         """the level-0 operator as the hierarchy will hold it (the caller's canonical CSR, or CSR of the stored CSC)"""
         if hasattr(A, "ptrs"):
@@ -365,15 +371,14 @@ class AlgebraicMG(Multigrid):
         slot = "own" if own else "other"
         c = self._amg_cache.get(slot)
         if c is None or c[0] is not A or len(c[1]) < levels - 1:
-            b = self._ab()
-            qs = b.define_hierarchy(self._amg_source(A), levels, self.theta)
-            c = self._amg_cache[slot] = (A, qs, [dict(s) for s in b.stats])
+            qs, head = self._define_transfers(self._amg_source(A), levels)
+            c = self._amg_cache[slot] = (A, qs, [dict(s) for s in self._ab().stats], head)
         qs = list(c[1][:levels - 1])
         if own:
             stats = [dict(s) for s in c[2][:levels]]
             stats[-1] = {"level": levels - 1, "rows": stats[-1]["rows"], "nnz": stats[-1]["nnz"]}
             gc, oc = complexities([s["rows"] for s in stats], [s["nnz"] for s in stats])
-            self.amg_stats = {"theta": self.theta, "levels": stats, "grid_complexity": gc, "operator_complexity": oc}
+            self.amg_stats = dict(c[3], levels=stats, grid_complexity=gc, operator_complexity=oc)
             self.l_hierarchy = qs
         return qs
 
@@ -389,6 +394,35 @@ class AlgebraicMG(Multigrid):
             return super()._build(A, levels, smoother, gs_order, colors, first_call, **kw)
         finally:
             del self._solver_matrix
+
+
+class SmoothedAggregationMG(AlgebraicMG):
+    """SmoothedAggregationMG(matrix, rhs, theta=0.0, omega=4/3) -- smoothed aggregation AMG (extension): the transfer
+    operators come from the matrix alone, built on the device by learnmultigrid_b200/sa.py (symmetric strength of
+    connection with threshold `theta`, MIS(2) aggregation, the tentative prolongator of the constant vector and one
+    Jacobi smoothing step with weight `omega / lambda_max(D^-1 A)`), one level at a time.  This is the solver PyAMG calls
+    smoothed_aggregation_solver; the aggregation is parallel (MIS(2)), not PyAMG's serial standard aggregation, so the
+    aggregates differ from PyAMG's.
+
+    Caching, the prefix property, l_hierarchy, amg_stats (which also carries omega) and every smoother, PCG and
+    distribute() work as for AlgebraicMG.  A level that cannot be coarsened, or has a non-positive diagonal, raises
+    ValueError."""
+
+    def __init__(self, matrix, rhs, theta=0.0, omega=4.0 / 3.0):
+        super().__init__(matrix, rhs, theta)
+        from ..sa import check_omega
+        self.label = "SmoothedAggregationMG"
+        self.omega = check_omega(omega)
+
+    def _ab(self):
+        if self._builder is None:
+            from ..sa import SaBuilder
+            self._builder = SaBuilder()
+        return self._builder
+
+    def _define_transfers(self, source, levels):
+        return (self._ab().define_hierarchy(source, levels, self.theta, self.omega),
+                {"theta": self.theta, "omega": self.omega})
 
 
 class NeuralMG(Multigrid):

@@ -198,6 +198,15 @@ class DistributedHierarchy(DeviceHierarchy):
                  n_dist=None, dense_coarse_max=DENSE_COARSE_MAX, keep_host=False, region_bytes=16 << 20,
                  max_sites=512, timeout_s=10.0, split_coarse_solve=True, bcr_split_min_blocks=32, cheby_degree=2,
                  cheby_bounds=None):
+        self._init_rank(fabric, smoother, len(Q_list) + 1, device, split_coarse_solve, bcr_split_min_blocks,
+                        cheby_degree, cheby_bounds)
+        self.keep_host = keep_host
+        self._setup_dist(A, Q_list, colors, dense_coarse_max, min_rows_per_rank, n_dist)
+        self._start(region_bytes, max_sites, timeout_s)
+
+    def _init_rank(self, fabric, smoother, nlevels, device, split_coarse_solve, bcr_split_min_blocks, cheby_degree=2,
+                   cheby_bounds=None):
+        """This rank's state before any level exists: device, smoother, fabric."""
         torch = _lib.require_cuda()
         self.split_coarse_solve = bool(split_coarse_solve)
         self.bcr_split_min_blocks = int(bcr_split_min_blocks)
@@ -208,18 +217,20 @@ class DistributedHierarchy(DeviceHierarchy):
             raise ValueError("partitioned levels support 'jacobi', 'mcgs' and 'chebyshev' (index-order Gauss-Seidel is "
                              "serial across row blocks)")
         self.smoother = smoother
-        self.nlevels = len(Q_list) + 1
+        self.nlevels = nlevels
         if self.nlevels < 2:
             raise ValueError("need at least one transfer operator (levels >= 2)")
         self._chebyshev_args(cheby_degree, cheby_bounds)
         self.fabric = fabric
         self.rank, self.world = fabric.rank, fabric.world
-        self.keep_host = keep_host
         self._graphs = {}
         self._keep = []
         self.setup_kind = "device"
-        self._setup_dist(A, Q_list, colors, dense_coarse_max, min_rows_per_rank, n_dist)
-        self.comm = PeerComm(fabric, torch, region_bytes, max_sites, timeout_s)
+
+    def _start(self, region_bytes, max_sites, timeout_s):
+        """Communicator, level structs and warm-up once the levels are built; returns when every rank is ready."""
+        torch = self.torch
+        self.comm = PeerComm(self.fabric, torch, region_bytes, max_sites, timeout_s)
         self._finish_structs()
         self._norm_local = torch.zeros(1, dtype=torch.float64, device=self.device)
         self._norm_slots = torch.zeros(_lib.MG_MAX_RANKS, dtype=torch.float64, device=self.device)
@@ -227,7 +238,7 @@ class DistributedHierarchy(DeviceHierarchy):
                                               self._norm_slots.data_ptr(), self._norm_out.data_ptr())
         self._warm_up()
         torch.cuda.current_stream().synchronize()
-        fabric.barrier()
+        self.fabric.barrier()
 
     def _warm_up(self):
         """Launch every kernel of the cycle once with the exchanges disabled (mg_comm.dry_run), so that CUDA's lazy
@@ -286,10 +297,10 @@ class DistributedHierarchy(DeviceHierarchy):
         return self.torch.unique(cols[(cols < c0) | (cols >= c1)])
 
     def _setup_dist(self, A, Q_list, colors, dense_coarse_max, min_rows, n_dist):
+        """The levels from the GLOBAL operators, formed on every rank; this rank's row blocks are cut out of them."""
         torch, dev = self.torch, self.device
         W, rank = self.world, self.rank
         S = SD.DeviceSetup(torch, dev)
-        self._setup = S
         L = self.nlevels
         A_host0, A_nat, Q_nat, QT_nat = SD.build_natural(S, A, Q_list)
         if self.smoother == "chebyshev":
@@ -308,14 +319,12 @@ class DistributedHierarchy(DeviceHierarchy):
             n_dist = max(n_dist, 1)
         if not 1 <= n_dist <= L - 1:
             raise ValueError("n_dist must be between 1 and levels-1")
-        self.n_dist = Lp = int(n_dist)
         self.colors = SD.level_colors(S, self.smoother, colors, A_host0, A_nat)
         offs = [PT.block_offsets(n, W) for n in ns]
-        self.offsets = offs
 
         # ---- halo plans of the partitioned levels
         plans = []
-        for l in range(Lp):
+        for l in range(int(n_dist)):
             o0, o1 = int(offs[l][rank]), int(offs[l][rank + 1])
             parts = [self._ext(A_nat[l], o0, o1, o0, o1)]
             c0, c1 = int(offs[l + 1][rank]), int(offs[l + 1][rank + 1])
@@ -325,7 +334,32 @@ class DistributedHierarchy(DeviceHierarchy):
                 parts.append(self._ext(Q_nat[l - 1], f0, f1, o0, o1))
             ext = torch.unique(torch.cat(parts)).cpu().numpy()
             plans.append(PT.RankPlan(offs[l], rank, ext, self.colors[l]))
-        self.plans = plans
+
+        def row_block(l, m):
+            M, o = {"A": (A_nat, offs[l]), "Q": (Q_nat, offs[l]), "QT": (QT_nat, offs[l + 1])}[m]
+            return self._rowblock(M[l], int(o[rank]), int(o[rank + 1]))
+
+        self._build_levels(S, offs, plans, row_block, A_nat, Q_nat, QT_nat, dense_coarse_max)
+        if self.keep_host:
+            self._dev_A_nat = A_nat
+            self._dev_Q_nat = Q_nat
+
+    def _build_levels(self, S, offs, plans, row_block, A_nat, Q_nat, QT_nat, dense_coarse_max):
+        """This rank's levels, from
+          offs                   : partition.block_offsets of every level
+          plans                  : the RankPlans of the partitioned levels 0 .. n_dist-1 (n_dist = len(plans))
+          row_block(l, m)        : this rank's row block of A_l (m = "A"), of Q_l (m = "Q", the fine rows it owns) or of
+                                   Q_l^T (m = "QT", the coarse rows it owns) as a DevCSR with global column ids; called
+                                   once per block, level by level, and the block is dropped once it is packed, so a
+                                   source that forms blocks on demand holds one at a time
+          A_nat, Q_nat, QT_nat   : the replicated levels' operators in natural order (entries below n_dist not read)
+        self.colors[l] (l >= n_dist) and self._global_n / _global_nnzA / _global_nnzQ must be set."""
+        torch, dev = self.torch, self.device
+        W, rank = self.world, self.rank
+        L, Lp = self.nlevels, len(plans)
+        ns = self._global_n
+        self._setup = S
+        self.n_dist, self.offsets, self.plans = Lp, offs, plans
         # who needs what from whom: every rank tells the others which of their rows it reads, in its halo order
         mine = []
         for l in range(Lp):
@@ -357,10 +391,9 @@ class DistributedHierarchy(DeviceHierarchy):
             if self.colors[l] is not None:
                 perms[l], iperms[l], cptrs[l] = S.color_perm(self.colors[l])
         dummy = torch.zeros(1, dtype=torch.int32, device=dev)
-        if Lp < L:
-            lays[Lp] = _Layout(0, ns[Lp], iperms[Lp], ns[Lp], dummy, ns[Lp])
+        lays[Lp] = _Layout(0, ns[Lp], iperms[Lp], ns[Lp], dummy, ns[Lp])
 
-        # ---- partitioned levels
+        # ---- partitioned levels: the row blocks (global column ids) are remapped to my level vector and packed
         self.levels = []
         for l in range(Lp):
             p = plans[l]
@@ -371,25 +404,32 @@ class DistributedHierarchy(DeviceHierarchy):
             lev.plan = p
             lev.perm = None if p.perm is None else torch.from_numpy(p.perm).to(dev)
             lev.color_ptr = p.color_ptr
-            lev.nnz_A, lev.nnz_Q = A_nat[l].nnz, Q_nat[l].nnz
-            if self.colors[l] is not None:
-                # what the cycle may assume (mg_level.flags) must hold for the GLOBAL operator: a row of this block may
-                # couple to a halo row of its own colour; every rank holds the global level here and gets the same answer
-                lev.flags = S.coloring_flags(A_nat[l], self.colors[l])
-            blk = self._rowblock(A_nat[l], p.o0, p.o1)
+            lev.nnz_A, lev.nnz_Q = self._global_nnzA[l], self._global_nnzQ[l]
+            blk = row_block(l, "A")
             loc = SD.DevCSR((p.n_own, lev.n_vec), blk.indptr, self._remap(S, blk.indices, lays[l]), blk.values)
             Ap = S.permute(loc, lev.perm, None)
             lev.A = S.to_sell(Ap)
             lev.dinv = S.dinv(Ap, None)
             lev.local_nnz_A = Ap.nnz
+            if p.color_ptr is not None:
+                # mg_level.flags must hold for the GLOBAL operator and be the same on every rank (they decide the
+                # launch sequence, hence the exchange sites): this block's rows against the colours of everything they
+                # read -- own rows by colour block, halo slots by (owner, colour) segment -- then AND over the ranks
+                vcol = np.full(lev.n_vec, -1, dtype=np.int32)
+                for c in range(len(p.color_ptr) - 1):
+                    vcol[int(p.color_ptr[c]):int(p.color_ptr[c + 1])] = c
+                for (q, c), (a, b) in p.seg_color.items():
+                    vcol[p.n_own + a:p.n_own + b] = c
+                mine_flags = S.coloring_flags(Ap, vcol)
+                lev.flags = int(np.bitwise_and.reduce([int(f) for f in self.fabric.allgather(mine_flags)]))
             del blk, loc, Ap
-            blk = self._rowblock(Q_nat[l], p.o0, p.o1)
+            blk = row_block(l, "Q")
             loc = SD.DevCSR((p.n_own, lays[l + 1].length), blk.indptr, self._remap(S, blk.indices, lays[l + 1]),
                             blk.values)
             lev.Q = S.to_sell(S.permute(loc, lev.perm, None))
             del blk, loc
             c0, c1 = int(offs[l + 1][rank]), int(offs[l + 1][rank + 1])
-            blk = self._rowblock(QT_nat[l], c0, c1)
+            blk = row_block(l, "QT")
             loc = SD.DevCSR((c1 - c0, lev.n_vec), blk.indptr, self._remap(S, blk.indices, lays[l]), blk.values)
             cperm = None
             if l + 1 < Lp and plans[l + 1].perm is not None:
@@ -410,16 +450,13 @@ class DistributedHierarchy(DeviceHierarchy):
         del lays
         # ---- replicated levels
         for l in range(Lp, L):
-            self.levels.append(SD.build_replicated_level(self, S, l, L, A_host0, A_nat, Q_nat, QT_nat, perms, iperms,
+            self.levels.append(SD.build_replicated_level(self, S, l, L, None, A_nat, Q_nat, QT_nat, perms, iperms,
                                                          cptrs, dense_coarse_max))
         last = self.levels[-1]
         if last.coarse_kind == _lib.MG_COARSE_BCR and self.split_coarse_solve:
             last.coarse_bcr_dist = last.coarse.make_dist(rank, W, self.bcr_split_min_blocks)
         self.host_A = None
         self.host_Q = None
-        if self.keep_host:
-            self._dev_A_nat = A_nat
-            self._dev_Q_nat = Q_nat
         S._temp = None
         torch.cuda.current_stream().synchronize()
 

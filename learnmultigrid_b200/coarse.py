@@ -233,6 +233,14 @@ class BcrCoarse:
 
 
 BCR_MAX_FACTOR_BYTES = 24 << 30     # refuse factorisations beyond this (5 n m doubles)
+BCR_MAX_BLOCK = 4096                # largest block the batched inverse takes (kGjMaxM in csrc/bcr.cu)
+
+
+def bcr_fits(n, half_bw):
+    """whether BcrCoarse takes n unknowns of half bandwidth half_bw (with its default min_block of 64): at least four
+    block rows, blocks the batched inverse can invert, and factors within BCR_MAX_FACTOR_BYTES"""
+    m = max(int(half_bw), 64)
+    return m <= BCR_MAX_BLOCK and (n + m - 1) // m >= 4 and 5 * n * m * 8 <= BCR_MAX_FACTOR_BYTES
 
 
 def rcm_ordering(indptr, indices, n):
@@ -251,6 +259,25 @@ def permuted_half_bandwidth(indptr, indices, perm):
     return int(np.abs(iperm[indices] - iperm[rows]).max()) if len(indices) else 0
 
 
+def bcr_ordering(n, indptr, indices):
+    """(half bandwidth, perm) for block cyclic reduction of the n x n pattern (indptr, indices) on the host: perm is
+    None to keep the numbering, else the reverse Cuthill-McKee permutation.  Raises MgError when neither numbering
+    fits bcr_fits."""
+    bw = half_bandwidth(indptr, indices)
+    # a structured grid in natural order has half bandwidth ~ sqrt(n): keep it (no permutation in the solve)
+    if bcr_fits(n, bw) and bw * bw <= 4 * n:
+        return bw, None
+    perm = rcm_ordering(indptr, indices, n)
+    bw_p = permuted_half_bandwidth(indptr, indices, perm)
+    if bw_p >= bw and bcr_fits(n, bw):
+        return bw, None
+    if not bcr_fits(n, bw_p):
+        raise _lib.MgError("direct solve: %d unknowns with half bandwidth %d (%d after reverse Cuthill-McKee) are neither "
+                           "small enough for a dense inverse nor banded enough for block cyclic reduction"
+                           % (n, bw, bw_p))
+    return bw_p, perm
+
+
 def build_coarse_solver(torch, dev, n, ip, ix, va, dense_max, host_pattern=None):
     """Direct solver for an operator given as device CSR (ip, ix, va) -- the coarsest level of a hierarchy
     (Multigrid.py:106) or the system of DirectSolver (Solver.py:56-59):
@@ -262,23 +289,9 @@ def build_coarse_solver(torch, dev, n, ip, ix, va, dense_max, host_pattern=None)
         return DenseCoarse(torch, dev, n, ip, ix, va)
     if host_pattern is None:
         host_pattern = (ip.cpu().numpy(), ix.cpu().numpy())
-    hp, hx = host_pattern
-    bw = half_bandwidth(hp, hx)
-
-    def fits(b):
-        m = max(b, 64)
-        return (n + m - 1) // m >= 4 and 5 * n * m * 8 <= BCR_MAX_FACTOR_BYTES
-    # a structured grid in natural order has half bandwidth ~ sqrt(n): keep it (no permutation in the solve)
-    if fits(bw) and bw * bw <= 4 * n:
+    bw, perm = bcr_ordering(n, *host_pattern)
+    if perm is None:
         return BcrCoarse(torch, dev, n, ip, ix, va, bw)
-    perm = rcm_ordering(hp, hx, n)
-    bw_p = permuted_half_bandwidth(hp, hx, perm)
-    if bw_p >= bw and fits(bw):
-        return BcrCoarse(torch, dev, n, ip, ix, va, bw)
-    if not fits(bw_p):
-        raise _lib.MgError("direct solve: %d unknowns with half bandwidth %d (%d after reverse Cuthill-McKee) are neither "
-                           "small enough for a dense inverse nor banded enough for block cyclic reduction"
-                           % (n, bw, bw_p))
     # P A P^T on the device: rows gathered by perm, columns relabelled by its inverse (entry order inside a row is
     # irrelevant to the block extraction)
     from .setup_device import DevCSR, DeviceSetup
@@ -287,4 +300,4 @@ def build_coarse_solver(torch, dev, n, ip, ix, va, dense_max, host_pattern=None)
     iperm = S.empty(n, torch.int32)
     _lib.check(S.lib.mg_invert_permutation(n, dperm.data_ptr(), iperm.data_ptr(), S.st()), "mg_invert_permutation")
     Ap = S.permute(DevCSR((n, n), ip, ix, va), dperm, iperm)
-    return BcrCoarse(torch, dev, n, Ap.indptr, Ap.indices, Ap.values, bw_p, perm=perm)
+    return BcrCoarse(torch, dev, n, Ap.indptr, Ap.indices, Ap.values, bw, perm=perm)

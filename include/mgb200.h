@@ -35,7 +35,7 @@ typedef enum {
 int mg_version(void);
 const char *mg_last_error(void);
 /* sizeof of the ABI structs as compiled (0 mg_sell, 1 mg_level, 2 mg_cycle_params, 3 mg_bcr, 4 mg_comm, 5 mg_xfer,
- * 6 mg_dist_level, 7 mg_bcr_dist, 8 mg_dist_norm): lets a binding verify its own layout */
+ * 6 mg_dist_level, 7 mg_bcr_dist, 8 mg_dist_norm, 9 mg_gmres): lets a binding verify its own layout */
 int64_t mg_struct_size(int which);
 /* 1 (default): the kernels of the cycle are launched with programmatic stream serialization (each kernel waits for
  * its predecessor with griddepcontrol.wait and lets its successor be scheduled early); 0: plain stream order.
@@ -377,6 +377,10 @@ int mg_comm_begin(mg_comm *comm);
 int mg_comm_exchange(mg_comm *comm, const mg_xfer *xfer, const double *d_src, double *d_dst, void *stream);
 /* *d_out = sum over ranks of *d_value, added in rank order (identical bits on every rank); d_slots: world doubles */
 int mg_comm_allreduce_sum(mg_comm *comm, const double *d_value, double *d_slots, double *d_out, void *stream);
+/* d_out[i] = sum over ranks of d_values[i], i < k, added in rank order at ONE exchange site; d_slots: world * k doubles.
+ * mg_comm_allreduce_sum is its k = 1 case. */
+int mg_comm_allreduce_sum_n(mg_comm *comm, const double *d_values, int32_t k, double *d_slots, double *d_out,
+                            void *stream);
 int mg_comm_end(mg_comm *comm, void *stream);                /* epoch += 1                                           */
 /* synchronises the stream; *h_error = 0, or 1 + the first site whose wait timed out */
 int mg_comm_error(mg_comm *comm, int32_t *h_error, void *stream);
@@ -745,6 +749,51 @@ typedef struct {
 int mg_pcg_start(mg_comm *comm, const mg_level *levels, const mg_pcg *pcg, void *stream);
 int mg_pcg_iterate(mg_comm *comm, const mg_level *levels, int nlevels, const mg_cycle_params *params, const mg_pcg *pcg,
                    int first, void *stream);
+/* Restarted GMRES, right-preconditioned by one V-cycle per step (z_j = M^-1 v_j, w = A z_j; params == NULL: z_j = v_j),
+ * everything in the level-0 ordering and on the device; the right-hand side is in levels[0].d_b.  Column-major buffers:
+ * basis vector k of V (Z) starts at d_V + k * ld (d_Z + k * ld); the Hessenberg matrix d_H is (restart+1) x restart
+ * with leading dimension restart + 1.  Arnoldi uses classical Gram-Schmidt in one pass, the least-squares problem is
+ * kept triangular by Givens rotations.  Scalars:
+ *     d_scalars[8]: [0] the squared residual the host reads  [1] divisor of the next basis vector  [2..7] scratch
+ * mg_gmres_start: v_0 = r / beta with r = b - A x, beta = ||r|| (x's halo exchanged first when partitioned), g = beta e_1,
+ *     [0] = beta^2; beta == 0 divides nothing.
+ * mg_gmres_iterate(j): z_j = M^-1 v_j (one V-cycle from zero on the level-0 struct with d_b = v_j, d_x = z_j: nothing
+ *     is copied), w = A z_j into slot j+1 of V, h = V^T w (multi-dot), w -= sum h_k v_k together with ||w||^2
+ *     (multi-axpy), the Givens step (h_{j+1,j} = ||w||, rotations, g), v_{j+1} = w / h_{j+1,j} unless that is 0;
+ *     [0] = |g_{j+1}|^2.  Launches only: one call can be captured in a CUDA graph.
+ * mg_gmres_finish(k): R y = g over the first k columns, x += sum_{c<k} y_c z_c (params == NULL: v_c).
+ * comm != NULL: levels[0] is row-partitioned (d_x, d_V and d_Z vectors hold n + n_halo entries, ld >= that); start and
+ * iterate are one program each and the dot products are summed over the ranks in rank order. */
+typedef struct {
+    double *d_x;          /* ld: the solution, level-0 ordering                                          */
+    double *d_V, *d_Z;    /* (restart + 1) * ld each                                                     */
+    int64_t ld;           /* >= n (+ halo), a multiple of 32                                             */
+    int32_t restart, pad_;
+    double *d_H;          /* (restart + 1) * restart                                                     */
+    double *d_g, *d_cs, *d_sn;  /* restart + 1 each                                                      */
+    double *d_y;          /* restart + 1: y; during an iteration the rank's own dot products             */
+    double *d_scalars;    /* 8 doubles                                                                   */
+    double *d_partials;   /* max(mg_norm_workspace_size(n), mg_krylov_partials(n, restart + 1)) doubles  */
+    double *d_slots;      /* MG_MAX_RANKS * (restart + 1) doubles (partitioned runs; NULL otherwise)     */
+} mg_gmres;
+int mg_gmres_start(mg_comm *comm, const mg_level *levels, const mg_gmres *gmres, void *stream);
+int mg_gmres_iterate(mg_comm *comm, const mg_level *levels, int nlevels, const mg_cycle_params *params,
+                     const mg_gmres *gmres, int j, void *stream);
+int mg_gmres_finish(const mg_level *levels, const mg_cycle_params *params, const mg_gmres *gmres, int k, void *stream);
+/* The building blocks (csrc/krylov_kernels.cu) on their own; V holds m vectors of n entries at a stride ld.
+ * mg_krylov_partials: doubles of d_partials the two below need for n rows and m vectors. */
+int64_t mg_krylov_partials(int64_t n, int32_t m);
+/* d_out[k] = v_k . w, k < m, in a fixed order */
+int mg_multi_dot(int64_t n, const double *d_V, int64_t ld, int32_t m, const double *d_w, double *d_partials,
+                 double *d_out, void *stream);
+/* w -= h_k v_k for k = 0, 1, ..., m-1 (each product and difference rounded), then *d_norm2 = ||w||^2 */
+int mg_multi_axpy_norm(int64_t n, const double *d_V, int64_t ld, int32_t m, const double *d_h, double *d_w,
+                       double *d_partials, double *d_norm2, void *stream);
+/* v /= *d_h, nothing when *d_h == 0 */
+int mg_scale_inv(int64_t n, const double *d_h, double *d_v, void *stream);
+/* y = R^-1 g (R: upper triangle of the first k columns of d_H, leading dimension ldh), then x += y_c z_c, c = 0..k-1 */
+int mg_gmres_solve_update(int64_t n, const double *d_H, int32_t ldh, const double *d_g, int32_t k, double *d_y,
+                          const double *d_Z, int64_t ld, double *d_x, void *stream);
 /* number of kernels the last mg_vcycle call on this thread launched (bench.py's gpu_launches) */
 int64_t mg_last_launch_count(void);
 /* CUDA-graph helpers: capture whatever is enqueued on `stream` between begin and end. */

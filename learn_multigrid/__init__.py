@@ -5,7 +5,7 @@ import importlib
 import sys
 
 _SUBMODULES = [
-    "solvers", "solvers.Solver", "solvers.Jacobi", "solvers.GaussSeidel", "solvers.CG", "solvers.Multigrid",
+    "solvers", "solvers.Solver", "solvers.Jacobi", "solvers.GaussSeidel", "solvers.CG", "solvers.GMRES", "solvers.Multigrid",
     "L2_projection", "L2_projection.L2Projection", "L2_projection.CouplingOperator", "L2_projection.Intersection",
     "assembly", "assembly.MassMatrix", "assembly.StiffnessMatrix", "assembly.LoadVector", "assembly.LoadFunction",
     "assembly.Quadrature", "assembly.ShapeFunction", "assembly.MapReferenceElement",

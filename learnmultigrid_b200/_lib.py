@@ -85,6 +85,12 @@ class mg_pcg(ctypes.Structure):
                 ("d_slots", c_vp)]
 
 
+class mg_gmres(ctypes.Structure):
+    _fields_ = [("d_x", c_vp), ("d_V", c_vp), ("d_Z", c_vp), ("ld", c_i64), ("restart", ctypes.c_int32),
+                ("pad_", ctypes.c_int32), ("d_H", c_vp), ("d_g", c_vp), ("d_cs", c_vp), ("d_sn", c_vp), ("d_y", c_vp),
+                ("d_scalars", c_vp), ("d_partials", c_vp), ("d_slots", c_vp)]
+
+
 class mg_level(ctypes.Structure):
     _fields_ = [("n", c_i64), ("A", mg_sell), ("d_dinv", c_vp),
                 ("ncolors", ctypes.c_int32), ("h_color_ptr", ctypes.POINTER(c_i64)),
@@ -143,6 +149,17 @@ _SIGNATURES = {
     "mg_pcg_start": (c_int, [c_vp, ctypes.POINTER(mg_level), ctypes.POINTER(mg_pcg), c_vp]),
     "mg_pcg_iterate": (c_int, [c_vp, ctypes.POINTER(mg_level), c_int, ctypes.POINTER(mg_cycle_params),
                                ctypes.POINTER(mg_pcg), c_int, c_vp]),
+    "mg_gmres_start": (c_int, [c_vp, ctypes.POINTER(mg_level), ctypes.POINTER(mg_gmres), c_vp]),
+    "mg_gmres_iterate": (c_int, [c_vp, ctypes.POINTER(mg_level), c_int, ctypes.POINTER(mg_cycle_params),
+                                 ctypes.POINTER(mg_gmres), c_int, c_vp]),
+    "mg_gmres_finish": (c_int, [ctypes.POINTER(mg_level), ctypes.POINTER(mg_cycle_params), ctypes.POINTER(mg_gmres),
+                                c_int, c_vp]),
+    "mg_krylov_partials": (c_i64, [c_i64, ctypes.c_int32]),
+    "mg_multi_dot": (c_int, [c_i64, c_vp, c_i64, ctypes.c_int32, c_vp, c_vp, c_vp, c_vp]),
+    "mg_multi_axpy_norm": (c_int, [c_i64, c_vp, c_i64, ctypes.c_int32, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "mg_scale_inv": (c_int, [c_i64, c_vp, c_vp, c_vp]),
+    "mg_gmres_solve_update": (c_int, [c_i64, c_vp, ctypes.c_int32, c_vp, ctypes.c_int32, c_vp, c_vp, c_i64, c_vp,
+                                      c_vp]),
     "mg_set_implied_columns": (c_int, [c_int]),
     "mg_set_implied_transfers": (c_int, [c_int]),
     "mg_sell_residual": (c_int, [ctypes.POINTER(mg_sell), c_vp, c_vp, c_vp, c_vp]),
@@ -200,6 +217,7 @@ _SIGNATURES = {
     "mg_comm_begin": (c_int, [ctypes.POINTER(mg_comm)]),
     "mg_comm_exchange": (c_int, [ctypes.POINTER(mg_comm), ctypes.POINTER(mg_xfer), c_vp, c_vp, c_vp]),
     "mg_comm_allreduce_sum": (c_int, [ctypes.POINTER(mg_comm), c_vp, c_vp, c_vp, c_vp]),
+    "mg_comm_allreduce_sum_n": (c_int, [ctypes.POINTER(mg_comm), c_vp, ctypes.c_int32, c_vp, c_vp, c_vp]),
     "mg_comm_end": (c_int, [ctypes.POINTER(mg_comm), c_vp]),
     "mg_comm_error": (c_int, [ctypes.POINTER(mg_comm), ctypes.POINTER(ctypes.c_int32), c_vp]),
     "mg_csr_remap_cols": (c_int, [c_i64, c_vp, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp]),

@@ -48,6 +48,15 @@ __global__ void sum_slots_kernel(const double *value, const double *slots, int r
         *out = s;
     }
 }
+// the same for k values per rank: out[i] = sum_q (q == rank ? value[i] : slots[q * k + i]) in rank order, i < k
+__global__ void sum_slots_n_kernel(const double *value, const double *slots, int k, int rank, int world, double *out) {
+    pdl_prologue();
+    for (int i = threadIdx.x; i < k; i += blockDim.x) {
+        double s = 0.0;
+        for (int q = 0; q < world; ++q) s += (q == rank) ? value[i] : slots[(int64_t)q * k + i];
+        out[i] = s;
+    }
+}
 
 // column relabelling of a row block: global column -> local [owned (permuted) | halo] index through a lookup table:
 // slot_of[c] = halo slot (>= 0) or -1
@@ -210,23 +219,33 @@ int mg_comm_begin(mg_comm *comm) {
 int mg_comm_exchange(mg_comm *comm, const mg_xfer *xfer, const double *d_src, double *d_dst, void *stream) {
     return comm_exchange(comm, xfer, d_src, d_dst, (cudaStream_t)stream);
 }
-int mg_comm_allreduce_sum(mg_comm *comm, const double *d_value, double *d_slots, double *d_out, void *stream) {
-    MG_REQUIRE(comm && d_value && d_slots && d_out, "null argument");
+int mg_comm_allreduce_sum_n(mg_comm *comm, const double *d_values, int32_t k, double *d_slots, double *d_out,
+                            void *stream) {
+    MG_REQUIRE(comm && d_values && d_slots && d_out, "null argument");
+    MG_REQUIRE(k >= 1, "need at least one value");
     mg_xfer x;
     memset(&x, 0, sizeof(x));
     for (int q = 0; q < comm->world; ++q) {
         if (q == comm->rank) continue;
-        const int k = x.npeers++;
-        x.peer[k] = q;
-        x.send_cnt[k] = 1;
-        x.recv_off[k] = q;
-        x.recv_cnt[k] = 1;
+        const int p = x.npeers++;
+        x.peer[p] = q;
+        x.send_cnt[p] = k;
+        x.recv_off[p] = (int64_t)q * k;
+        x.recv_cnt[p] = k;
     }
-    int rc = comm_exchange(comm, &x, d_value, d_slots, (cudaStream_t)stream);
+    int rc = comm_exchange(comm, &x, d_values, d_slots, (cudaStream_t)stream);
     if (rc) return rc;
-    launch_k(sum_slots_kernel, (unsigned)(1), (unsigned)32, (cudaStream_t)stream, d_value, d_slots, comm->rank, comm->world, d_out);
+    if (k == 1)     // the single-value kernel of the V-cycle norm and of CG
+        launch_k(sum_slots_kernel, 1u, 32u, (cudaStream_t)stream, d_values, (const double *)d_slots, comm->rank,
+                 comm->world, d_out);
+    else
+        launch_k(sum_slots_n_kernel, 1u, 32u, (cudaStream_t)stream, d_values, (const double *)d_slots, (int)k,
+                 comm->rank, comm->world, d_out);
     MG_CHECK_LAUNCH("sum_slots");
     return MG_OK;
+}
+int mg_comm_allreduce_sum(mg_comm *comm, const double *d_value, double *d_slots, double *d_out, void *stream) {
+    return mg_comm_allreduce_sum_n(comm, d_value, 1, d_slots, d_out, stream);
 }
 int mg_comm_end(mg_comm *comm, void *stream) {
     MG_REQUIRE(comm && comm->d_arena[comm->rank], "null communicator");

@@ -6,6 +6,8 @@
 // cycle, are hoisted to setup; the arithmetic of a cycle is unchanged.
 #include "sell_api.cuh"
 
+#include <vector>
+
 namespace mgb {
 
 int comm_prepare(mg_comm *, const mg_xfer *, const double *, double *, ExArgs *, int *);
@@ -39,6 +41,13 @@ int vec_pcg_direction(int64_t, const double *, double *, const double *, int, cu
 int vec_pcg_update(int64_t, const double *, const double *, double *, double *, const double *, double *, int *, cudaStream_t);
 int vec_pcg_scalar(int, int, double *, const double *, cudaStream_t);
 int comm_exchange(mg_comm *, const mg_xfer *, const double *, double *, cudaStream_t);
+int krylov_multi_dot(int64_t, const double *, int64_t, int, const double *, double *, double *, cudaStream_t);
+int krylov_multi_axpy_norm(int64_t, const double *, int64_t, int, const double *, double *, double *, double *, cudaStream_t);
+int krylov_scale_inv(int64_t, const double *, double *, cudaStream_t);
+int krylov_gmres_start(const double *, double *, int, double *, cudaStream_t);
+int krylov_givens(double *, int, int, double *, double *, double *, const double *, double *, cudaStream_t);
+int krylov_solve_update(int64_t, const double *, int, const double *, int, double *, const double *, int64_t, double *,
+                        cudaStream_t);
 
 #define MG_TRY(expr)            \
     do {                        \
@@ -384,6 +393,7 @@ int64_t mg_struct_size(int which) {
         case 6: return sizeof(mg_dist_level);
         case 7: return sizeof(mg_bcr_dist);
         case 8: return sizeof(mg_dist_norm);
+        case 9: return sizeof(mg_gmres);
         default: return -1;
     }
 }
@@ -540,6 +550,113 @@ int mg_pcg_iterate(mg_comm *comm, const mg_level *levels, int nlevels, const mg_
     }
     g_last_cycle_launches = g_launch_count - before;
     return MG_OK;
+}
+
+/* ---- restarted GMRES, right-preconditioned by one V-cycle per Arnoldi step (include/mgb200.h, mg_gmres) ---------------
+ * Launch sequences only, the scalars on the device; after each call the host reads d_scalars[0] (8 bytes). */
+static int check_gmres(const mg_level *levels, const mg_gmres *G) {
+    MG_REQUIRE(levels && G && G->d_x && G->d_V && G->d_Z && G->d_H && G->d_g && G->d_cs && G->d_sn && G->d_y &&
+                   G->d_scalars && G->d_partials, "mg_gmres: null member");
+    MG_REQUIRE(G->restart >= 1, "mg_gmres: restart must be >= 1");
+    const mg_level &L = levels[0];
+    MG_REQUIRE(L.n > 0 && L.d_b, "level vectors missing");
+    MG_REQUIRE(G->ld >= vec_len(L) && G->ld % 32 == 0, "mg_gmres: ld must cover the level vector and be a multiple of 32");
+    return MG_OK;
+}
+// local sums -> the sums over all ranks (in place when there is one rank)
+static int gmres_allreduce(mg_comm *comm, const mg_gmres *G, double *local, int k, double *out, cudaStream_t st) {
+    MG_REQUIRE(G->d_slots, "mg_gmres.d_slots missing");
+    MG_TRY(flush_pending(comm, st));
+    return mg_comm_allreduce_sum_n(comm, local, k, G->d_slots, out, st);
+}
+int mg_gmres_start(mg_comm *comm, const mg_level *levels, const mg_gmres *gmres, void *stream) {
+    MG_TRY(check_gmres(levels, gmres));
+    cudaStream_t st = (cudaStream_t)stream;
+    const mg_level &L = levels[0];
+    MG_REQUIRE(!L.dist || comm, "partitioned level without a communicator");
+    const bool multi = comm && comm->world > 1;
+    if (comm) {
+        MG_TRY(mg_comm_begin(comm));
+        g_pend.x = nullptr;
+    }
+    double *r = gmres->d_V, *sc = gmres->d_scalars;
+    SellFuse f;
+    bool use = false;
+    if (L.dist) {
+        MG_TRY(issue_exchange(comm, L.dist->xfer_all, gmres->d_x, true, st));       // the residual reads halo entries of x
+        MG_TRY(take_pending(comm, gmres->d_x, &L.A, 0, L.A.nrows, L.dist->d_mask_A, &f, &use, st));
+    }
+    MG_TRY(sell_residual(&L.A, gmres->d_x, L.d_b, r, 0, L.A.nrows, use ? &f : nullptr, st));     // r = b - A x
+    MG_TRY(flush_pending(comm, st));
+    int nb = 0;
+    MG_TRY(vec_dot_partials(L.n, r, r, gmres->d_partials, &nb, st));
+    MG_TRY(sell_reduce_partials(gmres->d_partials, nb, sc + 2, st));
+    if (multi) MG_TRY(gmres_allreduce(comm, gmres, sc + 2, 1, sc + 3, st));
+    MG_TRY(krylov_gmres_start(multi ? sc + 3 : sc + 2, gmres->d_g, gmres->restart, sc, st));   // g = beta e_1
+    MG_TRY(krylov_scale_inv(L.n, sc + 1, r, st));                                              // v_0 = r / beta
+    if (comm) {
+        MG_TRY(flush_pending(comm, st));
+        g_pend.x = nullptr;
+        MG_TRY(mg_comm_end(comm, stream));
+    }
+    return MG_OK;
+}
+int mg_gmres_iterate(mg_comm *comm, const mg_level *levels, int nlevels, const mg_cycle_params *params,
+                     const mg_gmres *gmres, int j, void *stream) {
+    MG_TRY(check_gmres(levels, gmres));
+    MG_REQUIRE(j >= 0 && j < gmres->restart, "mg_gmres_iterate: step outside the cycle");
+    if (params) MG_TRY(check_levels(levels, nlevels, params, comm != nullptr));
+    cudaStream_t st = (cudaStream_t)stream;
+    const mg_level &L = levels[0];
+    MG_REQUIRE(!L.dist || comm, "partitioned level without a communicator");
+    const bool multi = comm && comm->world > 1;
+    const int64_t before = g_launch_count;
+    if (comm) {
+        MG_TRY(mg_comm_begin(comm));
+        g_pend.x = nullptr;
+    }
+    const int64_t ld = gmres->ld;
+    double *vj = gmres->d_V + (int64_t)j * ld, *w = vj + ld, *sc = gmres->d_scalars;
+    double *z = vj;
+    if (params) {
+        // z_j = M^-1 v_j: the cycle runs on a copy of the level structs whose level 0 reads v_j and writes z_j, so
+        // neither vector is copied.  Every smoother leaves its result in d_x (vcycle_rec picks the start buffer).
+        std::vector<mg_level> lv(levels, levels + nlevels);
+        z = gmres->d_Z + (int64_t)j * ld;
+        lv[0].d_b = vj;
+        lv[0].d_x = z;
+        mg_cycle_params P = *params;
+        P.x0_zero = 1;
+        MG_TRY(vcycle_rec(comm, lv.data(), nlevels, 0, P, st));
+    } else if (L.dist) {
+        MG_TRY(issue_exchange(comm, L.dist->xfer_all, vj, true, st));             // the SpMV reads halo entries of v_j
+    }
+    SellFuse f;
+    bool use = false;
+    if (L.dist) MG_TRY(take_pending(comm, z, &L.A, 0, L.A.nrows, L.dist->d_mask_A, &f, &use, st));
+    MG_TRY(sell_spmv(&L.A, z, w, 0, L.A.nrows, use ? &f : nullptr, st));           // w = A z_j in slot j+1
+    MG_TRY(flush_pending(comm, st));
+    const int m = j + 1, ldh = gmres->restart + 1;
+    double *hcol = gmres->d_H + (int64_t)j * ldh;
+    MG_TRY(krylov_multi_dot(L.n, gmres->d_V, ld, m, w, gmres->d_partials, multi ? gmres->d_y : hcol, st));
+    if (multi) MG_TRY(gmres_allreduce(comm, gmres, gmres->d_y, m, hcol, st));
+    MG_TRY(krylov_multi_axpy_norm(L.n, gmres->d_V, ld, m, hcol, w, gmres->d_partials, sc + 2, st));
+    if (multi) MG_TRY(gmres_allreduce(comm, gmres, sc + 2, 1, sc + 3, st));
+    MG_TRY(krylov_givens(gmres->d_H, ldh, j, gmres->d_cs, gmres->d_sn, gmres->d_g, multi ? sc + 3 : sc + 2, sc, st));
+    MG_TRY(krylov_scale_inv(L.n, sc + 1, w, st));                                  // v_{j+1} = w / h_{j+1,j}
+    if (comm) {
+        MG_TRY(flush_pending(comm, st));
+        g_pend.x = nullptr;
+        MG_TRY(mg_comm_end(comm, stream));
+    }
+    g_last_cycle_launches = g_launch_count - before;
+    return MG_OK;
+}
+int mg_gmres_finish(const mg_level *levels, const mg_cycle_params *params, const mg_gmres *gmres, int k, void *stream) {
+    MG_TRY(check_gmres(levels, gmres));
+    MG_REQUIRE(k >= 0 && k <= gmres->restart, "mg_gmres_finish: more steps than the cycle holds");
+    return krylov_solve_update(levels[0].n, gmres->d_H, gmres->restart + 1, gmres->d_g, k, gmres->d_y,
+                               params ? gmres->d_Z : gmres->d_V, gmres->ld, gmres->d_x, (cudaStream_t)stream);
 }
 
 int mg_graph_begin(void *stream) {

@@ -725,6 +725,138 @@ class DeviceHierarchy:
                                 "iterations": its}
         return sol, track, its
 
+    def gmres(self, rhs, params, error=1e-8, max_iterations=1000, restart=30, x0=None, view=False):
+        """Restarted GMRES(restart), right-preconditioned by one V-cycle from zero per Arnoldi step (params=None: no
+        preconditioner), entirely in the level-0 ordering of this hierarchy and on the device (mg_gmres_start /
+        mg_gmres_iterate / mg_gmres_finish): classical Gram-Schmidt in one pass, Givens rotations, the scalars on the
+        device; a step is one CUDA graph (per step index and parameter set; index-order Gauss-Seidel runs uncaptured)
+        after which the host reads 8 bytes.  Valid for nonsymmetric operators and preconditioners, unlike pcg.
+        Works on a partitioned hierarchy too (every rank makes the same call; dots are summed over the ranks in rank
+        order).
+
+        error is absolute, as in pcg.  The history is ||b - A x0||, then the GMRES estimate |g_{j+1}| of the residual
+        after every step.  At every restart, and when the estimate reaches `error`, x is updated and the true residual
+        recomputed; while it is above `error` and steps remain, the solve restarts from there.  max_iterations counts
+        Arnoldi steps over all restarts; when it runs out, x is the iterate of the last completed step.
+        Returns (solution (n,1) natural order -- this rank's block when partitioned --, history list, steps, true
+        residual of the solution); self.last_gmres_timing holds the wall-clock split transfer in / iterations /
+        transfer out (orthogonalisation: None, the steps run as graphs; tools/bench_gmres.py times its kernels)."""
+        import time
+        torch, lib = self.torch, self.lib
+        restart = int(restart)
+        if restart < 1:
+            raise ValueError("restart must be >= 1 (got %d)" % restart)
+        lev = self.levels[0]
+        n = self.n
+        st = _lib.stream_handle(torch)
+        comm = self._comm_ptr()
+        ws = getattr(self, "_gm", None)
+        if ws is None or ws["restart"] != restart:
+            self._gm = None
+            for key in [k for k in self._graphs if k[0] == "gmres"]:
+                lib.mg_graph_destroy(self._graphs.pop(key)[0])
+            ws = self._gm = self._gmres_workspace(restart, n, getattr(lev, "n_vec", n))
+        G = ctypes.byref(ws["struct"])
+        pp = None if params is None else ctypes.byref(params)
+        sc = ws["scalars"]
+
+        def read_r2():
+            self._norm_host.copy_(sc[0:1], non_blocking=True)
+            torch.cuda.current_stream().synchronize()
+            return float(np.sqrt(self._norm_host.item()))
+
+        pkey = None if params is None else (params.smoother, params.nu_pre, params.nu_post, params.omega,
+                                            params.zero_guess_skip, params.reverse_post, self._cheby_key)
+
+        def iterate(j):
+            key = ("gmres", j, pkey)
+            g = self._graphs.get(key)
+            if g is None:
+                if self.smoother == "lexgs" and params is not None:      # cooperative launches are not captured
+                    _lib.check(lib.mg_gmres_iterate(comm, self._level_structs, self.nlevels, pp, G, j, st),
+                               "mg_gmres_iterate")
+                    return
+                cap = torch.cuda.Stream(device=self.device)
+                cap.wait_stream(torch.cuda.current_stream())
+                with torch.cuda.stream(cap):
+                    h = cap.cuda_stream
+                    _lib.check(lib.mg_graph_begin(h), "mg_graph_begin")
+                    rc = lib.mg_gmres_iterate(comm, self._level_structs, self.nlevels, pp, G, j, h)
+                    out = ctypes.c_void_p()
+                    rc2 = lib.mg_graph_end(h, ctypes.byref(out))
+                    _lib.check(rc, "mg_gmres_iterate (capture)")
+                    _lib.check(rc2, "mg_graph_end")
+                torch.cuda.current_stream().wait_stream(cap)
+                g = self._graphs[key] = (out, 0)
+            _lib.check(lib.mg_graph_launch(g[0], st), "mg_graph_launch")
+
+        t0 = time.perf_counter()
+        self.set_rhs(rhs)
+        x = ws["x"]
+        if x0 is None:
+            x.zero_()
+        else:
+            self._to_level0(x0, x)
+        torch.cuda.current_stream().synchronize()
+        t1 = time.perf_counter()
+        its = 0
+        track = []
+        while True:
+            _lib.check(lib.mg_gmres_start(comm, self._level_structs, G, st), "mg_gmres_start")    # true residual
+            res = read_r2()
+            if not track:
+                track.append(res)
+            if res <= error or its >= max_iterations:
+                break
+            k = 0
+            while k < restart and its < max_iterations:
+                iterate(k)
+                its += 1
+                k += 1
+                est = read_r2()
+                track.append(est)
+                if est <= error:
+                    break
+            _lib.check(lib.mg_gmres_finish(self._level_structs, pp, G, k, st), "mg_gmres_finish")
+        t2 = time.perf_counter()
+        sol = self._from_level0(x, view)
+        t3 = time.perf_counter()
+        self.last_gmres_timing = {"transfer_in_s": t1 - t0, "iterations_s": t2 - t1, "orthogonalisation_s": None,
+                                  "transfer_out_s": t3 - t2, "iterations": its}
+        return sol, track, its, res
+
+    def gmres_residual_vector(self):
+        """b - A x of the last gmres solution, (n,1) natural order (this rank's block when partitioned: the halo of x
+        is current, the last mg_gmres_start exchanged it)"""
+        lev = self.levels[0]
+        _lib.check(self.lib.mg_sell_residual(ctypes.byref(lev.A.struct), self._gm["x"].data_ptr(), lev.b.data_ptr(),
+                                             lev.r.data_ptr(), _lib.stream_handle(self.torch)), "mg_sell_residual")
+        return self._from_level0(lev.r)
+
+    def _gmres_workspace(self, restart, n, n_vec):
+        """device buffers of mg_gmres for one restart length; ValueError when the two bases do not fit"""
+        torch, lib, dev = self.torch, self.lib, self.device
+        ld = (n_vec + 31) // 32 * 32
+        m = restart + 1
+        parts = max(int(lib.mg_norm_workspace_size(n)), int(lib.mg_krylov_partials(n, m)))
+        small = 4 * m + m * restart + 8 + parts + _lib.MG_MAX_RANKS * m
+        need = 8 * (2 * m * ld + ld + small)
+        free, _ = torch.cuda.mem_get_info(dev)
+        free += torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)     # cached by torch, reusable
+        if need > free:
+            raise ValueError("GMRES(%d) needs %d bytes of device memory for its bases (2 x %d vectors of %d entries), "
+                             "%d are free" % (restart, need, m, ld, free))
+        f64 = dict(dtype=torch.float64, device=dev)
+        ws = {"restart": restart, "x": torch.zeros(ld, **f64), "V": torch.zeros(m * ld, **f64),
+              "Z": torch.zeros(m * ld, **f64), "H": torch.zeros(m * restart, **f64), "g": torch.zeros(m, **f64),
+              "cs": torch.zeros(m, **f64), "sn": torch.zeros(m, **f64), "y": torch.zeros(m, **f64),
+              "scalars": torch.zeros(8, **f64), "partials": torch.zeros(parts, **f64),
+              "slots": torch.zeros(_lib.MG_MAX_RANKS * m, **f64)}
+        ws["struct"] = _lib.mg_gmres(*(ws[k].data_ptr() for k in ("x", "V", "Z")), ld, restart, 0,
+                                     *(ws[k].data_ptr() for k in ("H", "g", "cs", "sn", "y", "scalars", "partials",
+                                                                  "slots")))
+        return ws
+
     def __del__(self):
         try:
             for g, _ in self._graphs.values():

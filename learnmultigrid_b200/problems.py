@@ -87,6 +87,34 @@ def structured_laplacian_2d(N, coefficient=None, rows=None, Ny=None):
     return F.raw_csr(indptr.astype(np.int32), indices, data, (r1 - r0, n))
 
 
+def convection_diffusion_2d(N, eps, beta):
+    """-eps * Laplace(u) + beta . grad(u) on the mesh of structured_laplacian_2d(N), scaled like it (by h^2): the
+    5-point diffusion stencil times eps plus first-order upwind convection times h (for beta_x > 0 the row gets
+    +h beta_x on the diagonal and -h beta_x on its west neighbour, for beta_x < 0 the same with |beta_x| and the east
+    neighbour; likewise in y).  Boundary rows are identity rows as in structured_laplacian_2d, so for beta != 0 the
+    operator is nonsymmetric twice over; eps = 1, beta = (0, 0) gives structured_laplacian_2d(N) entry for entry.
+    Interior rows sum to zero, the diagonal is positive and the off-diagonals are negative (an M-matrix).
+    Canonical CSR."""
+    eps = float(eps)
+    bx, by = (float(v) for v in beta)
+    if not eps > 0.0:
+        raise ValueError("eps must be positive")
+    A = structured_laplacian_2d(N)
+    h = 1.0 / N
+    base = A.indptr[:-1][np.diff(A.indptr) == 5].astype(np.int64)    # interior rows: (south, west, diag, east, north)
+    d = A.data
+    idx = base[:, None] + np.arange(5)
+    d[idx] = eps * d[idx]
+    for b, lo, hi in ((bx, 1, 3), (by, 0, 4)):               # (component, upwind slot for b > 0, for b < 0)
+        c = h * abs(b)
+        if c == 0.0:
+            continue
+        d[base + 2] = d[base + 2] + c
+        up = lo if b > 0 else hi
+        d[base + up] = d[base + up] - c
+    return A
+
+
 def structured_rhs_2d(N, f_value=-1.0, rows=None, Ny=None):
     """load vector of f = const on the structured mesh with Dirichlet rows zeroed: interior entries f*h^2
     (six triangles of area h^2/2, each contributing f*area/3), thesis_structured_2d.py:17-19,403,414.

@@ -98,6 +98,21 @@ static int take_pending(mg_comm *comm, const double *xop, const mg_sell *M, int6
     return MG_OK;
 }
 
+// The bracket of every exported launch sequence that may exchange (comm != NULL; without a communicator both are
+// no-ops): the communicator's sites are numbered from the start of the program, nothing is pending on entry, and on
+// exit every halo is current (flush_pending leaves nothing pending) before mg_comm_end closes the program.
+static int program_begin(mg_comm *comm) {
+    if (!comm) return MG_OK;
+    MG_TRY(mg_comm_begin(comm));
+    g_pend.x = nullptr;
+    return MG_OK;
+}
+static int program_end(mg_comm *comm, cudaStream_t st) {
+    if (!comm) return MG_OK;
+    MG_TRY(flush_pending(comm, st));
+    return mg_comm_end(comm, st);
+}
+
 // Row-partitioned levels (mg_level.dist != NULL, SURVEY 8e): L.n counts the OWNED rows, the level vectors carry
 // dist->n_halo more entries behind them, and every kernel that changes a vector other ranks read is followed by an
 // exchange of the boundary values.  Invariant: the halo of the iterate is current on entry to and on return from
@@ -438,8 +453,7 @@ int mg_vcycle_dist(mg_comm *comm, const mg_level *levels, int nlevels, const mg_
     else MG_REQUIRE(levels && nlevels >= 1, "no level");
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t before = g_launch_count;
-    MG_TRY(mg_comm_begin(comm));
-    g_pend.x = nullptr;
+    MG_TRY(program_begin(comm));
     int rc = MG_OK;
     if (norm) MG_REQUIRE(norm->d_partials && norm->d_local && norm->d_slots && norm->d_norm2, "norm workspace missing");
     const bool after = norm && norm->after && params;
@@ -461,9 +475,7 @@ int mg_vcycle_dist(mg_comm *comm, const mg_level *levels, int nlevels, const mg_
         rc = flush_pending(comm, st);
         if (!rc) rc = finish_norm(no.nblocks);
     }
-    if (!rc) rc = flush_pending(comm, st);      // the halo of the iterate is current when the program ends
-    g_pend.x = nullptr;
-    if (!rc) rc = mg_comm_end(comm, stream);
+    if (!rc) rc = program_end(comm, st);
     g_last_cycle_launches = g_launch_count - before;
     return rc;
 }
@@ -497,16 +509,12 @@ int mg_pcg_start(mg_comm *comm, const mg_level *levels, const mg_pcg *pcg, void 
     MG_TRY(check_pcg(levels, pcg));
     cudaStream_t st = (cudaStream_t)stream;
     const mg_level &L = levels[0];
-    if (comm) {
-        MG_TRY(mg_comm_begin(comm));
-        g_pend.x = nullptr;
-        }
+    MG_TRY(program_begin(comm));
     MG_TRY(vec_fill(L.n, 0.0, pcg->d_x, st));
     int nb = 0;
     MG_TRY(vec_dot_partials(L.n, L.d_b, L.d_b, pcg->d_partials, &nb, st));
     MG_TRY(pcg_reduce(comm, pcg, nb, 0, 0, st));
-    if (comm) MG_TRY(mg_comm_end(comm, stream));
-    return MG_OK;
+    return program_end(comm, st);
 }
 int mg_pcg_iterate(mg_comm *comm, const mg_level *levels, int nlevels, const mg_cycle_params *params, const mg_pcg *pcg,
                    int first, void *stream) {
@@ -516,10 +524,7 @@ int mg_pcg_iterate(mg_comm *comm, const mg_level *levels, int nlevels, const mg_
     const mg_level &L = levels[0];
     MG_REQUIRE(!L.dist || comm, "partitioned level without a communicator");
     const int64_t before = g_launch_count;
-    if (comm) {
-        MG_TRY(mg_comm_begin(comm));
-        g_pend.x = nullptr;
-        }
+    MG_TRY(program_begin(comm));
     double *r = L.d_b;
     const double *z = r;
     if (params) {                               // z = M^-1 r: one V-cycle on (x, b) = (0, r), z lands in d_x
@@ -543,11 +548,7 @@ int mg_pcg_iterate(mg_comm *comm, const mg_level *levels, int nlevels, const mg_
     MG_TRY(pcg_reduce(comm, pcg, nb, 2, 0, st));                              // alpha = r.z / p.Ap
     MG_TRY(vec_pcg_update(L.n, pcg->d_p, pcg->d_Ap, pcg->d_x, r, pcg->d_scalars, pcg->d_partials, &nb, st));
     MG_TRY(pcg_reduce(comm, pcg, nb, 0, 0, st));                              // r.r of the new residual
-    if (comm) {
-        MG_TRY(flush_pending(comm, st));
-        g_pend.x = nullptr;
-            MG_TRY(mg_comm_end(comm, stream));
-    }
+    MG_TRY(program_end(comm, st));
     g_last_cycle_launches = g_launch_count - before;
     return MG_OK;
 }
@@ -575,10 +576,7 @@ int mg_gmres_start(mg_comm *comm, const mg_level *levels, const mg_gmres *gmres,
     const mg_level &L = levels[0];
     MG_REQUIRE(!L.dist || comm, "partitioned level without a communicator");
     const bool multi = comm && comm->world > 1;
-    if (comm) {
-        MG_TRY(mg_comm_begin(comm));
-        g_pend.x = nullptr;
-    }
+    MG_TRY(program_begin(comm));
     double *r = gmres->d_V, *sc = gmres->d_scalars;
     SellFuse f;
     bool use = false;
@@ -594,12 +592,7 @@ int mg_gmres_start(mg_comm *comm, const mg_level *levels, const mg_gmres *gmres,
     if (multi) MG_TRY(gmres_allreduce(comm, gmres, sc + 2, 1, sc + 3, st));
     MG_TRY(krylov_gmres_start(multi ? sc + 3 : sc + 2, gmres->d_g, gmres->restart, sc, st));   // g = beta e_1
     MG_TRY(krylov_scale_inv(L.n, sc + 1, r, st));                                              // v_0 = r / beta
-    if (comm) {
-        MG_TRY(flush_pending(comm, st));
-        g_pend.x = nullptr;
-        MG_TRY(mg_comm_end(comm, stream));
-    }
-    return MG_OK;
+    return program_end(comm, st);
 }
 int mg_gmres_iterate(mg_comm *comm, const mg_level *levels, int nlevels, const mg_cycle_params *params,
                      const mg_gmres *gmres, int j, void *stream) {
@@ -611,10 +604,7 @@ int mg_gmres_iterate(mg_comm *comm, const mg_level *levels, int nlevels, const m
     MG_REQUIRE(!L.dist || comm, "partitioned level without a communicator");
     const bool multi = comm && comm->world > 1;
     const int64_t before = g_launch_count;
-    if (comm) {
-        MG_TRY(mg_comm_begin(comm));
-        g_pend.x = nullptr;
-    }
+    MG_TRY(program_begin(comm));
     const int64_t ld = gmres->ld;
     double *vj = gmres->d_V + (int64_t)j * ld, *w = vj + ld, *sc = gmres->d_scalars;
     double *z = vj;
@@ -644,11 +634,7 @@ int mg_gmres_iterate(mg_comm *comm, const mg_level *levels, int nlevels, const m
     if (multi) MG_TRY(gmres_allreduce(comm, gmres, sc + 2, 1, sc + 3, st));
     MG_TRY(krylov_givens(gmres->d_H, ldh, j, gmres->d_cs, gmres->d_sn, gmres->d_g, multi ? sc + 3 : sc + 2, sc, st));
     MG_TRY(krylov_scale_inv(L.n, sc + 1, w, st));                                  // v_{j+1} = w / h_{j+1,j}
-    if (comm) {
-        MG_TRY(flush_pending(comm, st));
-        g_pend.x = nullptr;
-        MG_TRY(mg_comm_end(comm, stream));
-    }
+    MG_TRY(program_end(comm, st));
     g_last_cycle_launches = g_launch_count - before;
     return MG_OK;
 }

@@ -564,91 +564,58 @@ class DistributedHierarchy(DeviceHierarchy):
         return self._from_level0(self.levels[0].x, view)
 
     def get_x(self, view=False):
-        """the GLOBAL iterate on every rank (blocks exchanged through the fabric: an API convenience, not a hot path)"""
-        parts = self.fabric.allgather(self.get_x_local().reshape(-1))
-        return np.concatenate(parts).reshape(-1, 1)
+        """the GLOBAL iterate on every rank"""
+        return self.global_rows(self.get_x_local())[0]
+
+    def global_rows(self, *blocks):
+        """this rank's row blocks (n_own,1) of level-0 vectors -> the GLOBAL vectors (n,1), on every rank (blocks
+        exchanged through the fabric: an API convenience, not a hot path).  Every rank must make the same call."""
+        return [np.concatenate(self.fabric.allgather(v.reshape(-1))).reshape(-1, 1) for v in blocks]
 
     # ------------------------------------------------------------------------------------------------
     def residual_norm(self):
         """||b - A x||_2 over all row blocks (Multigrid.py:62-63): fused residual + norm on the owned rows, summed
         over the ranks in rank order by the peer-memory all-reduce; one D2H of 8 bytes."""
-        torch = self.torch
         _lib.check(self.lib.mg_vcycle_dist(ctypes.byref(self.comm.struct), self._level_structs, self.nlevels, None,
-                                           ctypes.byref(self._norm_struct), _lib.stream_handle(torch)),
+                                           ctypes.byref(self._norm_struct), _lib.stream_handle(self.torch)),
                    "mg_vcycle_dist (norm)")
-        self._norm_host.copy_(self._norm_out, non_blocking=True)
-        torch.cuda.current_stream().synchronize()
-        return float(np.sqrt(self._norm_host.item()))
+        return self._read_sqrt(self._norm_out)
 
     def residual_vector(self):
-        lev = self.levels[0]
-        _lib.check(self.lib.mg_sell_residual(ctypes.byref(lev.A.struct), lev.x.data_ptr(), lev.b.data_ptr(),
-                                             lev.r.data_ptr(), _lib.stream_handle(self.torch)), "mg_sell_residual")
-        parts = self.fabric.allgather(self._from_level0(lev.r).reshape(-1))
-        return np.concatenate(parts).reshape(-1, 1)
+        return self.global_rows(super().residual_vector())[0]
 
     def vcycle(self, params, nlevels=None, use_graph=True, with_norm=False, dry=False, norm_after=False):
         """One V-cycle as one program, optionally with the residual norm of the outer loop: with_norm -- of the iterate
         the program starts from, evaluated first; norm_after -- of the iterate the cycle leaves, its last colour's share
         summed by the last sweep (mg_dist_norm.after); read it with last_norm().  Every rank must make the same call.
-        Captured into a CUDA graph per parameter set.  dry=True captures the program with its exchanges disabled
+        Captured into a CUDA graph per parameter set.  dry=True runs the program with its exchanges disabled
         (results are meaningless; bench.py times it to separate kernel time from exchange time)."""
-        torch = self.torch
-        with_norm = bool(with_norm or norm_after)
-        self._norm_struct.after = 1 if norm_after else 0
         if nlevels is not None and int(nlevels) != self.nlevels:
             raise ValueError("a partitioned hierarchy runs all of its levels")
-        L = self.nlevels
-        st = _lib.stream_handle(torch)
+        with_norm = bool(with_norm or norm_after)
+        self._norm_struct.after = 1 if norm_after else 0
         norm = ctypes.byref(self._norm_struct) if with_norm else None
-        comm = ctypes.byref(self.comm.struct)
-        if not use_graph:
-            _lib.check(self.lib.mg_vcycle_dist(comm, self._level_structs, L, ctypes.byref(params), norm, st),
-                       "mg_vcycle_dist")
-            self.last_launches = int(self.lib.mg_last_launch_count())
-            return
-        key = (L, params.smoother, params.nu_pre, params.nu_post, params.omega, params.zero_guess_skip,
-               params.reverse_post, params.x0_zero, bool(with_norm), bool(norm_after), bool(dry), self._cheby_key)
-        g = self._graphs.get(key)
-        if g is None:
-            cap = torch.cuda.Stream(device=self.device)
-            cap.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(cap):
-                h = cap.cuda_stream
-                _lib.check(self.lib.mg_graph_begin(h), "mg_graph_begin")
-                self.comm.struct.dry_run = 1 if dry else 0
-                try:
-                    rc = self.lib.mg_vcycle_dist(comm, self._level_structs, L, ctypes.byref(params), norm, h)
-                finally:
-                    self.comm.struct.dry_run = 0
-                launches = int(self.lib.mg_last_launch_count())
-                out = ctypes.c_void_p()
-                rc2 = self.lib.mg_graph_end(h, ctypes.byref(out))
-                _lib.check(rc, "mg_vcycle_dist (capture)")
-                _lib.check(rc2, "mg_graph_end")
-            torch.cuda.current_stream().wait_stream(cap)
-            g = (out, launches)
-            self._graphs[key] = g
-        _lib.check(self.lib.mg_graph_launch(g[0], st), "mg_graph_launch")
-        self.last_launches = g[1]
+        comm = self.comm.struct
+
+        def enqueue(st):
+            comm.dry_run = 1 if dry else 0
+            try:
+                return self.lib.mg_vcycle_dist(ctypes.byref(comm), self._level_structs, self.nlevels,
+                                               ctypes.byref(params), norm, st)
+            finally:
+                comm.dry_run = 0
+        key = ("vcycle_dist", with_norm, bool(norm_after), bool(dry), self._params_key(params))
+        self.last_launches = self._run(key, enqueue, use_graph and self._capturable(params))
 
     def _comm_ptr(self):
         return ctypes.byref(self.comm.struct)
-
-    def last_norm(self):
-        """sqrt of the squared residual norm the last with_norm program computed (synchronises)"""
-        self._norm_host.copy_(self._norm_out, non_blocking=True)
-        self.torch.cuda.current_stream().synchronize()
-        return float(np.sqrt(self._norm_host.item()))
 
     def check(self):
         self.comm.check()
 
     def close(self):
         try:
-            for g, _ in self._graphs.values():
-                self.lib.mg_graph_destroy(g)
-            self._graphs = {}
+            self.drop_graphs()
         finally:
             self.comm.close()
 

@@ -569,21 +569,20 @@ class DeviceHierarchy:
     # ------------------------------------------------------------------------------------------------
     def residual_norm(self):
         """||b - A x||_2 on level 0, fused residual + norm (Multigrid.py:62-63), one D2H of 8 bytes."""
-        torch = self.torch
         lev = self.levels[0]
-        st = _lib.stream_handle(torch)
         _lib.check(self.lib.mg_sell_residual_norm2(ctypes.byref(lev.A.struct), lev.x.data_ptr(), lev.b.data_ptr(),
-                                                   self._norm_ws.data_ptr(), self._norm_out.data_ptr(), st),
-                   "mg_sell_residual_norm2")
-        self._norm_host.copy_(self._norm_out, non_blocking=True)
-        torch.cuda.current_stream().synchronize()
-        return float(np.sqrt(self._norm_host.item()))
+                                                   self._norm_ws.data_ptr(), self._norm_out.data_ptr(),
+                                                   _lib.stream_handle(self.torch)), "mg_sell_residual_norm2")
+        return self._read_sqrt(self._norm_out)
 
     def last_norm(self):
         """||b - A x||_2 left on the device by vcycle(with_norm=True): one D2H of 8 bytes."""
-        torch = self.torch
-        self._norm_host.copy_(self._norm_out, non_blocking=True)
-        torch.cuda.current_stream().synchronize()
+        return self._read_sqrt(self._norm_out)
+
+    def _read_sqrt(self, dev_slice):
+        """sqrt of the squared norm in the one-element device tensor dev_slice: one D2H of 8 bytes (synchronises)"""
+        self._norm_host.copy_(dev_slice, non_blocking=True)
+        self.torch.cuda.current_stream().synchronize()
         return float(np.sqrt(self._norm_host.item()))
 
     def residual_vector(self):
@@ -600,44 +599,70 @@ class DeviceHierarchy:
         return _lib.mg_cycle_params(sm, int(nu_pre), int(nu_pre if nu_post is None else nu_post), float(omega),
                                     1 if zero_guess_skip else 0, 1 if reverse_post else 0, 1 if x0_zero else 0, 0)
 
-    def _enqueue_cycle(self, L, params, with_norm, stream):
-        if with_norm:
-            return self.lib.mg_vcycle_norm(self._level_structs, L, ctypes.byref(params), self._norm_ws.data_ptr(),
-                                           self._norm_out.data_ptr(), stream)
-        return self.lib.mg_vcycle(self._level_structs, L, ctypes.byref(params), stream)
-
     def vcycle(self, params, nlevels=None, use_graph=True, with_norm=False):
         """One V-cycle on the level-0 vectors (x updated in place).  The launch sequence is captured into a CUDA
         graph the first time a parameter set is used and replayed afterwards.
         with_norm: the cycle also leaves ||b - A x||^2 of the NEW iterate on the device (mg_vcycle_norm: the last
         colour sweep sums its own rows' share from registers); read it with last_norm()."""
-        torch = self.torch
         L = self.nlevels if nlevels is None else int(nlevels)
-        st = _lib.stream_handle(torch)
-        if not use_graph or self.smoother == "lexgs":      # cooperative launches are not captured
-            _lib.check(self._enqueue_cycle(L, params, with_norm, st), "mg_vcycle")
-            self.last_launches = int(self.lib.mg_last_launch_count())
-            return
-        key = (L, params.smoother, params.nu_pre, params.nu_post, params.omega, params.zero_guess_skip,
-               params.reverse_post, params.x0_zero, bool(with_norm), self._cheby_key)
+
+        def enqueue(st):
+            if with_norm:
+                return self.lib.mg_vcycle_norm(self._level_structs, L, ctypes.byref(params), self._norm_ws.data_ptr(),
+                                               self._norm_out.data_ptr(), st)
+            return self.lib.mg_vcycle(self._level_structs, L, ctypes.byref(params), st)
+        self.last_launches = self._run(("vcycle", L, bool(with_norm), self._params_key(params)), enqueue,
+                                       use_graph and self._capturable(params))
+
+    # ------------------------------------------------------------------------------------------------
+    # device programs: one launch sequence per call, captured once into a CUDA graph and replayed
+    def _params_key(self, params):
+        """the part of a program's graph key that stands for its V-cycle: every mg_cycle_params field and the Chebyshev
+        tables; None without a preconditioner"""
+        if params is None:
+            return None
+        return tuple(getattr(params, f) for f, _ in params._fields_) + (self._cheby_key,)
+
+    def _capturable(self, params):
+        """a V-cycle with index-order Gauss-Seidel uses cooperative launches, which a graph cannot capture"""
+        return params is None or self.smoother != "lexgs"
+
+    def _run(self, key, enqueue, capture):
+        """Run one program: enqueue(stream) issues its launch sequence and returns the library's status.  capture: on
+        the first call with this key the sequence is captured into a CUDA graph, stored in self._graphs with its launch
+        count, and replayed from then on; otherwise it is enqueued on the current stream.  key[0] names the program
+        kind (drop_graphs).  Returns the program's launch count."""
+        torch, lib = self.torch, self.lib
+        if not capture:
+            _lib.check(enqueue(_lib.stream_handle(torch)), key[0])
+            return int(lib.mg_last_launch_count())
         g = self._graphs.get(key)
         if g is None:
             cap = torch.cuda.Stream(device=self.device)
             cap.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(cap):
                 h = cap.cuda_stream
-                _lib.check(self.lib.mg_graph_begin(h), "mg_graph_begin")
-                rc = self._enqueue_cycle(L, params, with_norm, h)
-                launches = int(self.lib.mg_last_launch_count())
+                _lib.check(lib.mg_graph_begin(h), "mg_graph_begin")
                 out = ctypes.c_void_p()
-                rc2 = self.lib.mg_graph_end(h, ctypes.byref(out))
-                _lib.check(rc, "mg_vcycle (capture)")
+                try:
+                    rc = enqueue(h)
+                    launches = int(lib.mg_last_launch_count())
+                finally:
+                    rc2 = lib.mg_graph_end(h, ctypes.byref(out))      # a capture is never left open
+                _lib.check(rc, "%s (capture)" % key[0])
                 _lib.check(rc2, "mg_graph_end")
             torch.cuda.current_stream().wait_stream(cap)
-            g = (out, launches)
-            self._graphs[key] = g
-        _lib.check(self.lib.mg_graph_launch(g[0], st), "mg_graph_launch")
-        self.last_launches = g[1]
+            g = self._graphs[key] = (out, launches)
+        _lib.check(lib.mg_graph_launch(g[0], _lib.stream_handle(torch)), "mg_graph_launch")
+        return g[1]
+
+    def drop_graphs(self, kind=None):
+        """Destroy the captured programs -- all of them, or those of one kind ("vcycle", "pcg", "gmres",
+        "vcycle_dist") -- so that the next call captures them anew.  A graph keeps the launch routes the library
+        switches (mg_set_cycle_fusion, mg_set_implied_*, mg_set_value_dict, ...) chose when it was captured: call
+        drop_graphs() after changing one."""
+        for key in [k for k in self._graphs if kind is None or k[0] == kind]:
+            self.lib.mg_graph_destroy(self._graphs.pop(key)[0])
 
     # ------------------------------------------------------------------------------------------------
     def _comm_ptr(self):
@@ -670,51 +695,26 @@ class DeviceHierarchy:
             self._cg = (x, p, Ap, sc, slots)
             self._cg_struct = _lib.mg_pcg(x.data_ptr(), p.data_ptr(), Ap.data_ptr(), sc.data_ptr(),
                                           self._norm_ws.data_ptr(), slots.data_ptr())
-            self._cg_graphs = {}
         x, p, Ap, sc, _ = self._cg
         pcg = ctypes.byref(self._cg_struct)
         pp = None if params is None else ctypes.byref(params)
-
-        def read_rr():
-            self._norm_host.copy_(sc[4:5], non_blocking=True)
-            torch.cuda.current_stream().synchronize()
-            return float(np.sqrt(self._norm_host.item()))
+        pkey, capture = self._params_key(params), self._capturable(params)
 
         def iterate(first):
-            key = (first, None if params is None else (params.smoother, params.nu_pre, params.nu_post, params.omega,
-                                                       params.zero_guess_skip, params.reverse_post, self._cheby_key))
-            g = self._cg_graphs.get(key)
-            if g is None:
-                if self.smoother == "lexgs" and params is not None:      # cooperative launches are not captured
-                    _lib.check(lib.mg_pcg_iterate(comm, self._level_structs, self.nlevels, pp, pcg, first, st),
-                               "mg_pcg_iterate")
-                    return
-                cap = torch.cuda.Stream(device=self.device)
-                cap.wait_stream(torch.cuda.current_stream())
-                with torch.cuda.stream(cap):
-                    h = cap.cuda_stream
-                    _lib.check(lib.mg_graph_begin(h), "mg_graph_begin")
-                    rc = lib.mg_pcg_iterate(comm, self._level_structs, self.nlevels, pp, pcg, first, h)
-                    out = ctypes.c_void_p()
-                    rc2 = lib.mg_graph_end(h, ctypes.byref(out))
-                    _lib.check(rc, "mg_pcg_iterate (capture)")
-                    _lib.check(rc2, "mg_graph_end")
-                torch.cuda.current_stream().wait_stream(cap)
-                g = self._cg_graphs[key] = out
-                self._graphs[("pcg",) + key] = (out, 0)        # destroyed with the other graphs
-            _lib.check(lib.mg_graph_launch(g, st), "mg_graph_launch")
+            self._run(("pcg", first, pkey),
+                      lambda s: lib.mg_pcg_iterate(comm, self._level_structs, self.nlevels, pp, pcg, first, s), capture)
 
         t0 = time.perf_counter()
         self.set_rhs(rhs)                      # r = b - A*0 = b
         torch.cuda.current_stream().synchronize()
         t1 = time.perf_counter()
         _lib.check(lib.mg_pcg_start(comm, self._level_structs, pcg, st), "mg_pcg_start")
-        track = [read_rr()]
+        track = [self._read_sqrt(sc[4:5])]
         its = 0
         for k in range(max_iterations):
             its += 1
             iterate(1 if k == 0 else 0)
-            res = read_rr()
+            res = self._read_sqrt(sc[4:5])
             track.append(res)
             if res <= error:
                 break
@@ -753,42 +753,16 @@ class DeviceHierarchy:
         ws = getattr(self, "_gm", None)
         if ws is None or ws["restart"] != restart:
             self._gm = None
-            for key in [k for k in self._graphs if k[0] == "gmres"]:
-                lib.mg_graph_destroy(self._graphs.pop(key)[0])
+            self.drop_graphs("gmres")           # their steps address the old workspace
             ws = self._gm = self._gmres_workspace(restart, n, getattr(lev, "n_vec", n))
         G = ctypes.byref(ws["struct"])
         pp = None if params is None else ctypes.byref(params)
         sc = ws["scalars"]
-
-        def read_r2():
-            self._norm_host.copy_(sc[0:1], non_blocking=True)
-            torch.cuda.current_stream().synchronize()
-            return float(np.sqrt(self._norm_host.item()))
-
-        pkey = None if params is None else (params.smoother, params.nu_pre, params.nu_post, params.omega,
-                                            params.zero_guess_skip, params.reverse_post, self._cheby_key)
+        pkey, capture = self._params_key(params), self._capturable(params)
 
         def iterate(j):
-            key = ("gmres", j, pkey)
-            g = self._graphs.get(key)
-            if g is None:
-                if self.smoother == "lexgs" and params is not None:      # cooperative launches are not captured
-                    _lib.check(lib.mg_gmres_iterate(comm, self._level_structs, self.nlevels, pp, G, j, st),
-                               "mg_gmres_iterate")
-                    return
-                cap = torch.cuda.Stream(device=self.device)
-                cap.wait_stream(torch.cuda.current_stream())
-                with torch.cuda.stream(cap):
-                    h = cap.cuda_stream
-                    _lib.check(lib.mg_graph_begin(h), "mg_graph_begin")
-                    rc = lib.mg_gmres_iterate(comm, self._level_structs, self.nlevels, pp, G, j, h)
-                    out = ctypes.c_void_p()
-                    rc2 = lib.mg_graph_end(h, ctypes.byref(out))
-                    _lib.check(rc, "mg_gmres_iterate (capture)")
-                    _lib.check(rc2, "mg_graph_end")
-                torch.cuda.current_stream().wait_stream(cap)
-                g = self._graphs[key] = (out, 0)
-            _lib.check(lib.mg_graph_launch(g[0], st), "mg_graph_launch")
+            self._run(("gmres", j, pkey),
+                      lambda s: lib.mg_gmres_iterate(comm, self._level_structs, self.nlevels, pp, G, j, s), capture)
 
         t0 = time.perf_counter()
         self.set_rhs(rhs)
@@ -803,7 +777,7 @@ class DeviceHierarchy:
         track = []
         while True:
             _lib.check(lib.mg_gmres_start(comm, self._level_structs, G, st), "mg_gmres_start")    # true residual
-            res = read_r2()
+            res = self._read_sqrt(sc[0:1])
             if not track:
                 track.append(res)
             if res <= error or its >= max_iterations:
@@ -813,7 +787,7 @@ class DeviceHierarchy:
                 iterate(k)
                 its += 1
                 k += 1
-                est = read_r2()
+                est = self._read_sqrt(sc[0:1])
                 track.append(est)
                 if est <= error:
                     break
@@ -859,8 +833,7 @@ class DeviceHierarchy:
 
     def __del__(self):
         try:
-            for g, _ in self._graphs.values():
-                self.lib.mg_graph_destroy(g)
+            self.drop_graphs()
         except Exception:
             pass
 

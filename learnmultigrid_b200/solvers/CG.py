@@ -42,8 +42,7 @@ class CG(IterativeSolver):
             r = h._from_level0(h.levels[0].b)                         # the residual lives in the level-0 rhs buffer
             if getattr(h, "comm", None) is not None:                  # partitioned: x and r are this rank's row blocks
                 if not getattr(self, "local_solution", False):
-                    x = np.concatenate([v.reshape(-1) for v in h.fabric.allgather(x.reshape(-1))]).reshape(-1, 1)
-                    r = np.concatenate([v.reshape(-1) for v in h.fabric.allgather(r.reshape(-1))]).reshape(-1, 1)
+                    x, r = h.global_rows(x, r)
                 h.check()
             self.iterations += its
             self.solution = x

@@ -30,8 +30,7 @@ class GMRES(IterativeSolver):
         r = h.gmres_residual_vector()
         if getattr(h, "comm", None) is not None:            # partitioned: x and r are this rank's row blocks
             if not getattr(self, "local_solution", False):
-                x = np.concatenate([v.reshape(-1) for v in h.fabric.allgather(x.reshape(-1))]).reshape(-1, 1)
-                r = np.concatenate([v.reshape(-1) for v in h.fabric.allgather(r.reshape(-1))]).reshape(-1, 1)
+                x, r = h.global_rows(x, r)
             h.check()
         self.iterations += its
         self.solution = x

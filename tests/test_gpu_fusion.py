@@ -213,7 +213,7 @@ def test_fused_cycle_is_bit_identical_to_the_plain_cycle(env, kind, N, levels, n
                 lib.mg_set_implied_columns(implied)
                 lib.mg_set_value_dict(vdict)
                 lib.mg_set_implied_values(impv)
-                h._graphs = {}
+                h.drop_graphs()
                 h.set_rhs(rhs)
                 h.zero_x()
                 xs, norms = [], []

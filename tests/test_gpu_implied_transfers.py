@@ -59,7 +59,7 @@ def test_cycle_with_implied_transfers_is_bit_identical(env, kind, N, levels, nu,
         results = {}
         for on in (0, 1):
             lib.mg_set_implied_transfers(on)
-            h._graphs = {}
+            h.drop_graphs()
             h.set_rhs(rhs)
             h.zero_x()
             xs, norms = [], []

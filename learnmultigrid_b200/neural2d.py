@@ -212,7 +212,8 @@ class NeuralBuilder:
             pred = self.predict(model, patches, mean, std)
             B, dneigh = self.fill_B(pred, fill, cmap, mass.shape[0], nc, not_last=self.not_last)
             if keep_intermediates:
-                trace.append({"M": mass, "cmap": cmap, "clist": clist, "patches": patches, "fill": fill, "pred": pred,
+                trace.append({"M": mass, "cmap": cmap, "clist": clist, "patches": patches, "fill": fill,
+                              "not_last": self.not_last, "pred": pred,
                               "B": SD.DevCSR(B.shape, B.indptr, B.indices, B.values.clone()), "dneigh": dneigh,
                               "rounds": self.last_rounds})
             Q = self.normalise(B)

@@ -678,6 +678,12 @@ typedef struct {
     int32_t cheb_degree;
     int32_t pad2_;
     const double *h_cheb_coef;
+    /* singular operator with a declared null vector (coarsest level solved by block cyclic reduction only; NULL
+     * otherwise): the cycle runs mg_project_out(n, d_null, null_inv_nn, null_pin, d_b) before the solve and
+     * mg_project_out(n, d_null, null_inv_nn, -1, d_x) after it, with d_tmp as the partials workspace */
+    const double *d_null;
+    double null_inv_nn;                   /* 1 / (nu^T nu)                                                           */
+    int64_t null_pin;                     /* the pinned row of the factor, in this level's ordering                  */
 } mg_level;
 /* multicolour Gauss-Seidel only.  PROPER_COLORING: no row has a non-zero entry in the column of ANOTHER row of its own
  * colour.  NONZERO_DIAG: every row has a non-zero diagonal entry (so a colour sweep overwrites every row it visits). */
@@ -794,6 +800,16 @@ int mg_scale_inv(int64_t n, const double *d_h, double *d_v, void *stream);
 /* y = R^-1 g (R: upper triangle of the first k columns of d_H, leading dimension ldh), then x += y_c z_c, c = 0..k-1 */
 int mg_gmres_solve_update(int64_t n, const double *d_H, int32_t ldh, const double *d_g, int32_t k, double *d_y,
                           const double *d_Z, int64_t ld, double *d_x, void *stream);
+/* v <- v - (nu^T v * inv_nn) nu, then v[pin] = 0 if pin >= 0 (removes the null vector nu of a singular symmetric
+ * operator; inv_nn = 1 / nu^T nu).  The dot is accumulated in double-double and rounded once, so it does not depend on
+ * how the rows are split; d_dot (optional) receives it.  d_partials: mg_project_workspace_size(n) doubles.  Two
+ * launches, capturable.  mg_project_out_dist: the same on this rank's row block of a row-partitioned vector, the dot
+ * summed over the ranks of comm in rank order (one program; d_slots: 2 * world doubles); every rank gets the same bits. */
+int64_t mg_project_workspace_size(int64_t n);
+int mg_project_out(int64_t n, const double *d_nu, double inv_nn, int64_t pin, double *d_v, double *d_partials,
+                   double *d_dot, void *stream);
+int mg_project_out_dist(mg_comm *comm, int64_t n, const double *d_nu, double inv_nn, int64_t pin, double *d_v,
+                        double *d_partials, double *d_slots, double *d_dot, void *stream);
 /* number of kernels the last mg_vcycle call on this thread launched (bench.py's gpu_launches) */
 int64_t mg_last_launch_count(void);
 /* CUDA-graph helpers: capture whatever is enqueued on `stream` between begin and end. */

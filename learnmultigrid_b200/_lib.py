@@ -101,7 +101,8 @@ class mg_level(ctypes.Structure):
                 ("coarse_kind", ctypes.c_int32), ("d_coarse_inv", c_vp), ("coarse_bcr", c_vp),
                 ("dist", ctypes.POINTER(mg_dist_level)), ("coarse_bcr_dist", ctypes.POINTER(mg_bcr_dist)),
                 ("flags", ctypes.c_uint32), ("pad_", ctypes.c_uint32), ("d_diag", c_vp),
-                ("cheb_degree", ctypes.c_int32), ("pad2_", ctypes.c_int32), ("h_cheb_coef", ctypes.POINTER(c_dbl))]
+                ("cheb_degree", ctypes.c_int32), ("pad2_", ctypes.c_int32), ("h_cheb_coef", ctypes.POINTER(c_dbl)),
+                ("d_null", c_vp), ("null_inv_nn", c_dbl), ("null_pin", c_i64)]
 
 
 class mg_cycle_params(ctypes.Structure):
@@ -176,6 +177,9 @@ _SIGNATURES = {
     "mg_sell_gs_rows": (c_int, [ctypes.POINTER(mg_sell), c_vp, c_vp, c_i64, c_i64, c_vp]),
     "mg_sell_prolong_correct": (c_int, [ctypes.POINTER(mg_sell), c_vp, c_vp, c_vp, c_vp]),
     "mg_dot": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "mg_project_workspace_size": (c_i64, [c_i64]),
+    "mg_project_out": (c_int, [c_i64, c_vp, c_dbl, c_i64, c_vp, c_vp, c_vp, c_vp]),
+    "mg_project_out_dist": (c_int, [c_vp, c_i64, c_vp, c_dbl, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "mg_axpby": (c_int, [c_i64, c_dbl, c_vp, c_dbl, c_vp, c_vp, c_vp]),
     "mg_fill": (c_int, [c_i64, c_dbl, c_vp, c_vp]),
     "mg_gather": (c_int, [c_i64, c_vp, c_vp, c_vp, c_vp]),

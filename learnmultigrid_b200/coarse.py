@@ -278,18 +278,26 @@ def bcr_ordering(n, indptr, indices):
     return bw_p, perm
 
 
-def build_coarse_solver(torch, dev, n, ip, ix, va, dense_max, host_pattern=None):
+def build_coarse_solver(torch, dev, n, ip, ix, va, dense_max, host_pattern=None, singular=False, label="coarsest level"):
     """Direct solver for an operator given as device CSR (ip, ix, va) -- the coarsest level of a hierarchy
     (Multigrid.py:106) or the system of DirectSolver (Solver.py:56-59):
       * n <= dense_max: explicit inverse;
       * banded as it is numbered (structured grids in natural order): block cyclic reduction;
       * anything else: reverse Cuthill-McKee first (unstructured meshes, shuffled numberings), then block cyclic
-        reduction on P A P^T with the permutation applied inside the solve."""
+        reduction on P A P^T with the permutation applied inside the solve.
+    singular=True: the operator may be symmetric with a one-dimensional null space (singular_coarse_solver); `label`
+    names it in the errors."""
+    if singular:
+        return singular_coarse_solver(torch, dev, n, ip, ix, va, dense_max, host_pattern, label)
     if n <= dense_max:
         return DenseCoarse(torch, dev, n, ip, ix, va)
     if host_pattern is None:
         host_pattern = (ip.cpu().numpy(), ix.cpu().numpy())
     bw, perm = bcr_ordering(n, *host_pattern)
+    return _bcr_solver(torch, dev, n, ip, ix, va, bw, perm)
+
+
+def _bcr_solver(torch, dev, n, ip, ix, va, bw, perm):
     if perm is None:
         return BcrCoarse(torch, dev, n, ip, ix, va, bw)
     # P A P^T on the device: rows gathered by perm, columns relabelled by its inverse (entry order inside a row is
@@ -301,3 +309,122 @@ def build_coarse_solver(torch, dev, n, ip, ix, va, dense_max, host_pattern=None)
     _lib.check(S.lib.mg_invert_permutation(n, dperm.data_ptr(), iperm.data_ptr(), S.st()), "mg_invert_permutation")
     Ap = S.permute(DevCSR((n, n), ip, ix, va), dperm, iperm)
     return BcrCoarse(torch, dev, n, Ap.indptr, Ap.indices, Ap.values, bw, perm=perm)
+
+
+# A coarsest operator is taken as singular when the derived null vector nu_L leaves a residual in the pinned row of at most
+# this much relative to ||A||_inf ||nu_L||_inf, and the pseudo-inverse is accepted when ||A A+ A w - A w|| <= VERIFY_TOL ||A w||.
+SINGULAR_TOL = 1e-10
+VERIFY_TOL = 1e-8
+
+
+def apply_coarse(solver, rhs, out):
+    """out = the solver's inverse (pseudo-inverse of a singular operator) applied to rhs (device vectors; rhs of a
+    singular block cyclic reduction is overwritten with Z_k P rhs)"""
+    torch = solver.torch
+    lib = _lib.load()
+    st = _lib.stream_handle(torch)
+    if solver.kind == _lib.MG_COARSE_DENSE:
+        _lib.check(lib.mg_dense_gemv(solver.n, solver.n, solver.inv.data_ptr(), rhs.data_ptr(), out.data_ptr(), st),
+                   "mg_dense_gemv")
+        return
+    if solver.null is not None:
+        project_out(solver, rhs, solver.null_pin)
+    solver.solve(torch, rhs, out)
+    if solver.null is not None:
+        project_out(solver, out, -1)
+
+
+def project_out(solver, v, pin):
+    """v <- v - (nu^T v / nu^T nu) nu with the solver's null vector, then v[pin] = 0 if pin >= 0 (mg_project_out)"""
+    torch = solver.torch
+    lib = _lib.load()
+    _lib.check(lib.mg_project_out(solver.n, solver.null.data_ptr(), solver.null_inv_nn, int(pin), v.data_ptr(),
+                                  solver.null_work.data_ptr(), None, _lib.stream_handle(torch)), "mg_project_out")
+
+
+def singular_coarse_solver(torch, dev, n, ip, ix, va, dense_max, host_pattern, label):
+    """Direct solver of a symmetric operator A that may have a one-dimensional null space (DESIGN.md, singular systems).
+    In the solver's own ordering (after reverse Cuthill-McKee where block cyclic reduction uses it) k is the last row and
+    A_pin is A with row and column k replaced by e_k; the band, and with it the block structure, is unchanged.
+      nu_L = e_k - A_pin^-1 Z_k a_k            (a_k: column k of A; Z_k zeroes entry k)
+    is a null vector of A if A has one with a non-zero entry k.  A is taken as singular when
+    |(A nu_L)_k| <= SINGULAR_TOL ||A||_inf ||nu_L||_inf, and then solved with
+      A+ = P A_pin^-1 Z_k P,    P = I - nu_L nu_L^T / (nu_L^T nu_L)
+    (the minimum-norm solution for right-hand sides in range(A) = nu_L-perp, the least-squares one for others): dense,
+    as the explicit matrix mg_dense_gemv applies; by block cyclic reduction, as the projections around the solve
+    (cycle.cu, mg_project_out).  A pseudo-inverse that does not reproduce A w for the hashed vector w to VERIFY_TOL
+    (a null space of more than one vector) raises MgError.  Otherwise A is factored as it is.  The solver carries
+    null_info = {"singular", "pin", "null_ratio", "verify_ratio"} and, when singular, null / null_inv_nn / null_pin."""
+    import scipy.sparse as sp
+    from . import formats as F
+    hip, hix = (ip.cpu().numpy(), ix.cpu().numpy()) if host_pattern is None else host_pattern
+    A = sp.csr_matrix((va.cpu().numpy(), np.asarray(hix), np.asarray(hip)), shape=(n, n))
+    norm_A = float(abs(A).sum(axis=1).max()) if A.nnz else 0.0
+    if n <= dense_max:
+        bw, perm = 0, None
+    else:
+        bw, perm = bcr_ordering(n, hip, hix)
+    k = n - 1 if perm is None else int(perm[n - 1])          # the pinned row in the level's ordering
+    keep = np.ones(n)
+    keep[k] = 0.0
+    Z = sp.diags(keep)
+    A_pin = sp.csr_matrix(Z @ A @ Z + sp.csr_matrix(([1.0], ([k], [k])), shape=(n, n)))
+    A_pin.sort_indices()
+    dip, dix, dva = (torch.from_numpy(np.ascontiguousarray(a, dtype=t)).to(dev) for a, t in
+                     ((A_pin.indptr, np.int32), (A_pin.indices, np.int32), (A_pin.data, np.float64)))
+    solver = DenseCoarse(torch, dev, n, dip, dix, dva) if n <= dense_max else _bcr_solver(
+        torch, dev, n, dip, dix, dva, bw, perm)
+    solver.torch = torch
+    solver.null = None
+    a_k = np.asarray(A[:, [k]].todense()).ravel() * keep
+    y = torch.empty(n, dtype=torch.float64, device=dev)
+    apply_coarse(solver, torch.from_numpy(-a_k).to(dev), y)
+    nu = y.cpu().numpy()
+    nu[k] = 1.0
+    null_ratio = abs(float((A @ nu)[k])) / max(norm_A * float(np.abs(nu).max()), np.finfo(float).tiny)
+    info = {"singular": bool(null_ratio <= SINGULAR_TOL), "pin": k, "null_ratio": null_ratio, "verify_ratio": None}
+    if not info["singular"]:
+        # taken as nonsingular: factored as it is, and the factor checked the same way (a rank-deficient operator whose
+        # null vectors all vanish at k would pass the rule; its factor does not reproduce A w)
+        del solver
+        solver = build_coarse_solver(torch, dev, n, ip, ix, va, dense_max, (hip, hix))
+        solver.torch = torch
+        solver.null = None
+        info["verify_ratio"] = _verify(solver, A, label, "the factor taken as nonsingular")
+        solver.null_info = info
+        return solver
+    nn = float(nu @ nu)
+    d_nu = torch.from_numpy(nu).to(dev)
+    if solver.kind == _lib.MG_COARSE_DENSE:
+        # A+ = P M P with M = A_pin^-1 Z_k (column k of the inverse dropped); rank-one updates on the device
+        M = solver.inv.view(n, n)
+        M[:, k] = 0.0
+        Mnu = M @ d_nu
+        nuM = d_nu @ M
+        c = float(d_nu @ Mnu)
+        M -= torch.outer(d_nu, nuM) / nn
+        M -= torch.outer(Mnu, d_nu) / nn
+        M += torch.outer(d_nu, d_nu) * (c / (nn * nn))
+    solver.null = d_nu
+    solver.null_inv_nn = 1.0 / nn
+    solver.null_pin = k
+    solver.null_work = torch.zeros(int(_lib.load().mg_project_workspace_size(n)), dtype=torch.float64, device=dev)
+    info["verify_ratio"] = _verify(solver, A, label, "the pseudo-inverse pinned at row %d" % k)
+    solver.null_info = info
+    return solver
+
+
+def _verify(solver, A, label, what):
+    """||A X A w - A w|| / ||A w|| for the solver's X and the hashed vector w; MgError above VERIFY_TOL"""
+    from . import formats as F
+    torch = solver.torch
+    n = A.shape[0]
+    w = F.chebyshev_start_vector(np.arange(n, dtype=np.int64))
+    Aw = A @ w
+    x = torch.empty(n, dtype=torch.float64, device=solver.dev if hasattr(solver, "dev") else solver.inv.device)
+    apply_coarse(solver, torch.from_numpy(Aw).to(x.device), x)
+    ratio = float(np.linalg.norm(A @ x.cpu().numpy() - Aw)) / max(float(np.linalg.norm(Aw)), np.finfo(float).tiny)
+    if not ratio <= VERIFY_TOL:
+        raise _lib.MgError("%s: %s reproduces A w only to %.3e relative (limit %.0e): the null space has more than "
+                           "one vector" % (label, what, ratio, VERIFY_TOL))
+    return ratio

@@ -36,6 +36,7 @@ int csr_gs_lex(const int32_t *, const int32_t *, const double *, double *, const
                const int32_t *, int64_t, int64_t, int, cudaStream_t);
 int bcr_solve(const void *handle, const mg_bcr_dist *dist, mg_comm *comm, const double *rhs, double *x, cudaStream_t st);
 int vec_scatter(int64_t, const int32_t *, const double *, double *, cudaStream_t);
+int null_project(int64_t, const double *, double, int64_t, double *, double *, cudaStream_t, double *);
 int vec_dot_partials(int64_t, const double *, const double *, double *, int *, cudaStream_t);
 int vec_pcg_direction(int64_t, const double *, double *, const double *, int, cudaStream_t);
 int vec_pcg_update(int64_t, const double *, const double *, double *, double *, const double *, double *, int *, cudaStream_t);
@@ -258,7 +259,13 @@ static int vcycle_rec(mg_comm *comm, const mg_level *levels, int nlevels, int l,
             if (!L.d_coarse_inv) return set_error(MG_ERR_INVALID, "mg_vcycle", "coarsest level has no inverse");
             return dense_gemv(L.n, L.n, L.d_coarse_inv, L.d_b, L.d_x, st);
         }
-        if (L.coarse_kind == MG_COARSE_BCR) return bcr_solve(L.coarse_bcr, L.coarse_bcr_dist, comm, L.d_b, L.d_x, st);
+        if (L.coarse_kind == MG_COARSE_BCR) {
+            if (!L.d_null) return bcr_solve(L.coarse_bcr, L.coarse_bcr_dist, comm, L.d_b, L.d_x, st);
+            // singular operator: the factor is pinned at null_pin, x = P A_pin^-1 Z_pin P b (coarse.py, BcrCoarse)
+            MG_TRY(null_project(L.n, L.d_null, L.null_inv_nn, L.null_pin, L.d_b, L.d_tmp, st, nullptr));
+            MG_TRY(bcr_solve(L.coarse_bcr, L.coarse_bcr_dist, comm, L.d_b, L.d_x, st));
+            return null_project(L.n, L.d_null, L.null_inv_nn, -1, L.d_x, L.d_tmp, st, nullptr);
+        }
         return set_error(MG_ERR_INVALID, "mg_vcycle", "unknown coarse solver kind");
     }
     const mg_level &C = levels[l + 1];

@@ -184,6 +184,12 @@ class _Layout:
         self.c0, self.c1, self.own_iperm, self.n_own, self.slot_of, self.length = c0, c1, own_iperm, n_own, slot_of, length
 
 
+def _refuse_null_space(null_space, what):
+    """hierarchies built from row blocks only (StripHierarchy) cannot check the global operator against nu"""
+    if null_space is not None:
+        raise ValueError("%s does not support a declared null space; use DistributedHierarchy or DeviceHierarchy" % what)
+
+
 class DistributedHierarchy(DeviceHierarchy):
     """Multigrid hierarchy whose first `n_dist` levels are row-partitioned over the ranks of `fabric`.
 
@@ -197,12 +203,16 @@ class DistributedHierarchy(DeviceHierarchy):
     def __init__(self, A, Q_list, fabric, smoother="jacobi", colors=None, device=None, min_rows_per_rank=65536,
                  n_dist=None, dense_coarse_max=DENSE_COARSE_MAX, keep_host=False, region_bytes=16 << 20,
                  max_sites=512, timeout_s=10.0, split_coarse_solve=True, bcr_split_min_blocks=32, cheby_degree=2,
-                 cheby_bounds=None):
+                 cheby_bounds=None, null_space=None):
         self._init_rank(fabric, smoother, len(Q_list) + 1, device, split_coarse_solve, bcr_split_min_blocks,
                         cheby_degree, cheby_bounds)
         self.keep_host = keep_host
+        nu_nat = self._null_check(A, null_space)           # the GLOBAL operator: the same checks on every rank
         self._setup_dist(A, Q_list, colors, dense_coarse_max, min_rows_per_rank, n_dist)
         self._start(region_bytes, max_sites, timeout_s)
+        if nu_nat is not None:
+            self._null_slots = self.torch.zeros(2 * _lib.MG_MAX_RANKS, dtype=self.torch.float64, device=self.device)
+            self._null_level0(nu_nat)
 
     def _init_rank(self, fabric, smoother, nlevels, device, split_coarse_solve, bcr_split_min_blocks, cheby_degree=2,
                    cheby_bounds=None):
@@ -226,6 +236,7 @@ class DistributedHierarchy(DeviceHierarchy):
         self._graphs = {}
         self._keep = []
         self.setup_kind = "device"
+        self.null = self.null_info = self.rhs_null_component = self._null_space = None
 
     def _start(self, region_bytes, max_sites, timeout_s):
         """Communicator, level structs and warm-up once the levels are built; returns when every rank is ready."""
@@ -609,6 +620,20 @@ class DistributedHierarchy(DeviceHierarchy):
 
     def _comm_ptr(self):
         return ctypes.byref(self.comm.struct)
+
+    def _null_block(self, nu_nat):
+        p = self.levels[0].plan
+        return nu_nat[p.o0:p.o1]
+
+    def project_null(self, v, dot=None):
+        """the projection on this rank's row block, nu^T v summed over the ranks (mg_project_out_dist): one program,
+        the same bits on every rank and as on one GPU"""
+        if getattr(self, "null", None) is None:
+            return
+        _lib.check(self.lib.mg_project_out_dist(ctypes.byref(self.comm.struct), self.n, self.null.data_ptr(),
+                                                self.null_inv_nn, -1, v.data_ptr(), self._norm_ws.data_ptr(),
+                                                self._null_slots.data_ptr(), None if dot is None else dot.data_ptr(),
+                                                _lib.stream_handle(self.torch)), "mg_project_out_dist")
 
     def check(self):
         self.comm.check()

@@ -25,7 +25,7 @@ import scipy.sparse as sp
 from . import formats as F
 from . import partition_setup as PS
 from . import setup_device as SD
-from .distributed import DistributedHierarchy
+from .distributed import DistributedHierarchy, _refuse_null_space
 from .engine import DENSE_COARSE_MAX
 
 
@@ -58,7 +58,8 @@ class StripHierarchy(DistributedHierarchy):
 
     def __init__(self, A_blk, Q_blks, offsets, fabric, n_dist, smoother="jacobi", colors=None, device=None,
                  dense_coarse_max=DENSE_COARSE_MAX, region_bytes=16 << 20, max_sites=512, timeout_s=10.0,
-                 split_coarse_solve=True, bcr_split_min_blocks=32, device_products=True):
+                 split_coarse_solve=True, bcr_split_min_blocks=32, device_products=True, null_space=None):
+        _refuse_null_space(null_space, "StripHierarchy")
         if smoother == "chebyshev":
             raise ValueError("StripHierarchy supports 'jacobi' and 'mcgs'; the Chebyshev smoother needs the global "
                              "operators for its bounds (use DistributedHierarchy)")

@@ -284,10 +284,15 @@ class DeviceHierarchy:
     cheby_bounds : None (default: [0.3, 1.1] x a 10-step Lanczos estimate of lambda_max(D^-1 A) per level) or one
                    (lo, hi) pair per smoothing level (levels - 1 of them)
     setup    : "device" (SpGEMM / transposes / SELL build by CUDA kernels) or "host" (NumPy/SciPy cross-check)
+    null_space : None, "constant" or n values: the null vector nu of a singular SYMMETRIC A (pure Neumann problems).
+               The coarsest level then derives its own null vector and is solved with the pseudo-inverse
+               (coarse.singular_coarse_solver); solve / pcg / gmres remove nu from the right-hand side before they start
+               (rhs_null_component: nu^T b / ||nu|| of what was removed) and from x before it is returned, so x is the
+               minimum-norm solution.  null_info holds the checks' ratios and the coarse decision.
     """
 
     def __init__(self, A, Q_list, smoother="jacobi", colors=None, device=None, setup="device",
-                 dense_coarse_max=DENSE_COARSE_MAX, keep_host=True, cheby_degree=2, cheby_bounds=None):
+                 dense_coarse_max=DENSE_COARSE_MAX, keep_host=True, cheby_degree=2, cheby_bounds=None, null_space=None):
         torch = _lib.require_cuda()
         self.torch = torch
         self.lib = _lib.load()
@@ -303,6 +308,10 @@ class DeviceHierarchy:
         self._graphs = {}
         self._keep = []          # tensors / ctypes buffers that must outlive the level structs
         self.setup_kind = setup
+        self.null = None
+        self.null_info = None
+        self.rhs_null_component = None
+        nu_nat = self._null_check(A, null_space)
         if setup == "host":
             self._setup_host(A, Q_list, colors, dense_coarse_max)
         elif setup == "device":
@@ -310,6 +319,52 @@ class DeviceHierarchy:
         else:
             raise ValueError("setup must be 'device' or 'host'")
         self._finish_structs()
+        if nu_nat is not None:
+            self._null_level0(nu_nat)
+
+    # ------------------------------------------------------------------------------------------------
+    # singular operators with a declared null vector
+    def _null_check(self, A, null_space):
+        """declared_null_vector for this hierarchy's operator, or None without a null space"""
+        self._null_space = null_space
+        if null_space is None:
+            return None
+        nu, ratio = declared_null_vector(self.torch, self.device, A, null_space)
+        self.null_info = {"fine_ratio": ratio}
+        return nu
+
+    def _null_level0(self, nu_nat):
+        """level 0 keeps nu in its own ordering (its row block on a partitioned hierarchy); the coarsest level's
+        decision joins null_info"""
+        lev = self.levels[0]
+        self.null_inv_nn = 1.0 / float(nu_nat @ nu_nat)          # of the global vector: the same bits on every rank
+        blk = self._null_block(nu_nat)
+        self.null = blk if lev.perm is None else blk[lev.perm.long()].contiguous()
+        self._null_dot = self.torch.zeros(1, dtype=self.torch.float64, device=self.device)
+        self.null_info.update(getattr(self.levels[-1].coarse, "null_info", {}) or {})
+
+    def _null_block(self, nu_nat):
+        """the rows of nu level 0 holds (natural order): all of them on one GPU"""
+        return nu_nat
+
+    def project_null(self, v, dot=None):
+        """v <- v - (nu^T v / nu^T nu) nu on a level-0 device vector (mg_project_out: the dot in double-double, so it
+        does not depend on how the rows are split); dot: optional one-element device tensor that receives nu^T v.
+        Nothing without a null space."""
+        if getattr(self, "null", None) is None:
+            return
+        _lib.check(self.lib.mg_project_out(self.n, self.null.data_ptr(), self.null_inv_nn, -1, v.data_ptr(),
+                                           self._norm_ws.data_ptr(), None if dot is None else dot.data_ptr(),
+                                           _lib.stream_handle(self.torch)), "mg_project_out")
+
+    def project_rhs(self):
+        """remove nu from the level-0 right-hand side; rhs_null_component = nu^T b / ||nu|| of what was removed"""
+        if getattr(self, "null", None) is None:
+            return
+        self.project_null(self.levels[0].b, self._null_dot)
+        self._norm_host.copy_(self._null_dot, non_blocking=True)
+        self.torch.cuda.current_stream().synchronize()
+        self.rhs_null_component = float(self._norm_host.item()) * float(np.sqrt(self.null_inv_nn))
 
     # ------------------------------------------------------------------------------------------------
     def _chebyshev_args(self, degree, bounds):
@@ -388,7 +443,9 @@ class DeviceHierarchy:
         self._coarsest(lev, A_dev.shape[0], A_dev.indptr, A_dev.indices, A_dev.values, dense_coarse_max, None)
 
     def _coarsest(self, lev, n, ip, ix, va, dense_coarse_max, host_pattern):
-        solver = build_coarse_solver(self.torch, self.device, n, ip, ix, va, dense_coarse_max, host_pattern)
+        solver = build_coarse_solver(self.torch, self.device, n, ip, ix, va, dense_coarse_max, host_pattern,
+                                     singular=getattr(self, "_null_space", None) is not None,
+                                     label="level %d" % (self.nlevels - 1))
         lev.coarse = solver
         lev.coarse_kind = solver.kind
         lev.coarse_bytes = solver.bytes
@@ -461,6 +518,10 @@ class DeviceHierarchy:
                     s.d_coarse_inv = lev.coarse_inv.data_ptr()
                 else:
                     s.coarse_bcr = lev.coarse_bcr
+                    if getattr(lev.coarse, "null", None) is not None:
+                        s.d_null = lev.coarse.null.data_ptr()
+                        s.null_inv_nn = lev.coarse.null_inv_nn
+                        s.null_pin = lev.coarse.null_pin
                     if getattr(lev, "coarse_bcr_dist", None) is not None:
                         s.coarse_bcr_dist = ctypes.pointer(lev.coarse_bcr_dist)
         self._level_structs = arr
@@ -706,6 +767,7 @@ class DeviceHierarchy:
 
         t0 = time.perf_counter()
         self.set_rhs(rhs)                      # r = b - A*0 = b
+        self.project_rhs()
         torch.cuda.current_stream().synchronize()
         t1 = time.perf_counter()
         _lib.check(lib.mg_pcg_start(comm, self._level_structs, pcg, st), "mg_pcg_start")
@@ -719,6 +781,7 @@ class DeviceHierarchy:
             if res <= error:
                 break
         t2 = time.perf_counter()
+        self.project_null(x)
         sol = self._from_level0(x, view)
         t3 = time.perf_counter()
         self.last_pcg_timing = {"transfer_in_s": t1 - t0, "iterations_s": t2 - t1, "transfer_out_s": t3 - t2,
@@ -766,6 +829,7 @@ class DeviceHierarchy:
 
         t0 = time.perf_counter()
         self.set_rhs(rhs)
+        self.project_rhs()
         x = ws["x"]
         if x0 is None:
             x.zero_()
@@ -793,6 +857,7 @@ class DeviceHierarchy:
                     break
             _lib.check(lib.mg_gmres_finish(self._level_structs, pp, G, k, st), "mg_gmres_finish")
         t2 = time.perf_counter()
+        self.project_null(x)
         sol = self._from_level0(x, view)
         t3 = time.perf_counter()
         self.last_gmres_timing = {"transfer_in_s": t1 - t0, "iterations_s": t2 - t1, "orthogonalisation_s": None,
@@ -920,3 +985,41 @@ class DeviceHierarchy:
         if self.host_A is not None and self.host_A[l] is not None:
             return self.host_A[l]
         return SD.download_level_matrix(self, l)
+
+
+NULL_TOL = 1e-10            # a declared null vector: ||A nu||_inf <= NULL_TOL ||A||_inf ||nu||_inf
+SYMMETRY_TOL = 1e-12        # and a symmetric A: |A - A^T| <= SYMMETRY_TOL ||A||_inf entry by entry
+
+
+def declared_null_vector(torch, dev, A, null_space):
+    """(nu, ratio): the declared null vector of A ("constant" or n values) as a float64 device tensor in natural order,
+    and ||A nu||_inf / (||A||_inf ||nu||_inf).  ValueError for a vector of the wrong length, a vector A does not
+    annihilate (with the ratio) and a nonsymmetric A (the transpose is formed on the device): only symmetric operators
+    have range(A) = nu-perp, which the projections rely on.  A: anything SciPy accepts, or a DevCSR."""
+    S = SD.DeviceSetup(torch, dev)
+    Ad = A if hasattr(A, "ptrs") else S.upload(A)
+    n = Ad.shape[0]
+    if isinstance(null_space, str):
+        if null_space != "constant":
+            raise ValueError("null_space must be None, 'constant' or an array of %d values" % n)
+        nu = torch.ones(n, dtype=torch.float64, device=dev)
+    else:
+        v = np.asarray(null_space, dtype=np.float64).reshape(-1)
+        if v.size != n:
+            raise ValueError("null space vector has %d entries, operator has %d rows" % (v.size, n))
+        nu = torch.from_numpy(np.ascontiguousarray(v)).to(dev)
+    rows = torch.repeat_interleave(torch.arange(n, device=dev), torch.diff(Ad.indptr.long()))
+    norm_A = float(torch.zeros(n, dtype=torch.float64, device=dev).index_add_(
+        0, rows, Ad.values.abs()).max().item()) if Ad.nnz else 0.0
+    Anu = torch.zeros(n, dtype=torch.float64, device=dev).index_add_(0, rows, Ad.values * nu[Ad.indices.long()])
+    nu_max = float(nu.abs().max().item())
+    ratio = float(Anu.abs().max().item()) / max(norm_A * nu_max, np.finfo(float).tiny)
+    if nu_max == 0.0 or not ratio <= NULL_TOL:
+        raise ValueError("the declared null space is not one of the operator: ||A nu||_inf / (||A||_inf ||nu||_inf) = "
+                         "%.3e (limit %.0e)" % (ratio, NULL_TOL))
+    del rows, Anu
+    T = S.transpose(Ad)
+    if not (torch.equal(T.indptr, Ad.indptr) and torch.equal(T.indices, Ad.indices)
+            and float((T.values - Ad.values).abs().max().item()) <= SYMMETRY_TOL * norm_A):
+        raise ValueError("a declared null space needs a symmetric operator (range(A) = nu-perp); this one is not")
+    return nu, ratio

@@ -30,9 +30,34 @@ def boundary_nodes_2d(N):
     return np.flatnonzero((ix == 0) | (ix == N) | (iy == 0) | (iy == N))
 
 
-def structured_laplacian_2d(N, coefficient=None, rows=None, Ny=None):
+def _check_boundary(boundary):
+    if boundary not in ("dirichlet", "neumann"):
+        raise ValueError("boundary must be 'dirichlet' or 'neumann' (got %r)" % (boundary,))
+
+
+def neumann_stencil_2d(ix, iy, N, Ny, k1, k2, xp=np):
+    """(south, west, diag, east, north) couplings of the P1 stiffness rows of the nodes (ix, iy) as the element loop
+    gives them without Dirichlet rows: an edge coupling is -1/2 of the coefficients of the (at most two) triangles that
+    have the edge as a leg, a triangle outside the domain contributes nothing, the diagonal is minus the sum of the
+    others (rows sum to zero).  k1(sx, sy) / k2(sx, sy): coefficient of the lower / upper triangle of square (sx, sy)
+    (float arrays); `xp`: numpy or torch.  Couplings to nodes outside the grid are 0 with exists False."""
+    def on(mask, v):
+        return xp.where(mask, v, xp.zeros_like(v))
+    x, y = ix, iy
+    up, down, right, left = y < Ny, y > 0, x < N, x > 0
+    east = -0.5 * (on(up & right, k1(x, y)) + on(down & right, k2(x, y - 1)))
+    west = -0.5 * (on(up & left, k1(x - 1, y)) + on(down & left, k2(x - 1, y - 1)))
+    north = -0.5 * (on(up & right, k2(x, y)) + on(up & left, k1(x - 1, y)))
+    south = -0.5 * (on(down & right, k2(x, y - 1)) + on(down & left, k1(x - 1, y - 1)))
+    diag = -(east + west + north + south)
+    return (south, west, diag, east, north), (down, left, xp.ones_like(up), right, up)
+
+
+def structured_laplacian_2d(N, coefficient=None, rows=None, Ny=None, boundary="dirichlet"):
     """P1 stiffness matrix of -div(k grad u) on the reference's structured mesh Mesh2D(N*N) ((N+1)^2 nodes, row
     major), with boundary rows replaced by identity rows exactly as test/thesis_structured_2d.py:407-414.
+    boundary="neumann": no rows are replaced, every row is what the element loop gives (natural boundary conditions):
+    the rows sum to zero and the constant vector spans the null space (DeviceHierarchy(null_space="constant")).
     k = 1 gives the 5-point stencil [-1,-1,4,-1,-1] (hypotenuse couplings are exact zeros and not stored);
     `coefficient(x, y)` is evaluated at element centroids.  Returns canonical CSR.
     rows=(r0, r1): only that row block (global column ids) -- what one rank of a row-partitioned run generates, so
@@ -47,7 +72,18 @@ def structured_laplacian_2d(N, coefficient=None, rows=None, Ny=None):
         raise ValueError("row block outside the matrix")
     if (r1 - r0) * 5 >= 2 ** 31 or n >= 2 ** 31:
         raise OverflowError("nnz does not fit int32")
+    _check_boundary(boundary)
     iy, ix = np.divmod(np.arange(r0, r1, dtype=np.int64), W)
+    if boundary == "neumann":
+        h = 1.0 / N
+        kf = (lambda sx, sy: np.ones(np.shape(sx))) if coefficient is None else coefficient
+        vals, exists = neumann_stencil_2d(ix, iy, N, Ny, lambda sx, sy: kf((sx + 2.0 / 3.0) * h, (sy + 1.0 / 3.0) * h),
+                                          lambda sx, sy: kf((sx + 1.0 / 3.0) * h, (sy + 2.0 / 3.0) * h))
+        keep = np.stack(exists, axis=1)
+        cols = np.stack([ix + iy * W + off for off in (-W, -1, 0, 1, W)], axis=1)
+        indptr = np.zeros(r1 - r0 + 1, dtype=np.int64)
+        np.cumsum(keep.sum(axis=1), out=indptr[1:])
+        return F.raw_csr(indptr.astype(np.int32), cols[keep].astype(np.int32), np.stack(vals, axis=1)[keep], (r1 - r0, n))
     interior = (ix > 0) & (ix < N) & (iy > 0) & (iy < Ny)
     counts = np.where(interior, 5, 1).astype(np.int64)
     indptr = np.zeros(r1 - r0 + 1, dtype=np.int64)
@@ -115,15 +151,22 @@ def convection_diffusion_2d(N, eps, beta):
     return A
 
 
-def structured_rhs_2d(N, f_value=-1.0, rows=None, Ny=None):
+def structured_rhs_2d(N, f_value=-1.0, rows=None, Ny=None, boundary="dirichlet"):
     """load vector of f = const on the structured mesh with Dirichlet rows zeroed: interior entries f*h^2
     (six triangles of area h^2/2, each contributing f*area/3), thesis_structured_2d.py:17-19,403,414.
+    boundary="neumann": no entry is zeroed, a boundary node gets f*area/3 of the triangles it has.
     rows / Ny as in structured_laplacian_2d."""
     Ny = N if Ny is None else int(Ny)
     W = N + 1
     h = 1.0 / N
     r0, r1 = (0, W * (Ny + 1)) if rows is None else (int(rows[0]), int(rows[1]))
+    _check_boundary(boundary)
     iy, ix = np.divmod(np.arange(r0, r1, dtype=np.int64), W)
+    if boundary == "neumann":
+        up, down, right, left = iy < Ny, iy > 0, ix < N, ix > 0
+        # triangles at the node: 2 in square (x, y), 1 in (x-1, y), 2 in (x-1, y-1), 1 in (x, y-1)
+        count = 2 * (up & right) + (up & left) + 2 * (down & left) + (down & right)
+        return (f_value * h * h * (count / 6.0)).reshape(-1, 1)
     interior = (ix > 0) & (ix < N) & (iy > 0) & (iy < Ny)
     return np.where(interior, f_value * h * h, 0.0).reshape(-1, 1)
 
@@ -274,12 +317,14 @@ def coloring_is_valid(A, colors):
     return not np.any(colors[A.row[off]] == colors[A.col[off]])
 
 
-def irregular_p1_2d(N, seed=42, f_value=-1.0):
+def irregular_p1_2d(N, seed=42, f_value=-1.0, boundary="dirichlet"):
     """BASELINE configs[1] (C2): the reference's own notion of an unstructured mesh -- Mesh2D((N/2)^2) followed by one
     irregular red refinement (Mesh2D.refine(regular=False): new edge points at r in [0.3, 0.7] along each edge,
     Mesh2D.py:110-135; parents are numbered first, edge nodes in element-edge discovery order) -- with P1 stiffness,
     mass and load (f = const) and row-replaced Dirichlet rows (thesis_structured_2d.py:407-414).  (N+1)^2 nodes.
+    boundary="neumann": the stiffness matrix and load vector as assembled, no row replaced.
     Returns dict(A, M, rhs, boundary, mesh)."""
+    _check_boundary(boundary)
     from .mesh.Mesh2D import Mesh2D
     from .assembly.MassMatrix import MassMatrix
     from .assembly.StiffnessMatrix import StiffnessMatrix
@@ -298,13 +343,17 @@ def irregular_p1_2d(N, seed=42, f_value=-1.0):
     rhs = LoadVector(mesh).compute_rhs_2d(LoadFunction(lambda pts: f_value), FunctionTriangle(1), q)
     p = np.asarray(mesh.get_points())
     eps = 1e-12
-    boundary = np.flatnonzero((p[:, 0] < eps) | (p[:, 0] > 1 - eps) | (p[:, 1] < eps) | (p[:, 1] > 1 - eps))
+    nodes = np.flatnonzero((p[:, 0] < eps) | (p[:, 0] > 1 - eps) | (p[:, 1] < eps) | (p[:, 1] > 1 - eps))
+    rhs = np.asarray(rhs, dtype=np.float64).reshape(-1, 1).copy()
+    if boundary == "neumann":
+        return {"A": F.canonical_csr(sp.csr_matrix(A)), "M": F.canonical_csr(sp.csr_matrix(M)), "rhs": rhs,
+                "boundary": nodes, "mesh": mesh}
+    boundary = nodes
     A = sp.lil_matrix(A)
     for i in boundary:                      # A[nodes,:] = I[nodes,:]
         A.rows[i] = [int(i)]
         A.data[i] = [1.0]
     A = F.canonical_csr(sp.csr_matrix(A))
-    rhs = np.asarray(rhs, dtype=np.float64).reshape(-1, 1).copy()
     rhs[boundary] = 0.0
     return {"A": A, "M": F.canonical_csr(sp.csr_matrix(M)), "rhs": rhs, "boundary": boundary, "mesh": mesh}
 

@@ -30,13 +30,18 @@ def variable_coefficient(torch, x, y):
     return 1.0 + 0.9 * torch.sin(2 * np.pi * x) * torch.sin(2 * np.pi * y)
 
 
-def structured_laplacian_2d(N, coefficient=None, Ny=None, device=None, symmetric=False):
+def structured_laplacian_2d(N, coefficient=None, Ny=None, device=None, symmetric=False, boundary="dirichlet"):
     """problems.structured_laplacian_2d as a DevCSR; coefficient: None or a callable (torch, x, y) -> k.
     symmetric=True: problems.symmetric_dirichlet of it -- the couplings of interior rows to Dirichlet nodes are dropped
-    (their values are zero, so the solution is unchanged) and the operator is symmetric, as conjugate gradients need."""
+    (their values are zero, so the solution is unchanged) and the operator is symmetric, as conjugate gradients need.
+    boundary="neumann": no Dirichlet rows (problems.structured_laplacian_2d(boundary="neumann")); symmetric as it is."""
+    from .problems import _check_boundary
+    _check_boundary(boundary)
     torch = _lib.require_cuda()
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     Ny = N if Ny is None else int(Ny)
+    if boundary == "neumann":
+        return _neumann_laplacian_2d(torch, dev, N, coefficient, Ny)
     if symmetric:
         return _symmetric_laplacian_2d(torch, dev, N, coefficient, Ny)
     W, n, i, ix, iy = _grid(torch, dev, N, Ny)
@@ -110,6 +115,31 @@ def _symmetric_laplacian_2d(torch, dev, N, coefficient, Ny):
     if int(indptr[-1].item()) >= 2 ** 31:
         raise OverflowError("nnz does not fit int32")
     return DevCSR((n, n), indptr.to(torch.int32), cols[keep].to(torch.int32), vals[keep].contiguous())
+
+
+def _neumann_laplacian_2d(torch, dev, N, coefficient, Ny):
+    """the closed form of problems.neumann_stencil_2d: five candidate entries per row, those outside the grid removed"""
+    from .problems import neumann_stencil_2d
+    W, n, i, ix, iy = _grid(torch, dev, N, Ny)
+    h = 1.0 / N
+    if coefficient is None:
+        def kf(x, y):
+            return torch.ones_like(x)
+    else:
+        def kf(x, y):
+            return coefficient(torch, x, y)
+    x, y = ix.to(torch.float64), iy.to(torch.float64)
+    del ix, iy
+    vals, exists = neumann_stencil_2d(x, y, float(N), float(Ny),
+                                      lambda sx, sy: kf((sx + 2.0 / 3.0) * h, (sy + 1.0 / 3.0) * h),
+                                      lambda sx, sy: kf((sx + 1.0 / 3.0) * h, (sy + 2.0 / 3.0) * h), xp=torch)
+    keep = torch.stack(exists, dim=1)
+    cols = torch.stack([i - W, i - 1, i, i + 1, i + W], dim=1)
+    indptr = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(keep.sum(dim=1), 0, out=indptr[1:])
+    if int(indptr[-1].item()) >= 2 ** 31:
+        raise OverflowError("nnz does not fit int32")
+    return DevCSR((n, n), indptr.to(torch.int32), cols[keep].to(torch.int32), torch.stack(vals, dim=1)[keep].contiguous())
 
 
 def structured_rhs_2d(N, f_value=-1.0, Ny=None, device=None):

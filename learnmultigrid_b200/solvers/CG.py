@@ -51,6 +51,10 @@ class CG(IterativeSolver):
             self.residual_vector = r
             self.last_timing = getattr(h, "last_pcg_timing", None)
             return
+        if h is not None and getattr(h, "null", None) is not None:
+            # the host loop projects neither b nor x: with a singular operator it would not converge
+            raise ValueError("a multigrid preconditioner with a declared null space runs CG inside its hierarchy only: "
+                             "call solve() without initial_guess, on the preconditioner's own matrix")
         d = self._device_csr()
         torch, lib, n = d["torch"], d["lib"], d["n"]
         st = _lib.stream_handle(torch)

@@ -52,6 +52,30 @@ class Multigrid(IterativeSolver):
         self.setup = "device"
         self.fabric = None           # set by distribute(): run the V-cycle row-partitioned over several GPUs
         self.dist_options = {}
+        self.null_space = None       # set by set_null_space(): singular symmetric operator with this null vector
+        self._null_key = None
+
+    def set_null_space(self, null_space):
+        """Declare the null vector nu of a singular SYMMETRIC operator (pure Neumann problems; no reference
+        counterpart): None (default, a nonsingular operator), "constant" (the ones vector) or an array of n values.
+        The hierarchy then solves its coarsest level with the pseudo-inverse, and solve, v_cycle and the device PCG /
+        GMRES behind as_preconditioner remove nu from the right-hand side first (rhs_null_component holds
+        nu^T b / ||nu|| of what was removed: non-zero for a right-hand side that has no solution) and from the result,
+        which is then the minimum-norm (least-squares) solution.  Part of the hierarchy cache key; returns self."""
+        n = self.get_dimension()
+        if null_space is None or (isinstance(null_space, str) and null_space == "constant"):
+            key = null_space
+        elif isinstance(null_space, str):
+            raise ValueError("null_space must be None, 'constant' or an array of %d values" % n)
+        else:
+            null_space = np.asarray(null_space, dtype=np.float64).reshape(-1)
+            if null_space.size != n:
+                raise ValueError("null space vector has %d entries, operator has %d rows" % (null_space.size, n))
+            import hashlib
+            key = hashlib.sha1(null_space.tobytes()).hexdigest()
+        self.null_space = null_space
+        self._null_key = key
+        return self
 
     def distribute(self, fabric=None, **options):
         """Row-partition the fine levels over the ranks of `fabric` (default: the torch.distributed world, one
@@ -81,6 +105,7 @@ class Multigrid(IterativeSolver):
                             **self._cheby_kw(smoother, cheby_degree, cheby_bounds))
         params = h.make_params(nu_pre=smooth_steps, nu_post=smooth_steps, omega=omega)
         h.set_rhs(self.rhs)
+        self._project_rhs(h)
         if initial_guess is None:
             h.zero_x()
         else:
@@ -112,12 +137,27 @@ class Multigrid(IterativeSolver):
                 res = h.last_norm()
         if self.fabric is not None and hasattr(h, "check"):
             h.check()          # an exchange site that timed out leaves a wrong iterate behind: raise, do not return it
+        if self.null_space is not None:
+            h.project_null(h.levels[0].x)
         if self.fabric is not None and getattr(self, "local_solution", False) and hasattr(h, "get_x_local"):
             self.solution = h.get_x_local(view=getattr(self, "pinned_io", False))     # this rank's row block only
         else:
             self.solution = h.get_x(view=getattr(self, "pinned_io", False))
         self.track_res = track_res
         self._residual_dirty = True
+
+    def _project_rhs(self, h):
+        """remove the declared null vector from the hierarchy's right-hand side (set_null_space)"""
+        if self.null_space is not None:
+            h.project_rhs()
+
+    @property
+    def rhs_null_component(self):
+        """nu^T b / ||nu|| of what the last solve, v_cycle, CG or GMRES through this solver's hierarchy removed from its
+        right-hand side (None without a declared null space)"""
+        if self.null_space is None or self._hier is None:
+            return None
+        return getattr(self._hier, "rhs_null_component", None)
 
     def get_residual_vector(self):
         if getattr(self, "_residual_dirty", False) and self._hier is not None:
@@ -141,8 +181,11 @@ class Multigrid(IterativeSolver):
                             **self._cheby_kw(smoother, cheby_degree, cheby_bounds))
         params = h.make_params(nu_pre=smooth_steps, nu_post=smooth_steps, omega=omega)
         h.set_rhs(rhs)
+        self._project_rhs(h)
         h.set_x(u0)
         h.vcycle(params)
+        if self.null_space is not None:
+            h.project_null(h.levels[0].x)
         return h.get_x()
 
     def interpolator(self, dimension, _):
@@ -228,15 +271,18 @@ class Multigrid(IterativeSolver):
         if (A is save and src is not None and sp.isspmatrix_csr(src) and src.dtype == np.float64
                 and src.has_canonical_format):
             A = src
+        null = {} if self.null_space is None else {"null_space": self.null_space}
         if self.fabric is not None and self.fabric.world > 1:
             from ..distributed import DistributedHierarchy
-            return DistributedHierarchy(A, qs, self.fabric, smoother=kind, colors=colors, **cheby, **self.dist_options)
-        return DeviceHierarchy(A, qs, smoother=kind, colors=colors, setup=self.setup, **cheby)
+            return DistributedHierarchy(A, qs, self.fabric, smoother=kind, colors=colors, **cheby, **null,
+                                        **self.dist_options)
+        return DeviceHierarchy(A, qs, smoother=kind, colors=colors, setup=self.setup, **cheby, **null)
 
     def _hierarchy(self, levels, smoother, gs_order, colors, first_call, cheby_degree=2, cheby_bounds=None):
         cb = None if cheby_bounds is None else tuple(tuple(float(v) for v in b) for b in cheby_bounds)
         key = (levels, smoother, gs_order, bool(first_call), id(self.matrix), None if colors is None else id(colors),
-               cheby_degree if smoother == "Chebyshev" else None, cb if smoother == "Chebyshev" else None)
+               cheby_degree if smoother == "Chebyshev" else None, cb if smoother == "Chebyshev" else None,
+               self._null_key)
         if self._hier is None or self._hier_key != key:
             self._hier = self._build(self.matrix, levels, smoother, gs_order, colors, first_call,
                                      **self._cheby_kw(smoother, cheby_degree, cheby_bounds))

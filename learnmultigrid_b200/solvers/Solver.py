@@ -105,24 +105,46 @@ class DirectSolver(Solver):
     def __init__(self, matrix, rhs):
         super().__init__(matrix, rhs)
 
-    def solve(self):
-        from ..coarse import build_coarse_solver
+    def solve(self, null_space=None):
+        """null_space: None, "constant" or n values -- the null vector nu of a singular SYMMETRIC matrix.  The solve
+        then runs through the pinned factor and returns the minimum-norm solution of the system with nu removed from
+        the right-hand side (rhs_null_component: nu^T b / ||nu|| of what was removed; the least-squares solution when
+        it is not 0); the refinement steps work on that projected system."""
+        from ..coarse import build_coarse_solver, apply_coarse
         d = self._device_csr()
         torch, lib, n = d["torch"], d["lib"], d["n"]
         st = _lib.stream_handle(torch)
+        nu = None
+        if null_space is not None:
+            from ..engine import declared_null_vector
+            nu, _ = declared_null_vector(torch, d["dev"], d["host"], null_space)
         solver = build_coarse_solver(torch, d["dev"], n, d["indptr"], d["indices"], d["values"], self.DENSE_MAX,
-                                     (d["host"].indptr, d["host"].indices))
+                                     (d["host"].indptr, d["host"].indices), singular=nu is not None,
+                                     label="DirectSolver")
         self.method = "dense inverse" if solver.kind == _lib.MG_COARSE_DENSE else (
             "block cyclic reduction" + (" after reverse Cuthill-McKee" if getattr(solver, "perm", None) is not None else ""))
+        self.null_info = getattr(solver, "null_info", None)
 
         def apply(rhs, out):
-            if solver.kind == _lib.MG_COARSE_DENSE:
+            if nu is not None:
+                apply_coarse(solver, rhs.clone(), out)
+            elif solver.kind == _lib.MG_COARSE_DENSE:
                 _lib.check(lib.mg_dense_gemv(n, n, solver.inv.data_ptr(), rhs.data_ptr(), out.data_ptr(), st),
                            "mg_dense_gemv")
             else:
                 solver.solve(torch, rhs, out)
 
+        def project(v):
+            if nu is not None:
+                _lib.check(lib.mg_project_out(n, nu.data_ptr(), inv_nn, -1, v.data_ptr(), d["ws"].data_ptr(), None, st),
+                           "mg_project_out")
+
         b = self._upload(self.rhs)
+        self.rhs_null_component = None
+        if nu is not None:
+            inv_nn = 1.0 / self._dot(nu, nu)
+            self.rhs_null_component = self._dot(nu, b) * float(np.sqrt(inv_nn))
+            project(b)
         x = torch.empty_like(b)
         apply(b, x)
         r = torch.empty_like(b)
@@ -140,6 +162,7 @@ class DirectSolver(Solver):
             if not resn < res:
                 break
             x, r, res = xn, rn, resn
+        project(x)
         self.solution = x.cpu().numpy().reshape(self.dim, 1)
         self.residual_vector = r.cpu().numpy().reshape(self.dim, 1)
         self.residual = res
